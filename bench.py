@@ -3,11 +3,12 @@
 the glass dragon (100,000 triangles) + chessboard floor at 1024x1024, one round = 16 Mi photons per GPU
 (BASELINE.json configs[2], "c3_dragon_glass": 50 rounds x 16M photons).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one round of the hot path: trace `--photons` photons per GPU against the persistent hitpoint set (emission,
 closest hit, bounces, 27-cell deposits), all-reduce the per-hitpoint accumulators when N > 1, per-round radius/flux update.
-`value` times K rounds on the device (inputs resident: scene, BVH, hitpoints, grid). `e2e` times the whole render()
+`value` times K rounds on the device (inputs resident: scene, BVH, hitpoints, grid). `--dump-outputs DIR` writes the hitpoint
+state the last timed round left (see dump_outputs), so that two builds can be compared output for output. `e2e` times the whole render()
 of the named config through the C ABI from HOST buffers: scene H2D + LBVH build + eye pass + grid + `--e2e-rounds` rounds +
 image D2H, wall clock. `roofline` comes from a separate profiled round of the same run (every kernel launch bracketed by
 CUDA events on the library's stream). Prints ONE JSON line on rank 0.
@@ -210,6 +211,33 @@ def cpu_baseline(scene, cfg, photons, threads=None, warm_rounds=0, shipped_photo
     return out
 
 
+DUMP_BYTES = 64_000_000  # all files of --dump-outputs together
+NPY_HEADER = 128
+DUMP_NAMES = ("hitpoint_flux", "hitpoint_r2", "hitpoint_n", "hitpoint_index")
+
+
+def dump_outputs(out_dir, hp, limit=DUMP_BYTES):
+    """Writes what a round leaves for its caller, the per-hitpoint state in canonical order, as float64 .npy files: hitpoint_flux
+    [n, 3], hitpoint_r2 [n], hitpoint_n [n] (accepted-photon counts). When that exceeds `limit` bytes, the same seeded sample of
+    rows is taken from each array and the sampled row numbers go to hitpoint_index.npy. Files of an earlier dump into the same
+    directory are removed first, so that a stale hitpoint_index.npy never sits beside whole arrays."""
+    arrays = {"hitpoint_flux": hp["flux"], "hitpoint_r2": hp["r2"], "hitpoint_n": hp["n"]}
+    n = len(hp["r2"])
+    row_bytes = 8 * sum(a[:1].size for a in arrays.values())
+    if n * row_bytes + len(arrays) * NPY_HEADER > limit:
+        k = (limit - (len(arrays) + 1) * NPY_HEADER) // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["hitpoint_index"] = rows
+    os.makedirs(out_dir, exist_ok=True)
+    for name in DUMP_NAMES:
+        path = os.path.join(out_dir, name + ".npy")
+        if os.path.exists(path):
+            os.remove(path)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def run_reference(args):
     """The reference arm: the CPU implementation of the path on ALL host cores of the box. The timed value is the oracle port (pinned bit
     for bit to the compiled reference, lock-free Philox streams: the STRONGER baseline); the unmodified reference binary's own loop, which
@@ -236,6 +264,8 @@ def run_reference(args):
         o.round_update()
         if s >= args.warmup:
             times.append(sec)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, o.download_hitpoints(fields=("flux", "r2", "n")))
     c1 = o.counters()
     total = sum(times)
     v = sample * len(times) / total
@@ -343,6 +373,8 @@ def run_gpu(args):
     clocks = sampler.result()
     ms = e0.elapsed_time(e1)
     c2 = g.counters()
+    if args.dump_outputs and rank == 0:  # every rank holds the same state after a round's update
+        dump_outputs(args.dump_outputs, g.download_hitpoints(fields=("flux", "r2", "n")))
     if world > 1:
         t = torch.tensor([ms], device=f"cuda:{local}", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -545,6 +577,8 @@ def main():
                          "collective call in a round; fastest at 2 GPUs); torch: torch.distributed all-reduce on the library's stream")
     ap.add_argument("--f64-too", type=int, default=1, help="1: also time the same rounds with fp64 accumulators (value_f64_accumulators)")
     ap.add_argument("--e2e-rounds", type=int, default=-1, help="rounds of the end-to-end render() (default: the workload's own, c3 = 50; 0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the hitpoint state the last one left as DIR/<name>.npy "
+                                                          "(float64, at most 64 MB in all; a seeded sample of the hitpoints beyond that)")
     args = ap.parse_args()
     select_workload(args.workload)
     if args.e2e_rounds < 0:
