@@ -29,6 +29,7 @@ ABI_SYMBOLS = [
     "cgrt_download_accum", "cgrt_download_grid", "cgrt_get_counters", "cgrt_get_timings", "cgrt_set_counting", "cgrt_set_profiling", "cgrt_set_culling", "cgrt_set_overlap", "cgrt_average_u8", "cgrt_average_f64",
     "cgrt_check_guards", "cgrt_release_cached_memory", "cgrt_photon_chunk", "cgrt_deposit_record_bytes", "cgrt_trace",
     "cgrt_peer_export", "cgrt_peer_attach", "cgrt_comm_unique_id", "cgrt_comm_init_rank", "cgrt_comm_init_all", "cgrt_comm_destroy", "cgrt_allgather_hitpoints", "cgrt_set_comm",
+    "cgrt_set_sppm", "cgrt_sppm_begin_round", "cgrt_sppm_download_pixels",
 ]
 
 
@@ -264,6 +265,22 @@ class Context:
         rgb8 = np.zeros((self.cfg.height, self.cfg.width, 3), np.uint8) if want_rgb8 else None
         self._ck(self.L.cgrt_gather_image(self.h, C.c_double(n_emitted), _p(img, c_dp), _p(rgb8, c_u8p)))
         return (img, rgb8) if want_rgb8 else img
+
+    # -- stochastic progressive photon mapping
+    def set_sppm(self, mode):
+        """0 off (PPM), 1 jitter, 2 corner (include/cgrt.h CGRT_SPPM_*). After commit, before any eye pass."""
+        self._ck(self.L.cgrt_set_sppm(self.h, int(mode)))
+
+    def sppm_begin_round(self, r):
+        """Eye pass of round r with its own camera stream, grid at the pixels' current radii."""
+        self._ck(self.L.cgrt_sppm_begin_round(self.h, C.c_uint32(r)))
+
+    def sppm_download_pixels(self):
+        """-> dict tau [H, W, 3], r2 [H, W], n [H, W] (row h = image[h])."""
+        H, W = self.cfg.height, self.cfg.width
+        o = dict(tau=np.zeros((H, W, 3)), r2=np.zeros((H, W)), n=np.zeros((H, W), np.int32))
+        self._ck(self.L.cgrt_sppm_download_pixels(self.h, _p(o["tau"], c_dp), _p(o["r2"], c_dp), _p(o["n"], c_ip)))
+        return o
 
     # -- multi-run averaging (average.cpp)
     def average_u8(self, images):

@@ -262,6 +262,15 @@ struct cgrt_ctx {
     int *d_maxcnt = nullptr;
     size_t auto_chunk = 0;
     int counting = 0;  // 1: photon trace kernels also count BVH node visits / triangle tests (roofline accounting)
+    // stochastic PPM (cgrt_set_sppm): per-pixel statistics, and the visible-point count the per-round buffers are sized for. Every
+    // round rebuilds the grid; sizing its buffers from this capacity (grown with headroom, never shrunk) instead of the round's exact
+    // count makes every round ask the pool and the arena for the same sizes, so device memory reaches a steady state.
+    int sppm = CGRT_SPPM_OFF;
+    uint32_t sppm_round = 0;    // the round whose camera stream the eye pass draws
+    double *pix_tau = nullptr;  // [W*H][4] tau (+pad)
+    double *pix_r2 = nullptr;   // [W*H]
+    int *pix_cnt = nullptr;     // [W*H]
+    size_t sppm_cap = 0;
 };
 
 namespace {
@@ -448,9 +457,11 @@ int radix_sort_async(cgrt_ctx *ctx, SortScratch<K> &sc, size_t n, const K *keys_
     *perm = src_v;
     return 0;
 }
-int radix_sort_dev(cgrt_ctx *ctx, size_t n, const uint64_t *keys_in, int nbits, uint64_t *keys_out, uint32_t *perm_out) {
+// reserve > n: the scratch is allocated for `reserve` keys (stable allocation sizes from call to call)
+int radix_sort_dev(cgrt_ctx *ctx, size_t n, const uint64_t *keys_in, int nbits, uint64_t *keys_out, uint32_t *perm_out, size_t reserve = 0) {
     if (n == 0) return 0;
     SortScratch<uint64_t> sc;
+    if (reserve > n) CKS(sort_scratch_reserve(ctx, sc, reserve));
     const uint64_t *ks;
     const uint32_t *pm;
     CKS(radix_sort_async(ctx, sc, n, keys_in, nbits, &ks, &pm));
@@ -737,7 +748,7 @@ void peer_release(cgrt_ctx *ctx) {
 // =================================================================================================================
 extern "C" {
 
-int cgrt_version(void) { return 100; }
+int cgrt_version(void) { return 101; }
 
 void cgrt_default_config(cgrt_config *c) {
     memset(c, 0, sizeof *c);
@@ -860,6 +871,7 @@ int cgrt_set_config(cgrt_ctx *ctx, const cgrt_config *cfg) {
         FAIL(CGRT_ERR_CAPACITY, "config: width*height*samples must be < 2^28 (creation sequence is 32 bits)");
     if (cfg->max_depth > 5) FAIL(CGRT_ERR_CAPACITY, "config: max_depth > 5 needs more than 4 DFS bits");
     if (ctx->hp_count) FAIL(CGRT_ERR_INVALID, "config cannot change after the eye pass");
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "config cannot change while SPPM is on (the pixel statistics are sized and seeded from it)");
     if (cfg->update_mode != 0 && cfg->update_mode != 1) FAIL(CGRT_ERR_INVALID, "config: update_mode must be 0 (per photon) or 1 (per round)");
     if (cfg->update_mode == 0 && ctx->comm) FAIL(CGRT_ERR_INVALID, "config: the per-photon update is not shard-invariant (one GPU only)");
     ctx->cfg = *cfg;
@@ -1181,11 +1193,14 @@ static int eye_wavefront(cgrt_ctx *ctx, size_t n, int depth0, int r0, bool gener
         CK(cudaMemsetAsync(ctx->d_qcount + (cur ^ 1), 0, sizeof(unsigned int), ctx->stream));
         bool f32 = true;  // every tree within the float bound: the instantiation without fp64 box arithmetic
         for (int b = 0; b < ctx->S.nbvh; b++) f32 = f32 && ctx->S.bvh[b].f32_ok;
-#define LAUNCH_EYE(FIRSTV, F32V)                                                                                                             \
-    eye_bounce_kernel<FIRSTV, F32V><<<nblk(n, 128), 128, 0, ctx->stream>>>(ctx->S, P, depth, ctx->q[cur], (unsigned int)n, r0, ctx->q[cur ^ 1], \
-                                                                          ctx->d_qcount + (cur ^ 1), ctx->hp_rec, ctx->d_hp_count, ctx->hp_cap, ctx->d_ctr)
-        if (generate && depth == depth0) { if (f32) LAUNCH_EYE(true, true); else LAUNCH_EYE(true, false); }
-        else { if (f32) LAUNCH_EYE(false, true); else LAUNCH_EYE(false, false); }
+#define LAUNCH_EYE(FIRSTV, F32V, SPPMV)                                                                                                      \
+    eye_bounce_kernel<FIRSTV, F32V, SPPMV><<<nblk(n, 128), 128, 0, ctx->stream>>>(ctx->S, P, depth, ctx->q[cur], (unsigned int)n, r0, ctx->q[cur ^ 1], \
+                                                                          ctx->d_qcount + (cur ^ 1), ctx->hp_rec, ctx->d_hp_count, ctx->hp_cap, ctx->d_ctr, \
+                                                                          ctx->sppm_round)
+        if (generate && depth == depth0 && ctx->sppm == CGRT_SPPM_JITTER) { if (f32) LAUNCH_EYE(true, true, CGRT_SPPM_JITTER); else LAUNCH_EYE(true, false, CGRT_SPPM_JITTER); }
+        else if (generate && depth == depth0 && ctx->sppm == CGRT_SPPM_CORNER) { if (f32) LAUNCH_EYE(true, true, CGRT_SPPM_CORNER); else LAUNCH_EYE(true, false, CGRT_SPPM_CORNER); }
+        else if (generate && depth == depth0) { if (f32) LAUNCH_EYE(true, true, 0); else LAUNCH_EYE(true, false, 0); }
+        else { if (f32) LAUNCH_EYE(false, true, 0); else LAUNCH_EYE(false, false, 0); }
 #undef LAUNCH_EYE
         ctx->launches++;
         CK(cudaGetLastError());
@@ -1201,8 +1216,13 @@ static int eye_wavefront(cgrt_ctx *ctx, size_t n, int depth0, int r0, bool gener
 }
 
 // ---- eye pass ------------------------------------------------------------------------------------------------------
+static int eye_pass_impl(cgrt_ctx *ctx, int y0, int y1);
 int cgrt_eye_pass(cgrt_ctx *ctx, int y0, int y1) {
     if (!ctx) return CGRT_ERR_INVALID;
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is on: cgrt_sppm_begin_round traces the eye pass of every round");
+    return eye_pass_impl(ctx, y0, y1);
+}
+static int eye_pass_impl(cgrt_ctx *ctx, int y0, int y1) {
     if (!ctx->committed) FAIL(CGRT_ERR_INVALID, "commit the scene first");
     if (ctx->grid_built) FAIL(CGRT_ERR_INVALID, "grid already built");
     const PassParams &P = ctx->P;
@@ -1232,6 +1252,7 @@ int cgrt_export_hitpoints_dev(cgrt_ctx *ctx, void **records_dev, int64_t *count)
 }
 int cgrt_import_hitpoints_dev(cgrt_ctx *ctx, const void *records_dev, int64_t count) {
     if (!ctx || count < 0 || (count > 0 && !records_dev)) return CGRT_ERR_INVALID;
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is on: every round makes its own visible points (multi-GPU SPPM is not supported)");
     if (ctx->grid_built) FAIL(CGRT_ERR_INVALID, "grid already built");
     CK(cudaSetDevice(ctx->device));
     // replaces the current set (the caller passes the all-gathered union, which includes this rank's own records)
@@ -1264,27 +1285,36 @@ static int build_r2_table(cgrt_ctx *ctx, int cap) {
 }
 
 // ---- grid ----------------------------------------------------------------------------------------------------------
+static int build_grid_impl(cgrt_ctx *ctx);
 int cgrt_build_grid(cgrt_ctx *ctx) {
     if (!ctx) return CGRT_ERR_INVALID;
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is on: cgrt_sppm_begin_round builds the grid of every round");
+    return build_grid_impl(ctx);
+}
+static int build_grid_impl(cgrt_ctx *ctx) {
     if (ctx->grid_built) FAIL(CGRT_ERR_INVALID, "grid already built");
     CK(cudaSetDevice(ctx->device));
     PhaseTimer timer(ctx, 1);
     const PassParams &P = ctx->P;
     unsigned int n = ctx->hp_count;
     ctx->nhp = n;
+    // buffers are sized for m >= n hitpoints: m = n, except under SPPM (see cgrt_ctx::sppm_cap)
+    if (ctx->sppm && n > ctx->sppm_cap) ctx->sppm_cap = (size_t)n + n / 8 + 4096;
+    const size_t m = ctx->sppm ? ctx->sppm_cap : (size_t)n;
     size_t npix = (size_t)P.width * P.height;
     CKS(dalloc(ctx, &ctx->cell_start, (size_t)P.hashsize + 1));
     CKS(dalloc(ctx, &ctx->pix_start, npix + 1));
-    CKS(dalloc(ctx, &ctx->pix_perm, (size_t)n));
+    CKS(dalloc(ctx, &ctx->pix_perm, m));
     // The arrays the deposit kernel gathers from — prefilter, exact records, f, accumulators — live in one slab. (Marking the slab
     // persisting in L2 with an access-policy window was measured: the deposit kernel did not move (11.0 ms, it is not bound by L2
     // misses) while the counting sort lost its L2-resident cursors (1.2 -> 4.2 ms), so no window is set.)
     size_t acc_bytes = (size_t)n * 4 * (ctx->cfg.accum_mode == 0 ? sizeof(double) : sizeof(float));
     {
         auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-        size_t o_pre = 0, o_pren = o_pre + up((size_t)n * sizeof(float4)), o_pref = o_pren + up((size_t)n * sizeof(float4));
-        size_t o_hot = o_pref + up((size_t)n * sizeof(float4)), o_f = o_hot + up((size_t)n * sizeof(HpHot));
-        size_t o_acc = o_f + up((size_t)n * 4 * sizeof(double)), total = o_acc + up(acc_bytes);
+        const size_t acc_cap = m * 4 * (ctx->cfg.accum_mode == 0 ? sizeof(double) : sizeof(float));
+        size_t o_pre = 0, o_pren = o_pre + up(m * sizeof(float4)), o_pref = o_pren + up(m * sizeof(float4));
+        size_t o_hot = o_pref + up(m * sizeof(float4)), o_f = o_hot + up(m * sizeof(HpHot));
+        size_t o_acc = o_f + up(m * 4 * sizeof(double)), total = o_acc + up(acc_cap);
         char *slab;
         CKS(dalloc(ctx, &slab, total));
         ctx->A.pre = reinterpret_cast<float4 *>(slab + o_pre);
@@ -1300,22 +1330,26 @@ int cgrt_build_grid(cgrt_ctx *ctx) {
         CKS(dalloc(ctx, &ctx->d_maxcnt, 1));
         CK(cudaMemsetAsync(ctx->d_maxcnt, 0, sizeof(int), ctx->stream));
     }
-    CKS(dalloc(ctx, &ctx->A.flux, (size_t)n * 4));
-    CKS(dalloc(ctx, &ctx->A.cnt, (size_t)n));
-    CKS(dalloc(ctx, &ctx->A.hw, (size_t)n * 2));
-    CKS(dalloc(ctx, &ctx->A.key, (size_t)n));
-    CKS(dalloc(ctx, &ctx->A.seq, (size_t)n));
+    CKS(dalloc(ctx, &ctx->A.flux, m * 4));
+    CKS(dalloc(ctx, &ctx->A.cnt, m));
+    CKS(dalloc(ctx, &ctx->A.hw, m * 2));
+    CKS(dalloc(ctx, &ctx->A.key, m));
+    CKS(dalloc(ctx, &ctx->A.seq, m));
     if (n > 0) {
         uint64_t *keys, *keys_sorted, *pixkeys, *pixkeys_sorted;
         uint32_t *perm;
-        CKS(dalloc(ctx, &keys, (size_t)n)); CKS(dalloc(ctx, &keys_sorted, (size_t)n)); CKS(dalloc(ctx, &perm, (size_t)n));
-        CKS(dalloc(ctx, &pixkeys, (size_t)n)); CKS(dalloc(ctx, &pixkeys_sorted, (size_t)n));
+        CKS(dalloc(ctx, &keys, m)); CKS(dalloc(ctx, &keys_sorted, m)); CKS(dalloc(ctx, &perm, m));
+        CKS(dalloc(ctx, &pixkeys, m)); CKS(dalloc(ctx, &pixkeys_sorted, m));
         hp_extract_keys_kernel<<<nblk(n, 256), 256, 0, ctx->stream>>>(ctx->hp_rec, n, keys);
         ctx->launches++;
         int kbits = 32;
         while (kbits > 1 && !(((uint64_t)P.hashsize - 1) >> (kbits - 1))) kbits--;
-        CKS(radix_sort_dev(ctx, n, keys, 32 + kbits, keys_sorted, perm));
+        CKS(radix_sort_dev(ctx, n, keys, 32 + kbits, keys_sorted, perm, m));
         hp_gather_sorted_kernel<<<nblk(n, 256), 256, 0, ctx->stream>>>(ctx->hp_rec, perm, n, P.r2_init, ctx->A, pixkeys, P.width);
+        if (ctx->sppm) {
+            sppm_visible_radius_kernel<<<nblk(n, 256), 256, 0, ctx->stream>>>(n, ctx->A, ctx->pix_r2, P.width);
+            ctx->launches++;
+        }
         lower_bound_table_kernel<<<nblk((size_t)n + 1, 256), 256, 0, ctx->stream>>>(ctx->A.key, nullptr, n, P.hashsize, ctx->cell_start);
         CKS(dalloc(ctx, &ctx->reach, (size_t)1 << (CGRT_REACH_BITS - 5)));
         CK(cudaMemsetAsync(ctx->reach, 0, sizeof(uint32_t) << (CGRT_REACH_BITS - 5), ctx->stream));
@@ -1324,7 +1358,7 @@ int cgrt_build_grid(cgrt_ctx *ctx) {
         ctx->launches += 2;
         int pbits = 1;
         while (pbits < 40 && ((uint64_t)npix >> pbits)) pbits++;
-        CKS(radix_sort_dev(ctx, n, pixkeys, pbits, pixkeys_sorted, ctx->pix_perm));
+        CKS(radix_sort_dev(ctx, n, pixkeys, pbits, pixkeys_sorted, ctx->pix_perm, m));
         lower_bound_table_kernel<<<nblk((size_t)n + 1, 256), 256, 0, ctx->stream>>>(nullptr, pixkeys_sorted, n, (unsigned int)npix, ctx->pix_start);
         ctx->launches++;
         CK(cudaStreamSynchronize(ctx->stream));
@@ -1334,12 +1368,28 @@ int cgrt_build_grid(cgrt_ctx *ctx) {
         CK(cudaMemsetAsync(ctx->cell_start, 0, ((size_t)P.hashsize + 1) * sizeof(uint32_t), ctx->stream));
         CK(cudaMemsetAsync(ctx->pix_start, 0, (npix + 1) * sizeof(uint32_t), ctx->stream));
     }
-    // the raw records are no longer needed
-    CKS(dfree(ctx, ctx->hp_rec));
-    ctx->hp_rec = nullptr;
-    ctx->hp_cap = 0;
+    // the raw records are no longer needed (SPPM keeps the buffer at its capacity for the next round's eye pass)
+    if (!ctx->sppm) {
+        CKS(dfree(ctx, ctx->hp_rec));
+        ctx->hp_rec = nullptr;
+        ctx->hp_cap = 0;
+    }
     ctx->grid_built = true;
     timer.stop();
+    return CGRT_OK;
+}
+
+// SPPM: release the grid and the visible points of the last round (every buffer build_grid_impl allocated).
+static int release_grid(cgrt_ctx *ctx) {
+    HpArrays &A = ctx->A;
+    CKS(dfree(ctx, A.pre));  // the slab: pre, pre_n, pre_f, hot, f, accumulators
+    CKS(dfree(ctx, A.flux)); CKS(dfree(ctx, A.cnt)); CKS(dfree(ctx, A.hw)); CKS(dfree(ctx, A.key)); CKS(dfree(ctx, A.seq));
+    CKS(dfree(ctx, ctx->cell_start)); CKS(dfree(ctx, ctx->pix_start)); CKS(dfree(ctx, ctx->pix_perm)); CKS(dfree(ctx, ctx->reach));
+    memset(&A, 0, sizeof A);
+    ctx->acc = nullptr;
+    ctx->cell_start = ctx->pix_start = ctx->pix_perm = ctx->reach = nullptr;
+    ctx->grid_built = false;
+    ctx->nhp = 0;
     return CGRT_OK;
 }
 
@@ -1523,6 +1573,7 @@ int cgrt_trace(cgrt_ctx *ctx, int64_t n, const double *org, const double *dir, c
     if (!ctx || n < 0 || (n > 0 && (!org || !dir || !weight))) return CGRT_ERR_INVALID;
     if (!ctx->committed) FAIL(CGRT_ERR_INVALID, "commit the scene first");
     if (depth < 0) FAIL(CGRT_ERR_INVALID, "negative depth");
+    if (flag && ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is on: cgrt_sppm_begin_round makes every round's visible points");
     if (n == 0 || depth >= ctx->P.max_depth) return CGRT_OK;  // main.cpp:46: nothing is traced beyond MAX_DEPTH
     if (n >= (1ll << 28)) FAIL(CGRT_ERR_CAPACITY, "cgrt_trace: at most 2^28 rays per call");
     CK(cudaSetDevice(ctx->device));
@@ -1586,6 +1637,7 @@ int cgrt_allreduce_accum(cgrt_ctx *ctx, void *nccl_comm) {
 
 int cgrt_peer_export(cgrt_ctx *ctx, void *handle128) {
     if (!ctx || !handle128) return CGRT_ERR_INVALID;
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
     if (!ctx->grid_built) FAIL(CGRT_ERR_INVALID, "build the grid first");
     if (ctx->cfg.update_mode == 0) FAIL(CGRT_ERR_INVALID, "the per-photon update is not shard-invariant (one GPU only)");
     if (ctx->peer.block) FAIL(CGRT_ERR_INVALID, "peer block already exported");
@@ -1614,6 +1666,7 @@ int cgrt_peer_export(cgrt_ctx *ctx, void *handle128) {
 
 int cgrt_peer_attach(cgrt_ctx *ctx, int rank, int world, const void *handles) {
     if (!ctx || !handles || world < 1 || world > CGRT_MAX_PEERS || rank < 0 || rank >= world) return CGRT_ERR_INVALID;
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
     cgrt_ctx::Peer &P = ctx->peer;
     if (!P.block) FAIL(CGRT_ERR_INVALID, "cgrt_peer_export first");
     if (P.attached) FAIL(CGRT_ERR_INVALID, "peers already attached");
@@ -1651,6 +1704,7 @@ int cgrt_peer_attach(cgrt_ctx *ctx, int rank, int world, const void *handles) {
 
 int cgrt_set_comm(cgrt_ctx *ctx, void *nccl_comm, int world) {
     if (!ctx || world < 1) return CGRT_ERR_INVALID;
+    if (nccl_comm && ctx->sppm) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
     if (nccl_comm && ctx->cfg.update_mode == 0) FAIL(CGRT_ERR_INVALID, "the per-photon update is not shard-invariant (one GPU only)");
     if (nccl_comm && !nccl_api().ok) FAIL(CGRT_ERR_NCCL, "NCCL is not available: " + nccl_api().why);
     CKS(join_update(ctx));
@@ -1691,6 +1745,7 @@ int cgrt_comm_destroy(void *comm) {
 // order = row order, so the union is in creation order; the grid's sort key makes the order irrelevant anyway).
 int cgrt_allgather_hitpoints(cgrt_ctx *ctx, void *nccl_comm, int world) {
     if (!ctx || world < 1) return CGRT_ERR_INVALID;
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
     if (ctx->grid_built) FAIL(CGRT_ERR_INVALID, "grid already built");
     if (!nccl_comm || world == 1) return CGRT_OK;
     NcclApi &N = nccl_api();
@@ -1741,6 +1796,19 @@ int cgrt_round_update(cgrt_ctx *ctx) {
     CKS(join_update(ctx));
     PhaseTimer timer(ctx, 4, ctx->profiling != 0);  // asynchronous unless profiling
     unsigned int n = ctx->nhp;
+    if (ctx->sppm) {  // fold the round into the pixels, in stream order: the next round's eye pass waits for it anyway
+        const unsigned int npix = (unsigned int)((size_t)ctx->P.width * ctx->P.height);
+        if (n > 0) {
+            if (ctx->cfg.accum_mode == 0)
+                sppm_fold_kernel<0><<<nblk(npix, 256), 256, 0, ctx->stream>>>(npix, ctx->P.alpha, ctx->pix_start, ctx->pix_perm, ctx->acc, ctx->pix_tau, ctx->pix_r2, ctx->pix_cnt);
+            else
+                sppm_fold_kernel<1><<<nblk(npix, 256), 256, 0, ctx->stream>>>(npix, ctx->P.alpha, ctx->pix_start, ctx->pix_perm, ctx->acc, ctx->pix_tau, ctx->pix_r2, ctx->pix_cnt);
+            ctx->launches++;
+            CK(cudaGetLastError());
+        }
+        timer.stop();
+        return CGRT_OK;
+    }
     // the tail of a round on its own stream (see cgrt_ctx::ustream); on the main stream while profiling so that its events bracket it —
     // and when an NCCL all-reduce is part of it: measured on 8 GPUs, the collective on the side stream is SLOWER than in stream order
     // (c2: 5.40 vs 4.93 ms per round, c1: 5.72 vs 5.54): NCCL's blocks cannot become resident next to the persistent emission kernel of
@@ -1822,13 +1890,75 @@ int cgrt_gather_image(cgrt_ctx *ctx, double n_emitted, double *rgb, uint8_t *rgb
     CKS(dalloc(ctx, &d_rgb, npix * 3));
     if (rgb8) CKS(dalloc(ctx, &d_rgb8, npix * 3));
     // main.cpp:256 divides by num_photon*num_threads*num_of_samples: the caller states the photons, the samples factor comes from the config
-    image_gather_kernel<<<nblk(npix, 256), 256, 0, ctx->stream>>>(P.width, P.height, n_emitted * (double)P.samples, ctx->pix_start, ctx->pix_perm, ctx->A.hot, ctx->A.flux,
-                                                                  d_rgb, d_rgb8);
+    if (ctx->sppm)
+        sppm_image_kernel<<<nblk(npix, 256), 256, 0, ctx->stream>>>(P.width, P.height, n_emitted * (double)P.samples, ctx->pix_tau, ctx->pix_r2, d_rgb, d_rgb8);
+    else
+        image_gather_kernel<<<nblk(npix, 256), 256, 0, ctx->stream>>>(P.width, P.height, n_emitted * (double)P.samples, ctx->pix_start, ctx->pix_perm, ctx->A.hot,
+                                                                      ctx->A.flux, d_rgb, d_rgb8);
     ctx->launches++;
     CK(cudaGetLastError());
     CKS(download_free(ctx, rgb, d_rgb, npix * 3));
     if (rgb8) CKS(download_free(ctx, rgb8, d_rgb8, npix * 3));
     timer.stop();
+    return CGRT_OK;
+}
+
+// ---- stochastic progressive photon mapping --------------------------------------------------------------------------
+int cgrt_set_sppm(cgrt_ctx *ctx, int mode) {
+    if (!ctx) return CGRT_ERR_INVALID;
+    if (mode != CGRT_SPPM_OFF && mode != CGRT_SPPM_JITTER && mode != CGRT_SPPM_CORNER) FAIL(CGRT_ERR_INVALID, "SPPM mode must be 0 (off), 1 (jitter) or 2 (corner)");
+    if (!ctx->committed) FAIL(CGRT_ERR_INVALID, "commit the scene first");
+    if (ctx->hp_count || ctx->grid_built) FAIL(CGRT_ERR_INVALID, "SPPM must be chosen before any eye pass or grid");
+    if (mode && ctx->cfg.update_mode == 0) FAIL(CGRT_ERR_INVALID, "SPPM needs the per-round update (update_mode 1)");
+    if (mode && (ctx->comm || ctx->peer.block)) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
+    CK(cudaSetDevice(ctx->device));
+    CKS(dfree(ctx, ctx->pix_tau)); CKS(dfree(ctx, ctx->pix_r2)); CKS(dfree(ctx, ctx->pix_cnt));
+    ctx->pix_tau = ctx->pix_r2 = nullptr;
+    ctx->pix_cnt = nullptr;
+    ctx->sppm = mode;
+    ctx->sppm_round = 0;
+    if (!mode) return CGRT_OK;
+    const size_t npix = (size_t)ctx->P.width * ctx->P.height;
+    CKS(dalloc(ctx, &ctx->pix_tau, npix * 4));
+    CKS(dalloc(ctx, &ctx->pix_r2, npix));
+    CKS(dalloc(ctx, &ctx->pix_cnt, npix));
+    std::vector<double> r2(npix, ctx->P.r2_init);  // (200/height)^2, main.cpp:84,94
+    CK(cudaMemsetAsync(ctx->pix_tau, 0, npix * 4 * sizeof(double), ctx->stream));
+    CK(cudaMemsetAsync(ctx->pix_cnt, 0, npix * sizeof(int), ctx->stream));
+    CK(cudaMemcpyAsync(ctx->pix_r2, r2.data(), npix * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return CGRT_OK;
+}
+
+int cgrt_sppm_begin_round(cgrt_ctx *ctx, uint32_t round) {
+    if (!ctx) return CGRT_ERR_INVALID;
+    if (!ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is off: cgrt_set_sppm first");
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaStreamSynchronize(ctx->tstream));
+    CKS(join_update(ctx));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (ctx->grid_built) CKS(release_grid(ctx));
+    ctx->hp_count = 0;
+    CK(cudaMemsetAsync(ctx->d_hp_count, 0, sizeof(unsigned int), ctx->stream));
+    ctx->sppm_round = round;
+    CKS(eye_pass_impl(ctx, 0, ctx->P.height));
+    return build_grid_impl(ctx);
+}
+
+int cgrt_sppm_download_pixels(cgrt_ctx *ctx, double *tau, double *r2, int32_t *n) {
+    if (!ctx) return CGRT_ERR_INVALID;
+    if (!ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is off: cgrt_set_sppm first");
+    CK(cudaSetDevice(ctx->device));
+    CKS(join_update(ctx));
+    CK(cudaStreamSynchronize(ctx->stream));
+    const size_t npix = (size_t)ctx->P.width * ctx->P.height;
+    if (tau) {
+        std::vector<double> t(npix * 4);
+        CK(cudaMemcpy(t.data(), ctx->pix_tau, npix * 4 * sizeof(double), cudaMemcpyDeviceToHost));
+        for (size_t p = 0; p < npix; p++) { tau[3 * p] = t[4 * p]; tau[3 * p + 1] = t[4 * p + 1]; tau[3 * p + 2] = t[4 * p + 2]; }
+    }
+    if (r2) CK(cudaMemcpy(r2, ctx->pix_r2, npix * sizeof(double), cudaMemcpyDeviceToHost));
+    if (n) CK(cudaMemcpy(n, ctx->pix_cnt, npix * sizeof(int), cudaMemcpyDeviceToHost));
     return CGRT_OK;
 }
 

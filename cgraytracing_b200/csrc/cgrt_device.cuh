@@ -54,7 +54,8 @@ __host__ __device__ __forceinline__ double max3(double a, double b, double c) {
 // Philox4x32-10 counter RNG (replaces rand(), sampling.h). key = {seed_lo, seed_hi + pass},
 // counter = {path_lo, path_hi, dim, block}; u = (double)(word >> 1) * 2^-31 (a 31-bit lattice like rand()/RAND_MAX).
 // ---------------------------------------------------------------------------------------------------------------
-enum { PASS_EYE = 0, PASS_PHOTON = 1, PASS_BEZIER = 2 };
+// PASS_SPPM_EYE: the camera stream of stochastic progressive photon mapping, one per (eye path, round): dim = round.
+enum { PASS_EYE = 0, PASS_PHOTON = 1, PASS_BEZIER = 2, PASS_SPPM_EYE = 3 };
 
 struct Philox {
     uint32_t k0, k1, c0, c1, c2, c3;

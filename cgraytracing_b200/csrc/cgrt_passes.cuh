@@ -102,17 +102,22 @@ struct Counters {
 
 // F32: every tree lies within CGRT_F32_BOUND (all BASELINE scenes) — the traversal instantiation without fp64 box arithmetic, as in the photon pass
 // (c4: 3.58 -> 3.86 G eye rays/s). Register caps of 167 / 161 / 96 were measured: c3 within 1.78-1.94 ms either way.
-template <bool FIRST, bool F32>
+// SPPM (FIRST only): 0 = the PPM camera; CGRT_SPPM_JITTER / CGRT_SPPM_CORNER = the camera of round `sppm_round`, drawn from
+// (seed, PASS_SPPM_EYE, path, round): jitter ux, uy (jitter mode only), then the lens sample; the pixel position w + ux, h + uy enters
+// the expressions of main.cpp:188-198 in place of w, h. A template parameter and a trailing argument, so that the PPM instantiations
+// compile as before (the argument moves no other parameter; PassParams, which every photon kernel reads, is left as it is).
+template <bool FIRST, bool F32, int SPPM = 0>
 __global__ void __launch_bounds__(CGRT_TRACE_BLOCK) eye_bounce_kernel(const __grid_constant__ SceneDev S, const __grid_constant__ PassParams P, int depth,
                                                          RayQueue qin, unsigned int n_in, int y0, RayQueue qout, unsigned int *n_out,
-                                                         double *hp_rec, unsigned int *hp_count, unsigned int hp_cap, Counters *ctr) {
+                                                         double *hp_rec, unsigned int *hp_count, unsigned int hp_cap, Counters *ctr,
+                                                         uint32_t sppm_round) {
     __shared__ TraceShared<CGRT_TRACE_BLOCK> sm;
     unsigned int i = blockIdx.x * blockDim.x + threadIdx.x;
     const bool active = i < n_in;
     d3 o = mk(0, 0, 0), d = mk(0, 0, 1), adj = mk(0, 0, 0);
     uint32_t path = 0, code = 0;
     if (!active) {
-    } else if (FIRST) {
+    } else if (FIRST && SPPM == 0) {
         uint32_t s = i % (uint32_t)P.samples;
         uint32_t pix = i / (uint32_t)P.samples;
         int w = (int)(pix % (uint32_t)P.width), h = y0 + (int)(pix / (uint32_t)P.width);
@@ -127,6 +132,30 @@ __global__ void __launch_bounds__(CGRT_TRACE_BLOCK) eye_bounce_kernel(const __gr
             d3 pof = d * ((P.focus_plane - cam.z) / d.z) + cam;
             Philox g;
             g.init(P.seed, PASS_EYE, (uint64_t)path, 0);
+            o = cam + sample_circle(g, P.lens_radius);
+            d = normalize(pof - o);
+        }
+        adj = mk(1, 1, 1);
+    } else if (FIRST) {
+        uint32_t s = i % (uint32_t)P.samples;
+        uint32_t pix = i / (uint32_t)P.samples;
+        int w = (int)(pix % (uint32_t)P.width), h = y0 + (int)(pix / (uint32_t)P.width);
+        path = ((uint32_t)h * (uint32_t)P.width + (uint32_t)w) * (uint32_t)P.samples + s;
+        code = 0;
+        Philox g;
+        g.init(P.seed, PASS_SPPM_EYE, (uint64_t)path, sppm_round);
+        double xs = (double)w, ys = (double)h;
+        if (SPPM == CGRT_SPPM_JITTER) {
+            xs = (double)w + g.u01();
+            ys = (double)h + g.u01();
+        }
+        d3 cam = mk(P.cam[0], P.cam[1], P.cam[2]);
+        double x = (2.0 * (xs / P.width) - 1) * 10.0;
+        double y = (2.0 * (ys / P.height) - 1) * 10.0 * P.height / P.width;
+        d = normalize(mk(x, y, 0) - cam);
+        o = cam;
+        if (P.use_dof) {
+            d3 pof = d * ((P.focus_plane - cam.z) / d.z) + cam;
             o = cam + sample_circle(g, P.lens_radius);
             d = normalize(pof - o);
         }
@@ -259,6 +288,18 @@ __global__ void hp_gather_sorted_kernel(const double *__restrict__ rec, const ui
     int hh = (int)(hw >> 32), ww = (int)(uint32_t)hw;
     A.hw[2 * (size_t)k] = hh; A.hw[2 * (size_t)k + 1] = ww;
     pixkeys[k] = (uint64_t)hh * (uint64_t)width + (uint64_t)ww;
+}
+
+// SPPM: every visible point of a round takes its pixel's current radius (in place of the r2_init hp_gather_sorted_kernel wrote) and
+// the prefilter records follow it, exactly as round_update_kernel writes them when a radius shrinks.
+__global__ void sppm_visible_radius_kernel(unsigned int n, HpArrays A, const double *__restrict__ pix_r2, int width) {
+    unsigned int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const double r2 = pix_r2[(size_t)A.hw[2 * (size_t)k] * (size_t)width + (size_t)A.hw[2 * (size_t)k + 1]];
+    HpHot hh = A.hot[k];
+    A.hot[k].r2 = r2;
+    A.pre[k] = make_prefilter(hh.px, hh.py, hh.pz, r2);
+    A.pre_n[k].w = prefilter_inner(hh.px, hh.py, hh.pz, r2);
 }
 
 // start[v] = first sorted index whose key is >= v, for v in [0, nvals]; keys ascending.
@@ -1276,6 +1317,44 @@ __global__ void round_update_kernel(unsigned int n, double alpha, HpArrays A, vo
 }
 
 // =================================================================================================================
+// SPPM fold: the U2 rule above per PIXEL. One thread per pixel walks the round's visible points of that pixel in canonical order
+// (pix_perm, as image_gather_kernel does, so the fp64 sums are deterministic), sums their accumulators {dflux, M}, clears them, and
+// updates the pixel's statistics:  g = (n a + a M) / (n a + M);  tau = (tau + dflux) g;  R2 *= g;  n += M.
+// =================================================================================================================
+template <int ACC>
+__global__ void sppm_fold_kernel(unsigned int npix, double alpha, const uint32_t *__restrict__ pix_start, const uint32_t *__restrict__ pix_perm,
+                                 void *__restrict__ acc, double *__restrict__ tau, double *__restrict__ r2, int *__restrict__ cnt) {
+    unsigned int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= npix) return;
+    double dx = 0, dy = 0, dz = 0, m = 0;
+    for (uint32_t j = pix_start[p]; j < pix_start[p + 1]; j++) {
+        uint32_t k = pix_perm[j];
+        if (ACC == 0) {
+            double4 *ap = reinterpret_cast<double4 *>(acc) + k;
+            double4 a = *ap;
+            dx += a.x; dy += a.y; dz += a.z; m += a.w;
+            *ap = make_double4(0, 0, 0, 0);
+        } else {
+            float4 *ap = reinterpret_cast<float4 *>(acc) + k;
+            float4 a = *ap;
+            dx += (double)a.x; dy += (double)a.y; dz += (double)a.z; m += (double)a.w;
+            *ap = make_float4(0, 0, 0, 0);
+        }
+    }
+    if (m > 0) {
+        int c = cnt[p];
+        double na = c * alpha;
+        double g = (na + alpha * m) / (na + m);
+        double *t = tau + 4 * (size_t)p;
+        t[0] = (t[0] + dx) * g;
+        t[1] = (t[1] + dy) * g;
+        t[2] = (t[2] + dz) * g;
+        r2[p] *= g;
+        cnt[p] = c + (int)m;
+    }
+}
+
+// =================================================================================================================
 // The round's exchange over peer memory (one box, NVLink / NVSwitch) fused with the update: no collective library call in the round.
 // Every rank keeps its accumulators in a cudaMalloc block that all ranks have mapped (CUDA IPC between processes, peer access inside one
 // process). After its deposit kernel a rank publishes "round r deposited" in every peer's flag array; on a side stream a one-block
@@ -1411,6 +1490,25 @@ __global__ void image_gather_kernel(int width, int height, double n_emitted, con
     }
     rgb[3 * (size_t)p] = acc.x; rgb[3 * (size_t)p + 1] = acc.y; rgb[3 * (size_t)p + 2] = acc.z;
     if (rgb8) {  // main.cpp:403-411: row i of the PNG is image[height-1-i]
+        int h = p / width, w = p % width;
+        size_t q = (size_t)(height - 1 - h) * width + w;
+        rgb8[3 * q] = (uint8_t)(char)gamma_corr(acc.x);
+        rgb8[3 * q + 1] = (uint8_t)(char)gamma_corr(acc.y);
+        rgb8[3 * q + 2] = (uint8_t)(char)gamma_corr(acc.z);
+    }
+}
+
+// SPPM image: main.cpp:252-258 with the pixel's statistics in place of its hitpoints' — the expression and the tone map / flip of
+// image_gather_kernel, so that a pixel with a single visible point gives PPM's bits.
+__global__ void sppm_image_kernel(int width, int height, double n_emitted, const double *__restrict__ tau, const double *__restrict__ r2,
+                                  double *__restrict__ rgb, uint8_t *__restrict__ rgb8) {
+    unsigned int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= (unsigned int)(width * height)) return;
+    d3 acc = mk(0, 0, 0);
+    d3 fl = mk(tau[4 * (size_t)p], tau[4 * (size_t)p + 1], tau[4 * (size_t)p + 2]);
+    acc = acc + fl * (1.0 / (CGRT_PI * r2[p] * n_emitted));
+    rgb[3 * (size_t)p] = acc.x; rgb[3 * (size_t)p + 1] = acc.y; rgb[3 * (size_t)p + 2] = acc.z;
+    if (rgb8) {
         int h = p / width, w = p % width;
         size_t q = (size_t)(height - 1 - h) * width + w;
         rgb8[3 * q] = (uint8_t)(char)gamma_corr(acc.x);

@@ -1,7 +1,8 @@
 // example_main.cpp — what the reference's main() (main.cpp:268-414) looks like on top of cgrt_host.hpp: build the scene
 // objects on the stack, push raw Object* into a vector, call render(objs) once, tone-map and write the picture.
 //
-//   example_main <scene> <width> <height> <photons> <rounds> <out.ppm> [assets-dir] [gpus] [peer|nccl]
+//   example_main <scene> <width> <height> <photons> <rounds> <out.ppm> [assets-dir] [gpus] [peer|nccl] [off|jitter|corner]
+//   off|jitter|corner: PPM (default) or stochastic PPM with jittered / pixel-corner camera rays (RenderOptions::sppm)
 //   scenes: bunny (main.cpp:293 + chessboard floor), dragon (glass dragon, BASELINE config 3), spheres (main.cpp:288-290)
 //
 // Prints one line: "<hitpoints> <deposits> <fnv1a-64 of the fp64 image> <mean 8-bit level>" — tests/test_gpu_host_cpp.py
@@ -16,7 +17,8 @@ using namespace cgrt_host;
 
 int main(int argc, char **argv) {
     if (argc < 7) {
-        std::fprintf(stderr, "usage: %s <bunny|dragon|spheres> <width> <height> <photons> <rounds> <out.ppm> [assets-dir] [gpus] [peer|nccl]\n", argv[0]);
+        std::fprintf(stderr, "usage: %s <bunny|dragon|spheres> <width> <height> <photons> <rounds> <out.ppm> [assets-dir] [gpus] [peer|nccl] [off|jitter|corner]\n",
+                     argv[0]);
         return 2;
     }
     const std::string scene = argv[1], out = argv[6], assets = argc > 7 ? argv[7] : "cgraytracing_b200/assets";
@@ -25,6 +27,12 @@ int main(int argc, char **argv) {
     opt.num_photon = std::atoi(argv[4]); opt.num_threads = 1; opt.rounds = std::atoi(argv[5]);
     opt.num_gpus = argc > 8 ? std::atoi(argv[8]) : 1;  // > 1: rows and photon ranges split over that many GPUs of this box
     opt.peer_exchange = argc > 9 && std::string(argv[9]) == "peer";  // accumulators exchanged over peer memory instead of ncclAllReduce
+    if (argc > 10) {
+        const std::string mode = argv[10];
+        if (mode == "jitter") opt.sppm = CGRT_SPPM_JITTER;
+        else if (mode == "corner") opt.sppm = CGRT_SPPM_CORNER;
+        else if (mode != "off") { std::fprintf(stderr, "unknown mode %s (off|jitter|corner)\n", mode.c_str()); return 2; }
+    }
     try {
         // floor texture: Texture(tdata, Vec3(0,1,0), Vec3(-21,0,0), 42, 40, false) — main.cpp:320 with ChessBoard.png
         int tw = 0, th = 0;

@@ -173,6 +173,26 @@ int cgrt_round_update(cgrt_ctx *ctx);
  * from cgrt_config, so that every caller normalises a multi-sample image the same way. */
 int cgrt_gather_image(cgrt_ctx *ctx, double n_emitted, double *rgb, uint8_t *rgb8);
 
+/* ---- stochastic progressive photon mapping (SPPM, Hachisuka & Jensen 2009) ------------------------------------------
+ * Every round traces a new eye pass; the statistics (accepted photons n, radius R2, flux tau) live per pixel, shared by all the
+ * visible points one pixel's eye paths create in a round. Round r of eye path (pixel * samples + s) draws its camera from the Philox
+ * stream (seed, pass 3, path, dim = r): jitter ux, uy in [0,1)^2 (JITTER only), then the lens sample when use_dof is set; the ray goes
+ * through the image-plane point of main.cpp:188-198 with (w + ux, h + uy) in place of (w, h). One GPU, per-round update (update_mode 1).
+ *
+ * Per round: cgrt_sppm_begin_round(r) -> cgrt_photon_pass -> cgrt_round_update (folds the round's accumulators into the pixels).
+ * cgrt_gather_image then reads the pixels: tau / (pi R2 n_emitted num_of_samples). cgrt_download_hitpoints / cgrt_download_accum
+ * return the current round's visible points (their r2 is the pixel radius the round used). */
+#define CGRT_SPPM_OFF 0    /* default: PPM, one eye pass for the whole render */
+#define CGRT_SPPM_JITTER 1 /* camera ray through a uniformly jittered point of the pixel, new every round */
+#define CGRT_SPPM_CORNER 2 /* through the pixel corner as main.cpp:188-198; only the lens sample (use_dof) changes per round */
+/* After cgrt_commit_scene, before any eye pass or grid. Allocates the W*H pixel statistics: n = 0, tau = 0, R2 = (200/height)^2. */
+int cgrt_set_sppm(cgrt_ctx *ctx, int mode);
+/* Waits for the previous round's work, drops its visible points and grid, traces the eye pass of `round` over all rows and builds the
+ * grid with every visible point at its pixel's current radius. */
+int cgrt_sppm_begin_round(cgrt_ctx *ctx, uint32_t round);
+/* Pixel statistics, row h = image[h]: tau H*W*3, r2 H*W, n H*W (any may be NULL). */
+int cgrt_sppm_download_pixels(cgrt_ctx *ctx, double *tau, double *r2, int32_t *n);
+
 /* ---- multi-run averaging (average.cpp:19-65), the reference's way of combining separately rendered images ------------ */
 /* Bit-exact 8-bit mode: out[i] = sum over the n images of (img_k[i] / n) in integer arithmetic, exactly what average.cpp does with
  * n = 9 (truncating division before the sum; never overflows a byte). imgs: n host pointers to nbytes bytes each. */
