@@ -29,7 +29,7 @@ ABI_SYMBOLS = [
     "cgrt_download_accum", "cgrt_download_grid", "cgrt_get_counters", "cgrt_get_timings", "cgrt_set_counting", "cgrt_set_profiling", "cgrt_set_culling", "cgrt_set_overlap", "cgrt_average_u8", "cgrt_average_f64",
     "cgrt_check_guards", "cgrt_release_cached_memory", "cgrt_photon_chunk", "cgrt_deposit_record_bytes", "cgrt_trace",
     "cgrt_peer_export", "cgrt_peer_attach", "cgrt_comm_unique_id", "cgrt_comm_init_rank", "cgrt_comm_init_all", "cgrt_comm_destroy", "cgrt_allgather_hitpoints", "cgrt_set_comm",
-    "cgrt_set_sppm", "cgrt_sppm_begin_round", "cgrt_sppm_download_pixels",
+    "cgrt_set_sppm", "cgrt_sppm_begin_round", "cgrt_sppm_download_pixels", "cgrt_sppm_eye_pass",
 ]
 
 
@@ -275,6 +275,11 @@ class Context:
         """Eye pass of round r with its own camera stream, grid at the pixels' current radii."""
         self._ck(self.L.cgrt_sppm_begin_round(self.h, C.c_uint32(r)))
 
+    def sppm_eye_pass(self, r, y0=0, y1=-1):
+        """Eye pass of round r over rows [y0, y1) (y1 < 0: all rows) without the grid: exchange the records with the other ranks, then
+        build_grid. sppm_eye_pass(r, 0, H) + build_grid() is sppm_begin_round(r)."""
+        self._ck(self.L.cgrt_sppm_eye_pass(self.h, C.c_uint32(r), int(y0), int(y1)))
+
     def sppm_download_pixels(self):
         """-> dict tau [H, W, 3], r2 [H, W], n [H, W] (row h = image[h])."""
         H, W = self.cfg.height, self.cfg.width
@@ -391,7 +396,7 @@ class Context:
         ms = (C.c_double * 12)()
         self._ck(self.L.cgrt_get_timings(self.h, ms))
         names = ["eye", "grid", "photon_trace", "photon_deposit", "update", "gather", "deposit_sort", "trace_traverse", "trace_continue",
-                 "trace_emit", "r10", "r11"]
+                 "trace_emit", "allgather", "r11"]
         return {n: ms[i] for i, n in enumerate(names)}
 
 

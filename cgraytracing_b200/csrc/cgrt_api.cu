@@ -271,6 +271,8 @@ struct cgrt_ctx {
     double *pix_r2 = nullptr;   // [W*H]
     int *pix_cnt = nullptr;     // [W*H]
     size_t sppm_cap = 0;
+    bool sppm_traced = false;   // cgrt_sppm_eye_pass has traced this round's visible points and cgrt_build_grid has not run yet
+    size_t gather_cap = 0;      // SPPM: records per rank the all-gather's buffers are sized for (grown with headroom, never shrunk)
 };
 
 namespace {
@@ -748,7 +750,7 @@ void peer_release(cgrt_ctx *ctx) {
 // =================================================================================================================
 extern "C" {
 
-int cgrt_version(void) { return 101; }
+int cgrt_version(void) { return 102; }
 
 void cgrt_default_config(cgrt_config *c) {
     memset(c, 0, sizeof *c);
@@ -1219,7 +1221,7 @@ static int eye_wavefront(cgrt_ctx *ctx, size_t n, int depth0, int r0, bool gener
 static int eye_pass_impl(cgrt_ctx *ctx, int y0, int y1);
 int cgrt_eye_pass(cgrt_ctx *ctx, int y0, int y1) {
     if (!ctx) return CGRT_ERR_INVALID;
-    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is on: cgrt_sppm_begin_round traces the eye pass of every round");
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is on: cgrt_sppm_begin_round / cgrt_sppm_eye_pass trace the eye pass of every round");
     return eye_pass_impl(ctx, y0, y1);
 }
 static int eye_pass_impl(cgrt_ctx *ctx, int y0, int y1) {
@@ -1252,7 +1254,8 @@ int cgrt_export_hitpoints_dev(cgrt_ctx *ctx, void **records_dev, int64_t *count)
 }
 int cgrt_import_hitpoints_dev(cgrt_ctx *ctx, const void *records_dev, int64_t count) {
     if (!ctx || count < 0 || (count > 0 && !records_dev)) return CGRT_ERR_INVALID;
-    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is on: every round makes its own visible points (multi-GPU SPPM is not supported)");
+    if (ctx->sppm && !ctx->sppm_traced)
+        FAIL(CGRT_ERR_INVALID, "SPPM is on: import the round's visible points between cgrt_sppm_eye_pass and cgrt_build_grid");
     if (ctx->grid_built) FAIL(CGRT_ERR_INVALID, "grid already built");
     CK(cudaSetDevice(ctx->device));
     // replaces the current set (the caller passes the all-gathered union, which includes this rank's own records)
@@ -1288,7 +1291,7 @@ static int build_r2_table(cgrt_ctx *ctx, int cap) {
 static int build_grid_impl(cgrt_ctx *ctx);
 int cgrt_build_grid(cgrt_ctx *ctx) {
     if (!ctx) return CGRT_ERR_INVALID;
-    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is on: cgrt_sppm_begin_round builds the grid of every round");
+    if (ctx->sppm && !ctx->sppm_traced) FAIL(CGRT_ERR_INVALID, "SPPM is on: trace the round's visible points first (cgrt_sppm_eye_pass)");
     return build_grid_impl(ctx);
 }
 static int build_grid_impl(cgrt_ctx *ctx) {
@@ -1375,6 +1378,7 @@ static int build_grid_impl(cgrt_ctx *ctx) {
         ctx->hp_cap = 0;
     }
     ctx->grid_built = true;
+    ctx->sppm_traced = false;
     timer.stop();
     return CGRT_OK;
 }
@@ -1635,9 +1639,11 @@ int cgrt_allreduce_accum(cgrt_ctx *ctx, void *nccl_comm) {
 }
 
 
+// The peer block holds the accumulators of a fixed hitpoint set; under SPPM the visible-point count changes every round.
+#define SPPM_NO_PEER "multi-GPU SPPM exchanges over NCCL (cgrt_set_comm); the peer exchange is not supported (its block is sized for a fixed hitpoint count)"
 int cgrt_peer_export(cgrt_ctx *ctx, void *handle128) {
     if (!ctx || !handle128) return CGRT_ERR_INVALID;
-    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, SPPM_NO_PEER);
     if (!ctx->grid_built) FAIL(CGRT_ERR_INVALID, "build the grid first");
     if (ctx->cfg.update_mode == 0) FAIL(CGRT_ERR_INVALID, "the per-photon update is not shard-invariant (one GPU only)");
     if (ctx->peer.block) FAIL(CGRT_ERR_INVALID, "peer block already exported");
@@ -1666,7 +1672,7 @@ int cgrt_peer_export(cgrt_ctx *ctx, void *handle128) {
 
 int cgrt_peer_attach(cgrt_ctx *ctx, int rank, int world, const void *handles) {
     if (!ctx || !handles || world < 1 || world > CGRT_MAX_PEERS || rank < 0 || rank >= world) return CGRT_ERR_INVALID;
-    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
+    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, SPPM_NO_PEER);
     cgrt_ctx::Peer &P = ctx->peer;
     if (!P.block) FAIL(CGRT_ERR_INVALID, "cgrt_peer_export first");
     if (P.attached) FAIL(CGRT_ERR_INVALID, "peers already attached");
@@ -1704,7 +1710,7 @@ int cgrt_peer_attach(cgrt_ctx *ctx, int rank, int world, const void *handles) {
 
 int cgrt_set_comm(cgrt_ctx *ctx, void *nccl_comm, int world) {
     if (!ctx || world < 1) return CGRT_ERR_INVALID;
-    if (nccl_comm && ctx->sppm) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
+    if (nccl_comm && ctx->sppm) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM: attach the communicator before cgrt_set_sppm");
     if (nccl_comm && ctx->cfg.update_mode == 0) FAIL(CGRT_ERR_INVALID, "the per-photon update is not shard-invariant (one GPU only)");
     if (nccl_comm && !nccl_api().ok) FAIL(CGRT_ERR_NCCL, "NCCL is not available: " + nccl_api().why);
     CKS(join_update(ctx));
@@ -1745,12 +1751,13 @@ int cgrt_comm_destroy(void *comm) {
 // order = row order, so the union is in creation order; the grid's sort key makes the order irrelevant anyway).
 int cgrt_allgather_hitpoints(cgrt_ctx *ctx, void *nccl_comm, int world) {
     if (!ctx || world < 1) return CGRT_ERR_INVALID;
-    if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
+    if (ctx->sppm && !ctx->sppm_traced) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM: all-gather between cgrt_sppm_eye_pass and cgrt_build_grid");
     if (ctx->grid_built) FAIL(CGRT_ERR_INVALID, "grid already built");
     if (!nccl_comm || world == 1) return CGRT_OK;
     NcclApi &N = nccl_api();
     if (!N.ok) FAIL(CGRT_ERR_NCCL, "NCCL is not available: " + N.why);
     CK(cudaSetDevice(ctx->device));
+    PhaseTimer timer(ctx, 10);
     long long *d_counts;
     CKS(dalloc(ctx, &d_counts, (size_t)world + 1));
     long long mine = (long long)ctx->hp_count;
@@ -1764,9 +1771,16 @@ int cgrt_allgather_hitpoints(cgrt_ctx *ctx, void *nccl_comm, int world) {
     for (long long c : counts) { cap = c > cap ? c : cap; total += c; }
     if (total >= (1ll << 32)) FAIL(CGRT_ERR_CAPACITY, "more than 2^32 hitpoints");
     const size_t rec_bytes = (size_t)CGRT_HP_RECORD_DOUBLES * sizeof(double);
+    // SPPM gathers every round: the buffers are sized from a capacity that only grows, so that every round asks for the same sizes
+    // (the records still travel in slots of `cap`, the largest tile of this round)
+    size_t slots = (size_t)(cap ? cap : 1);
+    if (ctx->sppm) {
+        if ((size_t)cap > ctx->gather_cap) ctx->gather_cap = (size_t)cap + (size_t)cap / 8 + 4096;
+        slots = ctx->gather_cap;
+    }
     double *send, *recv;
-    CKS(dalloc(ctx, &send, (size_t)(cap ? cap : 1) * CGRT_HP_RECORD_DOUBLES));
-    CKS(dalloc(ctx, &recv, (size_t)(cap ? cap : 1) * CGRT_HP_RECORD_DOUBLES * world));
+    CKS(dalloc(ctx, &send, slots * CGRT_HP_RECORD_DOUBLES));
+    CKS(dalloc(ctx, &recv, slots * CGRT_HP_RECORD_DOUBLES * world));
     if (mine) CK(cudaMemcpyAsync(send, ctx->hp_rec, (size_t)mine * rec_bytes, cudaMemcpyDeviceToDevice, ctx->stream));
     if (cap) {
         r = N.AllGather(send, recv, (size_t)cap * rec_bytes, NCCL_UINT8, nccl_comm, ctx->stream);  // equal-size slots, ranks pad to the largest tile
@@ -1786,6 +1800,7 @@ int cgrt_allgather_hitpoints(cgrt_ctx *ctx, void *nccl_comm, int world) {
     ctx->hp_count = c;
     ctx->launches += 2;
     CKS(dfree(ctx, send)); CKS(dfree(ctx, recv)); CKS(dfree(ctx, d_counts));
+    timer.stop();
     return CGRT_OK;
 }
 
@@ -1798,6 +1813,8 @@ int cgrt_round_update(cgrt_ctx *ctx) {
     unsigned int n = ctx->nhp;
     if (ctx->sppm) {  // fold the round into the pixels, in stream order: the next round's eye pass waits for it anyway
         const unsigned int npix = (unsigned int)((size_t)ctx->P.width * ctx->P.height);
+        // several GPUs: every rank holds the same sorted union, so the accumulators line up and every rank folds the same sums
+        if (ctx->comm) CKS(allreduce_on(ctx, ctx->comm, ctx->stream));
         if (n > 0) {
             if (ctx->cfg.accum_mode == 0)
                 sppm_fold_kernel<0><<<nblk(npix, 256), 256, 0, ctx->stream>>>(npix, ctx->P.alpha, ctx->pix_start, ctx->pix_perm, ctx->acc, ctx->pix_tau, ctx->pix_r2, ctx->pix_cnt);
@@ -1910,7 +1927,7 @@ int cgrt_set_sppm(cgrt_ctx *ctx, int mode) {
     if (!ctx->committed) FAIL(CGRT_ERR_INVALID, "commit the scene first");
     if (ctx->hp_count || ctx->grid_built) FAIL(CGRT_ERR_INVALID, "SPPM must be chosen before any eye pass or grid");
     if (mode && ctx->cfg.update_mode == 0) FAIL(CGRT_ERR_INVALID, "SPPM needs the per-round update (update_mode 1)");
-    if (mode && (ctx->comm || ctx->peer.block)) FAIL(CGRT_ERR_INVALID, "multi-GPU SPPM is not supported");
+    if (mode && ctx->peer.block) FAIL(CGRT_ERR_INVALID, SPPM_NO_PEER);
     CK(cudaSetDevice(ctx->device));
     CKS(dfree(ctx, ctx->pix_tau)); CKS(dfree(ctx, ctx->pix_r2)); CKS(dfree(ctx, ctx->pix_cnt));
     ctx->pix_tau = ctx->pix_r2 = nullptr;
@@ -1930,18 +1947,27 @@ int cgrt_set_sppm(cgrt_ctx *ctx, int mode) {
     return CGRT_OK;
 }
 
-int cgrt_sppm_begin_round(cgrt_ctx *ctx, uint32_t round) {
+int cgrt_sppm_eye_pass(cgrt_ctx *ctx, uint32_t round, int y0, int y1) {
     if (!ctx) return CGRT_ERR_INVALID;
     if (!ctx->sppm) FAIL(CGRT_ERR_INVALID, "SPPM is off: cgrt_set_sppm first");
+    if (y1 < 0) y1 = ctx->P.height;
+    if (y0 < 0 || y1 > ctx->P.height || y0 > y1) FAIL(CGRT_ERR_INVALID, "bad row range");
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->tstream));
     CKS(join_update(ctx));
     CK(cudaStreamSynchronize(ctx->stream));
     if (ctx->grid_built) CKS(release_grid(ctx));
+    ctx->sppm_traced = false;
     ctx->hp_count = 0;
     CK(cudaMemsetAsync(ctx->d_hp_count, 0, sizeof(unsigned int), ctx->stream));
     ctx->sppm_round = round;
-    CKS(eye_pass_impl(ctx, 0, ctx->P.height));
+    if (y1 > y0) CKS(eye_pass_impl(ctx, y0, y1));  // an empty tile (more ranks than rows) contributes no visible points
+    ctx->sppm_traced = true;
+    return CGRT_OK;
+}
+
+int cgrt_sppm_begin_round(cgrt_ctx *ctx, uint32_t round) {
+    CKS(cgrt_sppm_eye_pass(ctx, round, 0, -1));
     return build_grid_impl(ctx);
 }
 

@@ -11,6 +11,14 @@ The reference's render() (main.cpp:169-266) runs its photon loop on 8 OpenMP thr
   round update one all-reduce(sum) of the per-hitpoint accumulators {dflux.xyz, m}, then every rank applies the same
                radius/flux update (main.cpp:119-122 in its per-round form) and stays bit-identical to its peers.
 
+Stochastic PPM (SPPM, `Context.set_sppm`) shards the same way, except that the eye pass and the exchange of its records run every round:
+
+  per round    rank g traces round r's eye pass over its row tile (the camera of eye path `path` in round r draws from
+               (seed, pass 3, path, dim = r), whoever traces it), the tiles are all-gathered and every rank builds the round's grid
+               from the same sorted union, with every visible point at its pixel's current radius; then the photon range as above,
+               one all-reduce of the round's visible-point accumulators, and the per-pixel fold (identical on every rank).
+               The peer-memory exchange is not available under SPPM: its block is sized for a fixed hitpoint count.
+
 `ShardedRenderer` is written against a small engine protocol so that the host logic (ranges, collective order) can be
 exercised on CPU with the gloo backend; the product engine is `GpuEngine` (a `Context` behind the C ABI).
 """
@@ -65,9 +73,12 @@ class GpuEngine:
 
     With `comm` (a handle from make_native_comm) both collectives of the path run INSIDE the library on its own streams
     (cgrt_allgather_hitpoints; the all-reduce is part of cgrt_round_update and overlaps the next round's trace launches).
-    Without it the host framework reduces the accumulator buffer itself (torch.distributed on the library's stream)."""
+    Without it the host framework reduces the accumulator buffer itself (torch.distributed on the library's stream).
 
-    def __init__(self, ctx, device: int, comm=None, world: int = 1, rank: int = 0, peer: bool = False, group=None):
+    `sppm` (CGRT_SPPM_JITTER / CGRT_SPPM_CORNER) turns stochastic PPM on for the committed context, after the communicator is
+    attached (the library requires that order)."""
+
+    def __init__(self, ctx, device: int, comm=None, world: int = 1, rank: int = 0, peer: bool = False, group=None, sppm: int = 0):
         import torch
 
         self.ctx, self.device, self.torch = ctx, device, torch
@@ -76,8 +87,13 @@ class GpuEngine:
         # peer = True: the per-round exchange runs over peer memory inside the library (cgrt_peer_*): no collective call in a round,
         # the reduction is fused with the update and overlaps the next round's trace. The communicator then only serves the eye tiles.
         self.peer = bool(peer) and world > 1
+        self.sppm = int(sppm)
+        if self.sppm and self.peer:
+            raise ValueError("SPPM exchanges over NCCL or torch.distributed; the peer-memory exchange is not supported under SPPM")
         if comm is not None and not self.peer:
             ctx.set_comm(comm, world)
+        if self.sppm:
+            ctx.set_sppm(self.sppm)
         # collectives are enqueued relative to the library's own stream: no host synchronisation between the photon pass, the
         # all-reduce and the update
         self.stream = torch.cuda.ExternalStream(ctx.stream(), device=torch.device("cuda", device))
@@ -90,6 +106,9 @@ class GpuEngine:
 
     def eye_pass(self, y0, y1):
         self.ctx.eye_pass(y0, y1)
+
+    def sppm_eye_pass(self, r, y0, y1):
+        self.ctx.sppm_eye_pass(r, y0, y1)
 
     def export_hitpoints(self):
         ptr, n = self.ctx.export_hitpoints_dev()
@@ -133,22 +152,31 @@ class GpuEngine:
 
 
 class ShardedRenderer:
+    """The host side of a sharded render over an engine. An engine whose `sppm` attribute is non-zero renders stochastic PPM: `eye()`
+    then traces the eye pass of the next round (`sppm_eye_pass(round, y0, y1)`) and `render()` calls it before every round."""
+
     def __init__(self, engine, rank: int = 0, world: int = 1, group=None, shard_eye: bool = True):
         self.e, self.rank, self.world, self.group, self.shard_eye = engine, rank, world, group, shard_eye
+        self.sppm = bool(getattr(engine, "sppm", 0))
         self.rounds_done = 0
         self.emitted = 0
 
-    # -- eye pass + grid
+    # -- eye pass + grid (SPPM: of round `rounds_done`)
+    def _eye_pass(self, y0: int, y1: int):
+        if self.sppm:
+            self.e.sppm_eye_pass(self.rounds_done, y0, y1)  # also on an empty tile: it starts the round's visible-point set
+        elif y1 > y0:
+            self.e.eye_pass(y0, y1)
+
     def eye(self, height: int):
         if self.world == 1 or not self.shard_eye:
-            self.e.eye_pass(0, height)
+            self._eye_pass(0, height)
         else:
             import torch
             import torch.distributed as dist
 
             y0, y1 = row_shard(height, self.rank, self.world)
-            if y1 > y0:
-                self.e.eye_pass(y0, y1)
+            self._eye_pass(y0, y1)
             if getattr(self.e, "native_collectives", False):
                 self.e.allgather_hitpoints()
                 self.e.build_grid()
@@ -189,8 +217,12 @@ class ShardedRenderer:
         self.emitted += photons_per_round
 
     def render(self, height: int, rounds: int, photons_per_round: int) -> np.ndarray:
-        """The whole of render(): eye pass, `rounds` photon rounds, image gather (identical on every rank)."""
-        self.eye(height)
+        """The whole of render(): eye pass, `rounds` photon rounds, image gather (identical on every rank). SPPM: an eye pass before
+        every round."""
+        if not self.sppm:
+            self.eye(height)
         for _ in range(rounds):
+            if self.sppm:
+                self.eye(height)
             self.round(photons_per_round)
         return self.e.gather_image(float(self.emitted))

@@ -317,7 +317,8 @@ struct RenderOptions {
                                          // image rows and photon index ranges are split between them, NCCL (through the C ABI) carries the
                                          // hitpoint records and the per-round accumulators (SURVEY section 8e)
     int sppm = CGRT_SPPM_OFF;            // CGRT_SPPM_JITTER / CGRT_SPPM_CORNER: stochastic PPM, a new eye pass every round and per-pixel statistics
-                                         // (cgrt_set_sppm); one GPU and the per-round update only
+                                         // (cgrt_set_sppm); per-round update only. With num_gpus > 1 every round's eye pass is row-tiled and
+                                         // its records all-gathered over NCCL; peer_exchange is not supported with it
 };
 
 struct Image {
@@ -362,9 +363,13 @@ inline Image render_rank(const std::vector<Object *> &objs, const RenderOptions 
     // main.cpp:185-219: contiguous row tiles, the remainder to the low ranks
     const int base = opt.height / world, rem = opt.height % world;
     const int y0 = rank * base + (rank < rem ? rank : rem), y1 = y0 + base + (rank < rem ? 1 : 0);
-    if (opt.sppm) c.check(cgrt_set_sppm(c.get(), opt.sppm));  // every round traces its own eye pass (cgrt_sppm_begin_round below)
-    else if (y1 > y0) c.check(cgrt_eye_pass(c.get(), y0, y1));
-    if (comm) {
+    if (opt.sppm) {  // every round traces its own eye pass (below); the communicator is attached first, as cgrt_set_sppm requires
+        if (comm) c.check(cgrt_set_comm(c.get(), comm, world));
+        c.check(cgrt_set_sppm(c.get(), opt.sppm));
+    } else if (y1 > y0) {
+        c.check(cgrt_eye_pass(c.get(), y0, y1));
+    }
+    if (comm && !opt.sppm) {
         c.check(cgrt_allgather_hitpoints(c.get(), comm, world));
         if (!hub) c.check(cgrt_set_comm(c.get(), comm, world));  // cgrt_round_update all-reduces the accumulators from now on
     }
@@ -385,7 +390,13 @@ inline Image render_rank(const std::vector<Object *> &objs, const RenderOptions 
         const uint64_t pb = n / world, pr = n % world;  // this rank's index range of the round
         const uint64_t first = done + (uint64_t)rank * pb + ((uint64_t)rank < pr ? (uint64_t)rank : pr);
         const uint64_t mine = pb + ((uint64_t)rank < pr ? 1 : 0);
-        if (opt.sppm) c.check(cgrt_sppm_begin_round(c.get(), (uint32_t)r));
+        if (opt.sppm && comm) {  // this rank's row tile, the union of all tiles, the same grid on every rank
+            c.check(cgrt_sppm_eye_pass(c.get(), (uint32_t)r, y0, y1));
+            c.check(cgrt_allgather_hitpoints(c.get(), comm, world));
+            c.check(cgrt_build_grid(c.get()));
+        } else if (opt.sppm) {
+            c.check(cgrt_sppm_begin_round(c.get(), (uint32_t)r));
+        }
         if (mine) c.check(cgrt_photon_pass(c.get(), first, mine));
         c.check(cgrt_round_update(c.get()));
         done += n;
@@ -402,7 +413,8 @@ inline Image render_rank(const std::vector<Object *> &objs, const RenderOptions 
 
 inline Image render(const std::vector<Object *> &objs, const RenderOptions &opt = RenderOptions(), cgrt_counters *counters = nullptr) {
     const int world = opt.num_gpus < 1 ? 1 : opt.num_gpus;
-    if (opt.sppm && world > 1) throw Error(CGRT_ERR_INVALID, "SPPM runs on one GPU (num_gpus = 1)");
+    if (opt.sppm && world > 1 && opt.peer_exchange)
+        throw Error(CGRT_ERR_INVALID, "SPPM on several GPUs exchanges over NCCL: the peer exchange (peer_exchange = true) is not supported with it");
     if (opt.sppm && opt.per_photon_update) throw Error(CGRT_ERR_INVALID, "SPPM needs the per-round update (per_photon_update = false)");
     if (world == 1) return render_rank(objs, opt, 0, 1, nullptr, counters);
     std::vector<int> devs((size_t)world);
