@@ -195,6 +195,34 @@ class Oracle:
         else:
             self.L.orc_eye_pass(self.h, y0, y1)
 
+    # -- stochastic PPM (Context.set_sppm): per round sppm_begin_round(r), or sppm_eye_pass -> export/import_hitpoints -> build_grid;
+    #    then photon_pass -> round_update (the per-pixel fold) as in PPM
+    def set_sppm(self, mode):
+        """mode 0 off, 1 jitter, 2 corner (include/cgrt.h CGRT_SPPM_*), after set_config; resets the pixel statistics."""
+        r = self.L.orc_set_sppm(self.h, int(mode))
+        if r == -1:
+            raise ValueError(f"SPPM mode must be 0 (off), 1 (jitter) or 2 (corner), got {mode}")
+        if r:
+            raise ValueError("SPPM needs the per-round update (update_mode=1)")
+
+    def sppm_begin_round(self, r, nthreads=1):
+        """A new table and round r's eye pass, every visible point at its pixel's radius."""
+        assert self.L.orc_sppm_begin_round(self.h, C.c_uint32(r), int(nthreads)) == 0
+
+    def sppm_eye_pass(self, r, y0=0, y1=-1, nthreads=1):
+        """Round r's eye pass over rows [y0, y1) into the pending visible points; build_grid inserts them."""
+        assert self.L.orc_sppm_eye_pass(self.h, C.c_uint32(r), int(y0), int(y1), int(nthreads)) == 0
+
+    def build_grid(self):
+        """SPPM: the pending visible points into the round's table in canonical order. PPM: nothing to do."""
+        assert self.L.orc_build_grid(self.h) == 0
+
+    def sppm_download_pixels(self):
+        H, W = self.cfg.height, self.cfg.width
+        o = dict(tau=np.zeros((H, W, 3)), r2=np.zeros((H, W)), n=np.zeros((H, W), np.int32))
+        self.L.orc_sppm_download_pixels(self.h, _p(o["tau"], c_dp), _p(o["r2"], c_dp), _p(o["n"], c_ip))
+        return o
+
     def num_hitpoints(self):
         return int(self.L.orc_num_hitpoints(self.h))
 
@@ -222,7 +250,8 @@ class Oracle:
         self.L.orc_upload_accum(self.h, _p(df, c_dp), _p(mm, c_ip))
 
     def export_hitpoints(self):
-        """-> float64 [n, 12] records in the GPU path's exchange format (cgrt_export_hitpoints_dev)."""
+        """-> float64 [n, 12] records in the GPU path's exchange format (cgrt_export_hitpoints_dev); under SPPM, between sppm_eye_pass and
+        build_grid, of the pending visible points."""
         self.L.orc_export_hitpoints.restype = C.c_int64
         n = self.L.orc_export_hitpoints(self.h, None)
         rec = np.zeros((n, 12))
@@ -232,7 +261,7 @@ class Oracle:
 
     def import_hitpoints(self, rec):
         rec = _d(rec).reshape(-1, 12)
-        self.L.orc_import_hitpoints(self.h, C.c_int64(len(rec)), _p(rec, c_dp))
+        assert self.L.orc_import_hitpoints(self.h, C.c_int64(len(rec)), _p(rec, c_dp)) == 0
 
     def photon_pass(self, first, count, nthreads=1):
         sec = C.c_double(0)
@@ -241,7 +270,7 @@ class Oracle:
         return sec.value
 
     def round_update(self):
-        self.L.orc_round_update(self.h)
+        assert self.L.orc_round_update(self.h) == 0
 
     def gather_image(self, n_emitted):
         img = np.zeros((self.cfg.height, self.cfg.width, 3))

@@ -27,6 +27,8 @@ struct SplitMix {
 };
 int splitmix_cb(void *st) { return ((SplitMix *)st)->next31(); }
 
+const uint32_t PASS_SPPM_EYE = 3;  // Philox pass of the SPPM camera: (seed, 3, path, dim = round)
+
 struct Ctx {
     Renderer R;
     std::vector<std::unique_ptr<Object>> owned;
@@ -41,16 +43,158 @@ struct Ctx {
         for (auto &b : R.htable->hashtable)
             for (auto &hp : b) canon.push_back(&hp);
     }
+
+    // Stochastic PPM (orc_set_sppm): the camera mode (0 off, 1 jitter, 2 corner), the statistics per pixel, and the visible points of a
+    // split round's eye pass, which wait in `pending` (open from orc_sppm_eye_pass until orc_build_grid inserts them).
+    int sppm = 0;
+    std::vector<Vec3> tau;
+    std::vector<double> r2;
+    std::vector<int> n;
+    std::vector<Hitpoint> pending;
+    bool pending_open = false;
+    size_t npix() const { return (size_t)R.cfg.width * R.cfg.height; }
+    size_t pixel(const Hitpoint &hp) const { return (size_t)hp.h * R.cfg.width + hp.w; }
+
+    // The U2 rule per pixel: the round's accumulators summed per pixel in canonical order (buckets ascending, insertion order inside a
+    // bucket), then g = (n a + a M) / (n a + M); tau = (tau + dflux) g; R2 *= g; n += M.
+    void fold() {
+        std::vector<Vec3> d(npix());
+        std::vector<long long> m(npix(), 0);
+        for (auto &b : R.htable->hashtable)
+            for (auto &hp : b) {
+                const size_t p = pixel(hp);
+                d[p] = d[p] + hp.dflux;
+                m[p] += hp.m;
+                hp.dflux = Vec3();
+                hp.m = 0;
+            }
+        for (size_t p = 0; p < npix(); p++)
+            if (m[p] > 0) {
+                double na = n[p] * R.cfg.alpha;
+                double mm = (double)m[p];
+                double g = (na + R.cfg.alpha * mm) / (na + mm);
+                tau[p] = (tau[p] + d[p]) * g;
+                r2[p] *= g;
+                n[p] += (int)m[p];
+            }
+    }
 };
 
 Vec3 v3(const double *p) { return Vec3(p[0], p[1], p[2]); }
 void st3(double *p, const Vec3 &v) { p[0] = v.x; p[1] = v.y; p[2] = v.z; }
 
+void new_table(Renderer &R) {
+    if (R.htable && R.owns_htable) delete R.htable;
+    R.htable = new Hashtable(R.cfg.hashsize, 200.0 / R.cfg.height);
+    R.owns_htable = true;
+}
+
+// Rows [y0, y1) of an eye pass in blocks of 8 rows on `nthreads` OpenMP threads: trace_rows(worker, rng, r0, r1) appends a block's
+// hitpoints to its own sink in creation order. Philox mode only: every path re-keys its own stream, so the result does not depend on
+// who traces a block. Returns the sinks in row order; the workers' eye counters are added to R's.
+template <class TraceRows>
+std::vector<std::vector<Hitpoint>> eye_blocks(Renderer &R, int y0, int y1, int nthreads, TraceRows trace_rows) {
+    const int block = 8, nblocks = y1 > y0 ? (y1 - y0 + block - 1) / block : 0;
+    std::vector<std::vector<Hitpoint>> sinks((size_t)nblocks);
+    std::vector<Counters> part((size_t)nblocks);
+    std::vector<KDCounters> kpart((size_t)nblocks);
+#ifdef _OPENMP
+#pragma omp parallel for schedule(dynamic, 1) num_threads(nthreads > 0 ? nthreads : 1)
+#endif
+    for (int b = 0; b < nblocks; b++) {
+        Renderer w = R.worker();
+        w.sink = &sinks[(size_t)b];
+        Rng rng = Rng::philox(R.cfg.seed, 0, 0, 0);
+        const int r0 = y0 + b * block;
+        trace_rows(w, rng, r0, std::min(r0 + block, y1));
+        part[(size_t)b] = w.ctr;
+        kpart[(size_t)b] = w.kdc;
+    }
+    for (auto &kp : kpart) { R.kdc.node_visits += kp.node_visits; R.kdc.tri_tests += kp.tri_tests; }
+    for (auto &p : part) { R.ctr.eye_segments += p.eye_segments; R.ctr.misses += p.misses; }
+    return sinks;
+}
+
+// The SPPM camera of eye path `path` in round `round`: jitter ux, uy first (jitter mode), then the lens sample; (w + ux, h + uy) in place of
+// (w, h) in the expressions of main.cpp:188-198.
+void sppm_camera(Renderer &W, int mode, uint32_t round, int w, int h, uint64_t path, Rng &rng) {
+    const Config &cfg = W.cfg;
+    Rng g = Rng::philox(cfg.seed, PASS_SPPM_EYE, path, round);
+    double xs = (double)w, ys = (double)h;
+    if (mode == 1) {
+        xs = (double)w + g.u01();
+        ys = (double)h + g.u01();
+    }
+    double x = (2.0 * (xs / cfg.width) - 1) * 10.0;
+    double y = (2.0 * (ys / cfg.height) - 1) * 10.0 * cfg.height / cfg.width;
+    Vec3 dir = (Vec3(x, y, 0) - cfg.camorg).normalize();
+    Vec3 org = cfg.camorg;
+    if (cfg.use_dof) {
+        Vec3 point_on_focus = dir * ((cfg.focus_plane - cfg.camorg.z) / dir.z) + cfg.camorg;
+        org = cfg.camorg + uniform_sampling_circle(g, cfg.lens_radius);
+        dir = (point_on_focus - org).normalize();
+    }
+    W.trace(org, dir, Vec3(), Vec3(1, 1, 1), true, 0, w, h, rng, path, 0);
+}
+
+// A new, empty table and SPPM round `round`'s eye pass over rows [y0, y1); returns the row blocks' visible points (eye_blocks).
+std::vector<std::vector<Hitpoint>> sppm_trace(Ctx *c, uint32_t round, int y0, int y1, int nthreads) {
+    new_table(c->R);
+    c->R.next_seq = 0;
+    c->pending.clear();
+    c->pending_open = false;
+    const int mode = c->sppm;
+    return eye_blocks(c->R, y0, y1, nthreads, [mode, round](Renderer &w, Rng &rng, int r0, int r1) {
+        const Config &g = w.cfg;
+        for (int h = r0; h < r1; h++)
+            for (int x = 0; x < g.width; x++)
+                for (int j = 0; j < g.num_of_samples; j++)
+                    sppm_camera(w, mode, round, x, h, ((uint64_t)h * g.width + x) * (uint64_t)g.num_of_samples + j, rng);
+    });
+}
+
+// The exchange record of the GPU path (cgrt_export_hitpoints_dev, include/cgrt.h), 12 doubles: pos, normal, f, bits(sort key),
+// bits(h << 32 | w), 0. The sort key key << 32 | path*16 + code orders a hitpoint set canonically (buckets ascending, then creation order).
+uint64_t sort_key(const Hashtable &ht, const Hitpoint &hp) {
+    int ix, iy, iz;
+    ht.compute_coord(hp.pos.x, hp.pos.y, hp.pos.z, ix, iy, iz);
+    return ((uint64_t)ht.hash(ix, iy, iz) << 32) | (uint64_t)(uint32_t)(hp.path * 16u + (hp.code & 15u));
+}
+void put_record(const Hashtable &ht, const Hitpoint &hp, double *r) {
+    st3(r, hp.pos); st3(r + 3, hp.normal); st3(r + 6, hp.f);
+    uint64_t sk = sort_key(ht, hp);
+    uint64_t hw = ((uint64_t)(uint32_t)hp.h << 32) | (uint64_t)(uint32_t)hp.w;
+    memcpy(r + 9, &sk, 8); memcpy(r + 10, &hw, 8); r[11] = 0.0;
+}
+// -> the hitpoint of record q (pos, normal, f, pixel, path, code; every other field as constructed) and its sort key.
+Hitpoint get_record(const double *q, uint64_t &sk) {
+    uint64_t hw;
+    memcpy(&sk, q + 9, 8); memcpy(&hw, q + 10, 8);
+    Hitpoint hp;
+    hp.pos = v3(q); hp.normal = v3(q + 3); hp.f = v3(q + 6);
+    hp.h = (int)(hw >> 32); hp.w = (int)(uint32_t)hw;
+    uint32_t lo = (uint32_t)sk;
+    hp.code = lo & 15u; hp.path = lo >> 4;
+    return hp;
+}
+
+// Inserts hitpoints with sort keys `sk` into R's table in canonical order: stable sort on the key, seq = sorted position.
+void insert_sorted(Renderer &R, std::vector<Hitpoint> &hps, const std::vector<uint64_t> &sk) {
+    std::vector<size_t> order(hps.size());
+    for (size_t i = 0; i < order.size(); i++) order[i] = i;
+    std::stable_sort(order.begin(), order.end(), [&sk](size_t a, size_t b) { return sk[a] < sk[b]; });
+    uint32_t seq = 0;
+    for (size_t i : order) {
+        hps[i].seq = seq++;
+        R.htable->insert(hps[i]);
+    }
+}
+
 }  // namespace
 
 extern "C" {
 
-struct orc_config {  // keep in sync with cgraytracing_b200/oracle_binding.py
+struct orc_config {  // keep in sync with OrcConfig in oracle/binding.py
     int32_t width, height, max_depth, num_of_samples, use_dof, consume_dof_rng, hashsize, update_mode, into_rule, pad;
     double alpha, focus_plane, lens_radius;
     double lightorg[3], camorg[3];
@@ -301,45 +445,94 @@ int orc_eye_pass(void *c_, int y0, int y1) {
     c->index();
     return 0;
 }
-// The same eye pass with the rows traced by `nthreads` OpenMP threads (Philox mode only: every path re-keys its own stream, so the
-// result does not depend on who traces it). Each block of rows collects its hitpoints in creation order; the blocks are then inserted
-// in row order with consecutive sequence numbers — exactly the table the sequential loop of main.cpp:185-219 builds.
+// The same eye pass with the rows traced by `nthreads` threads (eye_blocks, Philox mode only). The blocks are inserted in row order with
+// consecutive sequence numbers — exactly the table the sequential loop of main.cpp:185-219 builds.
 int orc_eye_pass_mt(void *c_, int y0, int y1, int nthreads) {
     Ctx *c = (Ctx *)c_;
     if (c->libc_mode || nthreads <= 1) return orc_eye_pass(c_, y0, y1);
-#ifdef _OPENMP
     Renderer &R = c->R;
     if (y1 < 0) y1 = R.cfg.height;
     if (!R.htable) R.htable = new Hashtable(R.cfg.hashsize, 200.0 / R.cfg.height);
-    const int rows = y1 - y0, block = 8, nblocks = (rows + block - 1) / block;
-    std::vector<std::vector<Hitpoint>> sinks((size_t)(nblocks > 0 ? nblocks : 0));
-    std::vector<Counters> part((size_t)nthreads);
-    std::vector<KDCounters> kpart((size_t)nthreads);
-#pragma omp parallel num_threads(nthreads)
-    {
-        Renderer w = R.worker();
-        Rng rng = Rng::philox(R.cfg.seed, 0, 0, 0);
-#pragma omp for schedule(dynamic, 1)
-        for (int b = 0; b < nblocks; b++) {
-            w.sink = &sinks[(size_t)b];
-            const int r0 = y0 + b * block, r1 = (r0 + block < y1) ? r0 + block : y1;
-            w.eye_pass(rng, r0, r1);
-        }
-        part[omp_get_thread_num()] = w.ctr;
-        kpart[omp_get_thread_num()] = w.kdc;
-    }
-    for (auto &kp : kpart) { R.kdc.node_visits += kp.node_visits; R.kdc.tri_tests += kp.tri_tests; }
-    for (auto &p : part) { R.ctr.eye_segments += p.eye_segments; R.ctr.misses += p.misses; }
-    for (auto &sk : sinks) {
+    for (auto &sk : eye_blocks(R, y0, y1, nthreads, [](Renderer &w, Rng &rng, int r0, int r1) { w.eye_pass(rng, r0, r1); })) {
         for (auto &hp : sk) { hp.seq = R.next_seq++; R.htable->insert(hp); }
         std::vector<Hitpoint>().swap(sk);
     }
     c->index();
     return 0;
-#else
-    return orc_eye_pass(c_, y0, y1);
-#endif
 }
+
+// ---- stochastic PPM (include/cgrt.h cgrt_set_sppm): a new eye pass every round, statistics per pixel -------------------------------
+// A round is orc_sppm_begin_round, or the split round of several ranks: orc_sppm_eye_pass (a row tile) -> orc_export_hitpoints /
+// orc_import_hitpoints (the union of the tiles) -> orc_build_grid; then orc_photon_pass -> orc_round_update (the per-pixel fold).
+
+// mode 0 off, 1 jitter, 2 corner; after orc_set_config. Resets the pixel statistics to tau = 0, R2 = (200/height)^2, n = 0.
+// Returns -1 for a bad mode, -2 when the config's update is not per round (U2).
+int orc_set_sppm(void *c_, int mode) {
+    Ctx *c = (Ctx *)c_;
+    if (mode < 0 || mode > 2) return -1;
+    if (mode && c->R.cfg.update != UPDATE_U2_PER_ROUND) return -2;
+    c->sppm = mode;
+    const double r = 200.0 / c->R.cfg.height;
+    c->tau.assign(c->npix(), Vec3());
+    c->r2.assign(c->npix(), r * r);
+    c->n.assign(c->npix(), 0);
+    c->pending.clear();
+    c->pending_open = false;
+    return 0;
+}
+// A new table and round `round`'s eye pass; the visible points inserted in the reference's creation order (h outer, w inner, samples,
+// DFS), every one at its pixel's R2.
+int orc_sppm_begin_round(void *c_, uint32_t round, int nthreads) {
+    Ctx *c = (Ctx *)c_;
+    if (!c->sppm) return -1;
+    Renderer &R = c->R;
+    for (auto &sk : sppm_trace(c, round, 0, R.cfg.height, nthreads))
+        for (auto &hp : sk) {
+            hp.seq = R.next_seq++;
+            hp.r2 = c->r2[c->pixel(hp)];
+            R.htable->insert(hp);
+        }
+    c->index();
+    return 0;
+}
+// A new, empty table and round `round`'s eye pass over rows [y0, y1) (y1 < 0: to the last row) into the pending visible points, in
+// creation order. Nothing is inserted until orc_build_grid.
+int orc_sppm_eye_pass(void *c_, uint32_t round, int y0, int y1, int nthreads) {
+    Ctx *c = (Ctx *)c_;
+    if (y1 < 0) y1 = c->R.cfg.height;
+    if (!c->sppm || y0 < 0 || y1 > c->R.cfg.height || y0 > y1) return -1;
+    for (auto &sk : sppm_trace(c, round, y0, y1, nthreads)) c->pending.insert(c->pending.end(), sk.begin(), sk.end());
+    c->pending_open = true;
+    c->index();
+    return 0;
+}
+// SPPM: the pending visible points into the round's table in canonical order, every one at its pixel's R2. PPM: nothing to do, the eye
+// pass filled the table.
+int orc_build_grid(void *c_) {
+    Ctx *c = (Ctx *)c_;
+    if (!c->sppm) return 0;
+    if (!c->pending_open) return -1;
+    std::vector<uint64_t> sk(c->pending.size());
+    for (size_t i = 0; i < sk.size(); i++) {
+        c->pending[i].r2 = c->r2[c->pixel(c->pending[i])];
+        sk[i] = sort_key(*c->R.htable, c->pending[i]);
+    }
+    insert_sorted(c->R, c->pending, sk);
+    c->pending.clear();
+    c->pending_open = false;
+    c->index();
+    return 0;
+}
+int orc_sppm_download_pixels(void *c_, double *tau, double *r2, int32_t *n) {
+    Ctx *c = (Ctx *)c_;
+    for (size_t p = 0; p < c->npix(); p++) {
+        if (tau) st3(tau + 3 * p, c->tau[p]);
+        if (r2) r2[p] = c->r2[p];
+        if (n) n[p] = c->n[p];
+    }
+    return 0;
+}
+
 int64_t orc_num_hitpoints(void *c_) { Ctx *c = (Ctx *)c_; c->index(); return (int64_t)c->canon.size(); }
 
 // Canonical order (buckets ascending, insertion order inside a bucket; main.cpp:252-254). Any pointer may be NULL.
@@ -379,8 +572,7 @@ int orc_download_accum(void *c_, double *dflux, int32_t *m) {
 }
 
 // Test plumbing for the 2-rank (gloo) sharding tests: write back all-reduced accumulators, and move hitpoint sets
-// between oracle instances in the GPU path's record format (12 doubles: pos, normal, f, bits(key<<32 | path*16+code),
-// bits(h<<32 | w), 0 — cgrt_export_hitpoints_dev, include/cgrt.h).
+// between oracle instances in the GPU path's record format (put_record / get_record).
 int orc_upload_accum(void *c_, const double *dflux, const int32_t *m) {
     Ctx *c = (Ctx *)c_;
     c->index();
@@ -391,44 +583,33 @@ int orc_upload_accum(void *c_, const double *dflux, const int32_t *m) {
     }
     return 0;
 }
+// The table in canonical order; under SPPM, while a split round's eye pass is open, its pending visible points. rec12 NULL: count only.
 int64_t orc_export_hitpoints(void *c_, double *rec12) {
     Ctx *c = (Ctx *)c_;
-    c->index();
-    for (size_t i = 0; rec12 && i < c->canon.size(); i++) {
-        const Hitpoint &hp = *c->canon[i];
-        double *r = rec12 + 12 * i;
-        st3(r, hp.pos); st3(r + 3, hp.normal); st3(r + 6, hp.f);
-        int ix, iy, iz;
-        c->R.htable->compute_coord(hp.pos.x, hp.pos.y, hp.pos.z, ix, iy, iz);
-        uint64_t sk = ((uint64_t)c->R.htable->hash(ix, iy, iz) << 32) | (uint64_t)(uint32_t)(hp.path * 16u + (hp.code & 15u));
-        uint64_t hw = ((uint64_t)(uint32_t)hp.h << 32) | (uint64_t)(uint32_t)hp.w;
-        memcpy(r + 9, &sk, 8); memcpy(r + 10, &hw, 8); r[11] = 0.0;
+    if (c->pending_open) {
+        for (size_t i = 0; rec12 && i < c->pending.size(); i++) put_record(*c->R.htable, c->pending[i], rec12 + 12 * i);
+        return (int64_t)c->pending.size();
     }
+    c->index();
+    for (size_t i = 0; rec12 && i < c->canon.size(); i++) put_record(*c->R.htable, *c->canon[i], rec12 + 12 * i);
     return (int64_t)c->canon.size();
 }
-// Replaces the hitpoint set: records in any order are inserted in canonical order (stable sort on the 64-bit sort key).
+// Replaces the hitpoint set: records in any order are inserted in canonical order (stable sort on the 64-bit sort key). Under SPPM
+// they replace the pending visible points of the open eye pass (-1 when none is open), which orc_build_grid inserts.
 int orc_import_hitpoints(void *c_, int64_t n, const double *rec12) {
     Ctx *c = (Ctx *)c_;
-    const Config &g = c->R.cfg;
-    double r = 200.0 / g.height;
-    if (c->R.htable && c->R.owns_htable) delete c->R.htable;
-    c->R.htable = new Hashtable(g.hashsize, r);
-    c->R.owns_htable = true;
-    std::vector<std::pair<uint64_t, int64_t>> order((size_t)n);
-    for (int64_t i = 0; i < n; i++) { uint64_t sk; memcpy(&sk, rec12 + 12 * i + 9, 8); order[(size_t)i] = {sk, i}; }
-    std::stable_sort(order.begin(), order.end(), [](const std::pair<uint64_t, int64_t> &a, const std::pair<uint64_t, int64_t> &b) { return a.first < b.first; });
-    uint32_t seq = 0;
-    for (auto &o : order) {
-        const double *q = rec12 + 12 * o.second;
-        uint64_t hw; memcpy(&hw, q + 10, 8);
-        Hitpoint hp;
-        hp.pos = v3(q); hp.normal = v3(q + 3); hp.f = v3(q + 6);
-        hp.flux = Vec3(0, 0, 0); hp.r2 = r * r; hp.n = 0;
-        hp.h = (int)(hw >> 32); hp.w = (int)(uint32_t)hw;
-        uint32_t lo = (uint32_t)o.first;
-        hp.code = lo & 15u; hp.path = lo >> 4; hp.seq = seq++;
-        c->R.htable->insert(hp);
+    std::vector<Hitpoint> hps((size_t)n);
+    std::vector<uint64_t> sk((size_t)n);
+    for (int64_t i = 0; i < n; i++) hps[(size_t)i] = get_record(rec12 + 12 * i, sk[(size_t)i]);
+    if (c->sppm) {
+        if (!c->pending_open) return -1;
+        c->pending.swap(hps);
+        return 0;
     }
+    const double r = 200.0 / c->R.cfg.height;
+    new_table(c->R);
+    for (auto &hp : hps) hp.r2 = r * r;
+    insert_sorted(c->R, hps, sk);
     c->index();
     return 0;
 }
@@ -468,13 +649,23 @@ int orc_photon_pass(void *c_, uint64_t first, uint64_t count, int nthreads, doub
     if (seconds) *seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     return 0;
 }
-int orc_round_update(void *c_) { ((Ctx *)c_)->R.round_update(); return 0; }
+// U2 per hitpoint; under SPPM the per-pixel fold (Ctx::fold).
+int orc_round_update(void *c_) {
+    Ctx *c = (Ctx *)c_;
+    if (!c->sppm) c->R.round_update();
+    else if (c->R.htable) c->fold();
+    else return -1;
+    return 0;
+}
 
 int orc_gather_image(void *c_, double n_emitted, double *rgb) {
     Ctx *c = (Ctx *)c_;
     std::vector<Vec3> img;
     // n_emitted = num_photon*num_threads; the num_of_samples factor of main.cpp:256 comes from the config (same convention as cgrt_gather_image)
-    c->R.gather_image(n_emitted * (double)c->R.cfg.num_of_samples, img);
+    const double ne = n_emitted * (double)c->R.cfg.num_of_samples;
+    if (!c->sppm) c->R.gather_image(ne, img);
+    else  // main.cpp:252-258 with the pixel's statistics
+        for (size_t p = 0; p < c->npix(); p++) img.push_back(Vec3() + c->tau[p] * (1.0 / (PI * c->r2[p] * ne)));
     for (size_t i = 0; i < img.size(); i++) st3(rgb + 3 * i, img[i]);
     return 0;
 }

@@ -6,12 +6,12 @@ import socket
 
 import numpy as np
 import pytest
-import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
 from cgraytracing_b200 import RenderConfig, preset
 from cgraytracing_b200.distributed import ShardedRenderer, photon_shard, row_shard, split_range
+from tests.util import OracleEngine
 
 W, H, ROUNDS, PHOTONS = 64, 48, 2, 5001  # odd photon count: the remainder path
 
@@ -28,42 +28,6 @@ def test_split_range_is_disjoint_and_covering():
     assert [row_shard(5, r, 8)[1] - row_shard(5, r, 8)[0] for r in range(8)] == [1, 1, 1, 1, 1, 0, 0, 0]
     with pytest.raises(ValueError):
         split_range(0, 10, 2, 2)
-
-
-class OracleEngine:
-    def __init__(self, scene, cfg):
-        from oracle import binding as ob
-
-        self.o = ob.Oracle(scene, cfg)
-
-    def eye_pass(self, y0, y1):
-        self.o.eye_pass(y0, y1)
-
-    def export_hitpoints(self):
-        return torch.from_numpy(self.o.export_hitpoints())
-
-    def import_hitpoints(self, rec):
-        self.o.import_hitpoints(rec.numpy())
-
-    def build_grid(self):
-        pass
-
-    def photon_pass(self, first, count):
-        self.o.photon_pass(first, count)
-
-    def accum_tensor(self):
-        df, m = self.o.download_accum()
-        return torch.from_numpy(np.concatenate([df, m[:, None].astype(np.float64)], 1).copy())
-
-    def accum_commit(self, t):
-        a = t.numpy()
-        self.o.upload_accum(a[:, :3], a[:, 3].astype(np.int32))
-
-    def round_update(self):
-        self.o.round_update()
-
-    def gather_image(self, n):
-        return self.o.gather_image(n)
 
 
 def _worker(rank, world, port, out):

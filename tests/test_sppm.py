@@ -1,7 +1,7 @@
 """Stochastic progressive photon mapping (SPPM, include/cgrt.h cgrt_set_sppm): a new eye pass every round, statistics per pixel.
 
-The CPU reference is tests/sppm_oracle.cpp: the unchanged PPM oracle (oracle/ppm_oracle.hpp) driven round by round with the SPPM camera,
-per-pixel statistics and fold.
+The CPU reference is the oracle's SPPM mode (oracle/oracle_capi.cpp, orc_set_sppm): the unchanged PPM oracle (oracle/ppm_oracle.hpp) driven
+round by round with the SPPM camera, per-pixel statistics and fold.
 CPU: corner mode on walls_only (one visible point per pixel) is the PPM oracle's estimator itself, bit for bit; the jittered camera stream
 is deterministic per round, different between rounds and stays inside the pixel.
 GPU: every round's visible points and the final pixel counts / radii equal the reference's bit for bit; corner mode equals the PPM path;
@@ -13,7 +13,6 @@ import sys
 import numpy as np
 import pytest
 
-from tests.sppm_oracle import SppmOracle
 from tests.util import assert_flux_close
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -27,14 +26,14 @@ def pixel_index(hw, width):
 
 def oracle_rounds(ob, scene, cfg, mode, rounds, nph, threads=1):
     """mode 0: the PPM oracle (one eye pass, per-hitpoint U2 updates); else the SPPM reference with that camera mode."""
+    o = ob.Oracle(scene, cfg)
     if mode:
-        o = SppmOracle(scene, cfg, mode)
+        o.set_sppm(mode)
     else:
-        o = ob.Oracle(scene, cfg)
         o.eye_pass(nthreads=threads)
     for r in range(rounds):
         if mode:
-            o.begin_round(r, threads)
+            o.sppm_begin_round(r, threads)
         o.photon_pass(r * nph, nph, threads)
         o.round_update()
     return o
@@ -52,7 +51,7 @@ def test_corner_mode_on_walls_is_ppm_bit_for_bit(oracle_lib):
     ppm = oracle_rounds(oracle_lib, s, cfg, 0, R, N)
     spp = oracle_rounds(oracle_lib, s, cfg, CORNER, R, N)
     hp = ppm.download_hitpoints()
-    px = spp.download_pixels()
+    px = spp.sppm_download_pixels()
     idx = pixel_index(hp["hw"], cfg.width)
     assert len(idx) == cfg.width * cfg.height and len(np.unique(idx)) == len(idx)  # exactly one visible point per pixel
     assert hp["n"].sum() > 0
@@ -71,12 +70,13 @@ def test_jitter_stream_is_per_round_and_inside_the_pixel(oracle_lib):
     ob = oracle_lib
     s = preset("walls_only")
     cfg = RenderConfig(width=40, height=30, update_mode=1, into_rule=1)
-    o = SppmOracle(s, cfg, JITTER)
-    o.begin_round(7)
+    o = ob.Oracle(s, cfg)
+    o.set_sppm(JITTER)
+    o.sppm_begin_round(7)
     a = o.download_hitpoints()
-    o.begin_round(7)
+    o.sppm_begin_round(7)
     b = o.download_hitpoints()
-    o.begin_round(8)
+    o.sppm_begin_round(8)
     c = o.download_hitpoints()
     for k in ("pos", "key", "hw", "r2"):
         assert np.array_equal(a[k], b[k]), k  # the same round traced twice: identical visible points
@@ -124,19 +124,20 @@ PARITY = [("c1_spheres", None, dict(width=96, height=72)),
 @pytest.mark.parametrize("accum", [0, 1])
 @pytest.mark.parametrize("mode", [JITTER, CORNER])
 @pytest.mark.parametrize("name,max_tris,kw", PARITY, ids=[p[0] for p in PARITY])
-def test_rounds_match_oracle(gpu, name, max_tris, kw, mode, accum):
-    """Five rounds against tests/sppm_oracle.cpp: each round's visible points (pos, key, r2, pixel) bit-equal, and the round's accepted
+def test_rounds_match_oracle(gpu, oracle_lib, name, max_tris, kw, mode, accum):
+    """Five rounds against the oracle's SPPM mode: each round's visible points (pos, key, r2, pixel) bit-equal, and the round's accepted
     photons per visible point equal; final pixel n and R2 bit-equal; tau and the image within the accumulator type's bounds
     (tests/util.assert_flux_close)."""
     R, N = 5, 20000
     s = gpu.preset(name, max_tris=max_tris)
     cfg = gpu.RenderConfig(update_mode=1, into_rule=1, **kw)
-    o = SppmOracle(s, cfg, mode)
+    o = oracle_lib.Oracle(s, cfg)
+    o.set_sppm(mode)
     th = max(1, len(os.sched_getaffinity(0)))
     with gpu_sppm(gpu, s, cfg, mode, accum) as g:
         for r in range(R):
             g.sppm_begin_round(r)
-            o.begin_round(r, th)
+            o.sppm_begin_round(r, th)
             a, b = g.download_hitpoints(), o.download_hitpoints()
             assert len(a["pos"]) == len(b["pos"]) > 0, r
             for k in ("pos", "key", "r2", "hw"):
@@ -144,10 +145,10 @@ def test_rounds_match_oracle(gpu, name, max_tris, kw, mode, accum):
             g.photon_pass(r * N, N)
             o.photon_pass(r * N, N, th)
             _, gm = g.download_accum()
-            assert np.array_equal(gm.astype(np.int64), o.download_hitpoints()["m"].astype(np.int64)), r
+            assert np.array_equal(gm.astype(np.int64), o.download_accum()[1].astype(np.int64)), r
             g.round_update()
             o.round_update()
-        pg, po = g.sppm_download_pixels(), o.download_pixels()
+        pg, po = g.sppm_download_pixels(), o.sppm_download_pixels()
         assert po["n"].sum() > 0
         assert np.array_equal(pg["n"], po["n"])
         assert np.array_equal(pg["r2"], po["r2"])

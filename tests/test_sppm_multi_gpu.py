@@ -2,8 +2,8 @@
 the same grid built from the union on every rank, disjoint photon ranges, one all-reduce of the round's accumulators before the per-pixel fold
 (include/cgrt.h, cgrt_sppm_eye_pass).
 
-CPU: cgraytracing_b200.distributed.ShardedRenderer in SPPM mode over the CPU reference with the split round (tests/sppm_split_oracle.cpp)
-with gloo, world 2, against one rank of the reference (tests/sppm_oracle.cpp).
+CPU: cgraytracing_b200.distributed.ShardedRenderer in SPPM mode over the oracle's split round (sppm_eye_pass, record exchange, build_grid)
+with gloo, world 2, against the oracle's one-call round (sppm_begin_round).
 One GPU: the split round equals the one-call round; two contexts of one device emulate two ranks (tests/sppm_two_ranks.py) and equal one
 context, also with fenced buffers; the refusals of the split round.
 Two GPUs: torch.distributed worker (tests/sppm_worker.py) with the library's communicator and with host-driven collectives, and the C++
@@ -16,8 +16,8 @@ import sys
 import numpy as np
 import pytest
 
-from tests.sppm_oracle import SppmOracle
-from tests.sppm_split_oracle import SppmSplitOracle
+from oracle import binding as ob
+from tests.util import OracleEngine
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 JITTER, CORNER = 1, 2
@@ -26,48 +26,19 @@ JITTER, CORNER = 1, 2
 # ---------------------------------------------------------------------------------------------------------------------
 # CPU: the host logic of the sharded SPPM round over the reference, world 2 (gloo)
 # ---------------------------------------------------------------------------------------------------------------------
-class SppmOracleEngine:
-    """The engine protocol of ShardedRenderer over the SPPM reference; keeps every round's union of visible points."""
+VP = ("pos", "key", "hw", "r2")
 
-    def __init__(self, scene, cfg, mode):
-        self.o = SppmSplitOracle(scene, cfg, mode)
-        self.sppm = mode
+
+class UnionEngine(OracleEngine):
+    """OracleEngine that keeps every round's union of visible points."""
+
+    def __init__(self, *args):
+        super().__init__(*args)
         self.unions = []
 
-    def sppm_eye_pass(self, r, y0, y1):
-        self.o.eye_rows(r, y0, y1)
-
-    def export_hitpoints(self):
-        import torch
-
-        return torch.from_numpy(self.o.export_pending())
-
-    def import_hitpoints(self, rec):
-        self.o.import_pending(rec.numpy())
-
     def build_grid(self):
-        self.o.build_table()
-        hp = self.o.download_hitpoints()
-        self.unions.append({k: hp[k] for k in ("pos", "key", "hw", "r2")})
-
-    def photon_pass(self, first, count):
-        self.o.photon_pass(first, count)
-
-    def accum_tensor(self):
-        import torch
-
-        hp = self.o.download_hitpoints()
-        return torch.from_numpy(np.concatenate([hp["dflux"], hp["m"][:, None].astype(np.float64)], 1).copy())
-
-    def accum_commit(self, t):
-        a = t.numpy()
-        self.o.upload_accum(a[:, :3], a[:, 3].astype(np.int32))
-
-    def round_update(self):
-        self.o.round_update()
-
-    def gather_image(self, n):
-        return self.o.gather_image(n)
+        super().build_grid()
+        self.unions.append(self.o.download_hitpoints(VP))
 
 
 W, H, ROUNDS, PHOTONS = 64, 48, 3, 5001  # odd photon count: the remainder path
@@ -83,9 +54,9 @@ def _gloo_worker(rank, world, port, out, mode):
     dist.init_process_group("gloo", rank=rank, world_size=world)
     try:
         cfg = RenderConfig(width=W, height=H, update_mode=1, into_rule=1)
-        eng = SppmOracleEngine(preset("c2_bunny_chess"), cfg, mode)
+        eng = UnionEngine(preset("c2_bunny_chess"), cfg, mode)
         img = ShardedRenderer(eng, rank, world).render(H, ROUNDS, PHOTONS)
-        px = eng.o.download_pixels()
+        px = eng.o.sppm_download_pixels()
         rounds = {f"{k}{r}": u[k] for r, u in enumerate(eng.unions) for k in u}
         np.savez(os.path.join(out, f"rank{rank}.npz"), img=img, n=px["n"], r2=px["r2"], tau=px["tau"], **rounds)
     finally:
@@ -107,16 +78,17 @@ def test_two_ranks_equal_one_rank(tmp_path, mode):
         assert np.array_equal(a[k], b[k]), k
     # one rank: the reference's one-call round (eye pass and table together)
     cfg = RenderConfig(width=W, height=H, update_mode=1, into_rule=1)
-    o = SppmOracle(preset("c2_bunny_chess"), cfg, mode)
+    o = ob.Oracle(preset("c2_bunny_chess"), cfg)
+    o.set_sppm(mode)
     for r in range(ROUNDS):
-        o.begin_round(r)
+        o.sppm_begin_round(r)
         hp = o.download_hitpoints()
         assert len(hp["pos"]) > 0
-        for k in ("pos", "key", "hw", "r2"):  # the union of the tiles is the round's visible-point set, in canonical order
+        for k in VP:  # the union of the tiles is the round's visible-point set, in canonical order
             assert np.array_equal(a[f"{k}{r}"], hp[k]), (r, k)
         o.photon_pass(r * PHOTONS, PHOTONS)
         o.round_update()
-    px = o.download_pixels()
+    px = o.sppm_download_pixels()
     assert np.array_equal(a["n"], px["n"]) and a["n"].sum() > 1000  # integer counts, hence the radii: exact
     assert np.array_equal(a["r2"], px["r2"])
     # sums differ only by fp64 association (two partial sums added by the all-reduce)
@@ -125,21 +97,23 @@ def test_two_ranks_equal_one_rank(tmp_path, mode):
 
 
 def test_pending_records_round_trip():
-    """Export -> import of the pending visible points, then the table: the same round as the one-call begin_round."""
+    """Export -> import of the pending visible points, then the table: the same round as the one-call sppm_begin_round."""
     from cgraytracing_b200 import RenderConfig, preset
 
     cfg = RenderConfig(width=40, height=30, update_mode=1, into_rule=1)
     s = preset("c2_bunny_chess")
-    a, b = SppmOracle(s, cfg, JITTER), SppmSplitOracle(s, cfg, JITTER)
-    a.begin_round(5)
+    a, b = ob.Oracle(s, cfg), ob.Oracle(s, cfg)
+    a.set_sppm(JITTER)
+    b.set_sppm(JITTER)
+    a.sppm_begin_round(5)
     lo, hi = 0, cfg.height
-    b.eye_rows(5, 17, hi)  # the tiles in reverse order: the table's sort makes the order irrelevant
-    rec = b.export_pending()
-    b.eye_rows(5, lo, 17)
-    b.import_pending(np.concatenate([rec, b.export_pending()], 0))
-    b.build_table()
+    b.sppm_eye_pass(5, 17, hi)  # the tiles in reverse order: the table's sort makes the order irrelevant
+    rec = b.export_hitpoints()
+    b.sppm_eye_pass(5, lo, 17)
+    b.import_hitpoints(np.concatenate([rec, b.export_hitpoints()], 0))
+    b.build_grid()
     ha, hb = a.download_hitpoints(), b.download_hitpoints()
-    for k in ("pos", "key", "hw", "r2"):
+    for k in VP:
         assert np.array_equal(ha[k], hb[k]), k
     assert len(ha["pos"]) >= cfg.width * cfg.height // 2
 
@@ -151,9 +125,6 @@ def _ctx(gpu, scene, cfg, mode, accum):
     from tests.sppm_two_ranks import sppm_context
 
     return sppm_context(gpu, scene, cfg, mode, accum)
-
-
-VP = ("pos", "key", "hw", "r2")
 
 
 def _flux_close(got, ref, n, accum):

@@ -42,3 +42,52 @@ def assert_flux_close(df, odf, om, accum):
         assert np.all(err <= bound), float((err / bound).max())
         pos = odf > 0
         assert np.median(err[pos] / odf[pos]) < 5e-7  # and typically a few ulp
+
+
+class OracleEngine:
+    """The engine protocol of cgraytracing_b200.distributed.ShardedRenderer over the CPU oracle. `sppm` (the oracle's SPPM mode, 0: PPM)
+    tells ShardedRenderer whether to call eye_pass once or sppm_eye_pass every round."""
+
+    def __init__(self, scene, cfg, sppm=0):
+        from oracle import binding as ob
+
+        self.o = ob.Oracle(scene, cfg)
+        self.sppm = sppm
+        if sppm:
+            self.o.set_sppm(sppm)
+
+    def eye_pass(self, y0, y1):
+        self.o.eye_pass(y0, y1)
+
+    def sppm_eye_pass(self, r, y0, y1):
+        self.o.sppm_eye_pass(r, y0, y1)
+
+    def export_hitpoints(self):
+        import torch
+
+        return torch.from_numpy(self.o.export_hitpoints())
+
+    def import_hitpoints(self, rec):
+        self.o.import_hitpoints(rec.numpy())
+
+    def build_grid(self):
+        self.o.build_grid()
+
+    def photon_pass(self, first, count):
+        self.o.photon_pass(first, count)
+
+    def accum_tensor(self):
+        import torch
+
+        df, m = self.o.download_accum()
+        return torch.from_numpy(np.concatenate([df, m[:, None].astype(np.float64)], 1).copy())
+
+    def accum_commit(self, t):
+        a = t.numpy()
+        self.o.upload_accum(a[:, :3], a[:, 3].astype(np.int32))
+
+    def round_update(self):
+        self.o.round_update()
+
+    def gather_image(self, n):
+        return self.o.gather_image(n)
