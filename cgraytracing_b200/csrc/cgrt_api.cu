@@ -235,7 +235,7 @@ struct cgrt_ctx {
         bool ipc[CGRT_MAX_PEERS] = {};      // opened with cudaIpcOpenMemHandle (to be closed)
     } peer;
     int sm_count = 148;
-    int overlap = 0;  // measured on c3: the two halves slow each other down by more than they overlap (25.3 vs 24.2 ms per round)
+    int overlap = 0;  // cgrt_set_overlap: off by default; its measurements are in DESIGN.md section 4
     // resident-grid sizes of the persistent photon kernels (SMs x occupancy), so that static striding leaves no tail of late blocks
     unsigned int grid_first = 592, grid_cont = 592, trav_grid = 0;
     std::vector<std::pair<cudaEvent_t, int>> prof_marks;

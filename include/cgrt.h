@@ -227,8 +227,8 @@ int cgrt_get_counters(cgrt_ctx *ctx, cgrt_counters *out);
 int cgrt_set_counting(cgrt_ctx *ctx, int on);
 /* on != 0: cgrt_photon_pass traces on a second internal stream into double-buffered deposit tables, so the trace of one chunk (or
  * of the next round) overlaps the sort + deposit of the previous one. Everything a caller can observe stays ordered on the stream
- * cgrt_get_stream returns. Off by default: on one B200 both halves are bound by the same SM issue slots and registers and slow each
- * other down by more than they overlap (25.3 vs 24.2 ms per 16 Mi-photon round); it pays when a slow collective sits between rounds. */
+ * cgrt_get_stream returns. Off by default. With the r02 kernels on one B200 at 1000 W it is 1.2-3.3 % faster per round on c1-c4
+ * (c3: 17.07 vs 17.33 ms, DESIGN.md section 4); the earlier 25.3 vs 24.2 ms against it predates those kernels. */
 int cgrt_set_overlap(cgrt_ctx *ctx, int on);
 /* on != 0 (default): photon hits whose cell is farther than 2 cells from every hitpoint are dropped before the gather — they
  * cannot pass the distance test of main.cpp:116 — and are not counted in counters.candidates. Deposits, accepted-photon
