@@ -174,6 +174,7 @@ struct cgrt_ctx {
     std::vector<HostTexture> textures;
     std::vector<HostObject> objects;
     bool committed = false;
+    bool bvh_f32 = true;  // every tree within CGRT_F32_BOUND (set by cgrt_commit_scene): the traversal without fp64 box arithmetic
     SceneDev S;
     BvhBuild bvh_src[CGRT_MAX_BVH];
     int obj_bvh[CGRT_MAX_OBJECTS];
@@ -237,9 +238,7 @@ struct cgrt_ctx {
     int sm_count = 148;
     int overlap = 0;  // cgrt_set_overlap: off by default; its measurements are in DESIGN.md section 4
     // resident-grid sizes of the persistent photon kernels (SMs x occupancy), so that static striding leaves no tail of late blocks
-    unsigned int grid_first = 592, grid_cont = 592, trav_grid = 0;
-    std::vector<std::pair<cudaEvent_t, int>> prof_marks;
-    std::vector<cudaEvent_t> timeline;  // dev: CGRT_TIMELINE=1 records (trace begin, trace end, deposit begin, deposit end) per chunk
+    unsigned int grid_first = 592, grid_cont = 592;
     PhotonState *pq[2] = {nullptr, nullptr};
     size_t pq_cap = 0;
     uint32_t *reach = nullptr;        // reach bitmap (cells within 2 cells of a hitpoint), built with the grid
@@ -666,9 +665,9 @@ int ensure_hp_capacity(cgrt_ctx *ctx, size_t need) {
     while (cap < need) cap = cap + cap / 2 + 1024;
     if (cap >= (1ull << 32)) FAIL(CGRT_ERR_CAPACITY, "more than 2^32 hitpoints");
     double *nrec;
-    CKS(dalloc(ctx, &nrec, cap * 12));
+    CKS(dalloc(ctx, &nrec, cap * CGRT_HP_RECORD_DOUBLES));
     if (ctx->hp_rec) {
-        CK(cudaMemcpyAsync(nrec, ctx->hp_rec, (size_t)ctx->hp_count * 12 * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(nrec, ctx->hp_rec, (size_t)ctx->hp_count * CGRT_HP_RECORD_DOUBLES * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
         CKS(dfree(ctx, ctx->hp_rec));
     }
@@ -785,10 +784,6 @@ int cgrt_create(int device, cgrt_ctx **out) {
         ctx->grid_first = occ((const void *)photon_trace_kernel<true>);
         ctx->grid_cont = occ((const void *)photon_trace_kernel<false>);
         if (const char *e = getenv("CGRT_PHOTON_CHUNK")) { long long c = atoll(e); if (c > 0) ctx->photon_chunk = (size_t)c; }  // tests: force multi-chunk passes
-        // resident blocks per SM of the two pipelined halves (dev knobs: how the trace and the deposit stream share an SM)
-        if (const char *e = getenv("CGRT_TRACE_BPS")) { unsigned int b = (unsigned int)atoi(e) * (unsigned int)sms; if (b) { ctx->grid_first = b; ctx->grid_cont = b; ctx->trav_grid = b; } }
-        if (const char *e = getenv("CGRT_TRAV_BPS")) { unsigned int b = (unsigned int)atoi(e) * (unsigned int)sms; if (b) ctx->trav_grid = b; }
-        if (const char *e = getenv("CGRT_DEPOSIT_BPS")) { unsigned int b = (unsigned int)atoi(e) * (unsigned int)sms; if (b) ctx->deposit_grid = b; }
         cudaGetLastError();
     }
     cgrt_default_config(&ctx->cfg);
@@ -895,15 +890,6 @@ int cgrt_synchronize(cgrt_ctx *ctx) {
         int perr = 0;
         CK(cudaMemcpy(&perr, ctx->peer.block + peer_err_off(ctx->peer), sizeof perr, cudaMemcpyDeviceToHost));
         if (perr) FAIL(CGRT_ERR_NCCL, "peer exchange: rank " + std::to_string(perr - 1) + " did not publish its round in time");
-    }
-    if (!ctx->timeline.empty()) {
-        for (size_t k = 0; k + 3 < ctx->timeline.size(); k += 4) {
-            float t[4];
-            for (int j = 0; j < 4; j++) cudaEventElapsedTime(&t[j], ctx->timeline[0], ctx->timeline[k + j]);
-            fprintf(stderr, "[cgrt timeline] chunk %zu: trace %8.2f .. %8.2f ms   deposit %8.2f .. %8.2f ms\n", k / 4, t[0], t[1], t[2], t[3]);
-        }
-        for (cudaEvent_t ev : ctx->timeline) cudaEventDestroy(ev);
-        ctx->timeline.clear();
     }
     return CGRT_OK;
 }
@@ -1059,6 +1045,7 @@ int cgrt_commit_scene(cgrt_ctx *ctx) {
     }
     S.nbvh = nbvh;
     S.nbez = nbez;
+    for (int b = 0; b < nbvh; b++) ctx->bvh_f32 = ctx->bvh_f32 && S.bvh[b].f32_ok;
     S.nplane = S.nsphere = S.ndeferred = 0;
     for (int i = 0; i < S.nobj; i++) {
         if (S.obj[i].kind == OBJ_PLANE) S.plane_ix[S.nplane++] = (unsigned char)i;
@@ -1193,8 +1180,7 @@ static int eye_wavefront(cgrt_ctx *ctx, size_t n, int depth0, int r0, bool gener
         CKS(ensure_queue(ctx, cur ^ 1, 2 * n > max_rays ? 2 * n : max_rays));  // glass splits: at most two children per ray
         CKS(ensure_hp_capacity(ctx, (size_t)ctx->hp_count + n));
         CK(cudaMemsetAsync(ctx->d_qcount + (cur ^ 1), 0, sizeof(unsigned int), ctx->stream));
-        bool f32 = true;  // every tree within the float bound: the instantiation without fp64 box arithmetic
-        for (int b = 0; b < ctx->S.nbvh; b++) f32 = f32 && ctx->S.bvh[b].f32_ok;
+        const bool f32 = ctx->bvh_f32;
 #define LAUNCH_EYE(FIRSTV, F32V, SPPMV)                                                                                                      \
     eye_bounce_kernel<FIRSTV, F32V, SPPMV><<<nblk(n, 128), 128, 0, ctx->stream>>>(ctx->S, P, depth, ctx->q[cur], (unsigned int)n, r0, ctx->q[cur ^ 1], \
                                                                           ctx->d_qcount + (cur ^ 1), ctx->hp_rec, ctx->d_hp_count, ctx->hp_cap, ctx->d_ctr, \
@@ -1261,7 +1247,7 @@ int cgrt_import_hitpoints_dev(cgrt_ctx *ctx, const void *records_dev, int64_t co
     // replaces the current set (the caller passes the all-gathered union, which includes this rank's own records)
     ctx->hp_count = 0;
     CKS(ensure_hp_capacity(ctx, (size_t)count));
-    if (count) CK(cudaMemcpyAsync(ctx->hp_rec, records_dev, (size_t)count * 12 * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+    if (count) CK(cudaMemcpyAsync(ctx->hp_rec, records_dev, (size_t)count * CGRT_HP_RECORD_DOUBLES * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
     unsigned int c = (unsigned int)count;
     CK(cudaMemcpyAsync(ctx->d_hp_count, &c, sizeof c, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
@@ -1426,51 +1412,44 @@ static int photon_pass_impl(cgrt_ctx *ctx, uint64_t first, uint64_t count, const
     const size_t first_chunk = count < chunk ? (size_t)count : chunk;
     if (first_chunk == 0) return CGRT_OK;
     CKS(ensure_photon_buffers(ctx, first_chunk, first_chunk * (size_t)P.max_depth));
-    std::vector<cudaEvent_t> evs;
-    const unsigned int resume_grid = ctx->trav_grid ? ctx->trav_grid : (unsigned int)ctx->sm_count * 8u;  // 8 resident blocks per SM, grid-stride over the queue
+    if (inj_org && first_chunk != count) FAIL(CGRT_ERR_CAPACITY, "cgrt_trace: more rays than one launch holds");
+    const unsigned int resume_grid = (unsigned int)ctx->sm_count * 8u;  // 8 resident blocks per SM, grid-stride over the queue
     const bool overlap = ctx->overlap && !ctx->profiling;
     cudaStream_t D = ctx->stream, T = overlap ? ctx->tstream : ctx->stream;
+    // Profiling runs on one stream and keeps one list of (event, timing slot) stamps: a stamp charges the time since the stamp before
+    // it to its slot, and a chunk opens with slot -1, so the gap between chunks is not charged. Slot 2 (the chunk's whole trace) gets
+    // the memsets and, in the reduction below, every emission (9), Bezier + traversal (7) and continuation (8) interval as well.
+    std::vector<std::pair<cudaEvent_t, int>> marks;
+    auto stamp = [&](int slot) {
+        cudaEvent_t ev;
+        if (ctx->profiling && cudaEventCreate(&ev) == cudaSuccess) {
+            cudaEventRecord(ev, D);
+            marks.push_back(std::make_pair(ev, slot));
+        }
+    };
     for (uint64_t done = 0; done < count; done += chunk) {
         const size_t n = (size_t)((count - done) < chunk ? (count - done) : chunk);
         const uint64_t base = first + done;
         const size_t slots = n * (size_t)P.max_depth;
         cgrt_ctx::DepBuf &B = ctx->dep[overlap ? (ctx->chunk_seq++ & 1u) : 0u];
-        cudaEvent_t e[4] = {nullptr, nullptr, nullptr, nullptr};
-        std::vector<std::pair<cudaEvent_t, int>> marks;  // profiling: (event after a launch, timing slot of that launch)
-        auto stamp = [&](int slot) {
-            if (!ctx->profiling) return;
-            cudaEvent_t ev;
-            cudaEventCreate(&ev);
-            cudaEventRecord(ev, D);
-            marks.push_back(std::make_pair(ev, slot));
-        };
-        if (ctx->profiling) {
-            for (int k = 0; k < 4; k++) { CK(cudaEventCreate(&e[k])); evs.push_back(e[k]); }
-            CK(cudaEventRecord(e[0], D));
-        }
+        stamp(-1);
         // ---- trace (stream T): may not overwrite the buffer before its previous deposit pass has drained it
         if (B.drained_valid) CK(cudaStreamWaitEvent(T, B.drained, 0));
-        static const bool timeline_on = getenv("CGRT_TIMELINE") != nullptr;
-        auto mark = [&](cudaStream_t st) { if (timeline_on) { cudaEvent_t ev; cudaEventCreate(&ev); cudaEventRecord(ev, st); ctx->timeline.push_back(ev); } };
-        mark(T);
         CK(cudaMemsetAsync(B.keys, 0xff, slots * sizeof(uint32_t), T));
         CK(cudaMemsetAsync(B.hist, 0, ((size_t)P.bin_mask + 1) * sizeof(uint32_t), T));
         CK(cudaMemsetAsync(ctx->d_qcount + 2, 0, 12 * sizeof(unsigned int), T));
+        stamp(2);
         unsigned int *qc = ctx->d_qcount + 2;
 #define LAUNCH_PT(F, GRID, QIN, NIN, QOUT, NOUT, CURSOR)                                                                            \
     photon_trace_kernel<F><<<GRID, CGRT_PHOTON_BLOCK, 0, T>>>(ctx->S, P, base, (unsigned int)n, QIN, NIN, QOUT, NOUT, B.rec, compact_records(ctx) ? 1 : 0, B.keys, B.hist, \
                                                              ctx->cull ? ctx->reach : nullptr, ctx->d_ctr, CURSOR)
         if (inj_org) {
-            if (n != count) FAIL(CGRT_ERR_CAPACITY, "cgrt_trace: more rays than one launch holds");
-            stamp(-1);
             photon_inject_kernel<<<nblk(n, 128), 128, 0, T>>>(ctx->S, (unsigned int)n, inj_depth, inj_org, inj_dir, inj_flux, ctx->pq[0], qc);
-            stamp(9);
         } else {
             unsigned int want = nblk(n, CGRT_PHOTON_BLOCK);
-            stamp(-1);
             LAUNCH_PT(true, (want < ctx->grid_first ? want : ctx->grid_first), nullptr, nullptr, ctx->pq[0], qc, qc + 6);
-            stamp(9);
         }
+        stamp(9);
         ctx->launches++;
         if (inj_org || ctx->S.nbvh > 0 || ctx->S.nbez > 0) {
             for (int pass = 1; pass <= P.max_depth; pass++) {  // a resumed photon advances at least one segment per pass
@@ -1482,10 +1461,8 @@ static int photon_pass_impl(cgrt_ctx *ctx, uint64_t first, uint64_t count, const
                     ctx->launches++;
                 }
                 if (ctx->S.nbvh > 0) {
-                    // every tree within CGRT_F32_BOUND (all BASELINE scenes): the instantiation without fp64 box arithmetic
                     static const bool trav_exact = getenv("CGRT_TRAV_EXACT") != nullptr;  // dev: force the fp64-slab instantiation
-                    bool f32 = !trav_exact;
-                    for (int b = 0; b < ctx->S.nbvh; b++) f32 = f32 && ctx->S.bvh[b].f32_ok;
+                    const bool f32 = ctx->bvh_f32 && !trav_exact;  // true on all BASELINE scenes
                     if (ctx->counting) {
                         if (f32) photon_traverse_kernel<true, true><<<resume_grid, 128, 0, T>>>(ctx->S, qin, nin, ctx->d_tc);
                         else photon_traverse_kernel<true, false><<<resume_grid, 128, 0, T>>>(ctx->S, qin, nin, ctx->d_tc);
@@ -1502,14 +1479,11 @@ static int photon_pass_impl(cgrt_ctx *ctx, uint64_t first, uint64_t count, const
             }
         }
 #undef LAUNCH_PT
-        if (ctx->profiling) CK(cudaEventRecord(e[1], D));
-        mark(T);
         // ---- sort + deposit (stream D) after the trace of this buffer
         if (overlap) {
             CK(cudaEventRecord(B.traced, T));
             CK(cudaStreamWaitEvent(D, B.traced, 0));
         }
-        mark(D);
         // the trace launches above read neither radii nor accumulators; the gather does: the previous round's update must have landed
         CKS(join_update(ctx));
         if (ctx->nhp > 0) {
@@ -1518,7 +1492,7 @@ static int photon_pass_impl(cgrt_ctx *ctx, uint64_t first, uint64_t count, const
             bin_scan_sums_kernel<<<1, CGRT_SCAN_BLOCK, 0, D>>>(B.bsum, nsb, B.nvalid);
             bin_scatter_kernel<<<ctx->deposit_grid, 256, 0, D>>>(B.keys, slots, B.hist, B.bsum, B.perm);
             ctx->launches += 3;
-            if (ctx->profiling) CK(cudaEventRecord(e[2], D));
+            stamp(6);
             size_t spans = (slots + CGRT_DEPOSIT_SPAN - 1) / CGRT_DEPOSIT_SPAN;
             size_t want = (spans * 32 + CGRT_DEPOSIT_BLOCK - 1) / CGRT_DEPOSIT_BLOCK;
             unsigned int dblocks = (unsigned int)(want < (size_t)ctx->deposit_grid ? want : (size_t)ctx->deposit_grid);
@@ -1534,38 +1508,27 @@ static int photon_pass_impl(cgrt_ctx *ctx, uint64_t first, uint64_t count, const
                 photon_deposit_kernel<1><<<dblocks, CGRT_DEPOSIT_BLOCK, 0, D>>>(P, reinterpret_cast<const DepositRec *>(B.rec), B.perm, B.nvalid, ctx->cell_start, ctx->A.pre, ctx->A.pre_n,
                                                                                 ctx->A.pre_f, ctx->A.hot, ctx->A.f, ctx->acc, ctx->d_ctr, U1);
             ctx->launches++;
-        } else if (ctx->profiling) {
-            CK(cudaEventRecord(e[2], D));
+        } else {
+            stamp(6);
         }
-        mark(D);
+        stamp(3);
         if (overlap) {
             CK(cudaEventRecord(B.drained, D));
             B.drained_valid = true;
         }
-        if (ctx->profiling) CK(cudaEventRecord(e[3], D));
-        for (auto &m : marks) ctx->prof_marks.push_back(m);
         CK(cudaGetLastError());
     }
     if (ctx->profiling) {
         CK(cudaStreamSynchronize(ctx->stream));
-        for (size_t k = 0; k + 3 < evs.size(); k += 4) {
-            float t01 = 0, t12 = 0, t23 = 0;
-            cudaEventElapsedTime(&t01, evs[k], evs[k + 1]);
-            cudaEventElapsedTime(&t12, evs[k + 1], evs[k + 2]);
-            cudaEventElapsedTime(&t23, evs[k + 2], evs[k + 3]);
-            ctx->ms[2] += t01;
-            ctx->ms[6] += t12;
-            ctx->ms[3] += t23;
-        }
-        for (cudaEvent_t ev : evs) cudaEventDestroy(ev);
-        for (size_t k = 1; k < ctx->prof_marks.size(); k++) {
-            if (ctx->prof_marks[k].second < 0) continue;  // -1 opens a chunk
+        for (size_t k = 1; k < marks.size(); k++) {
+            const int slot = marks[k].second;
+            if (slot < 0) continue;
             float t = 0;
-            cudaEventElapsedTime(&t, ctx->prof_marks[k - 1].first, ctx->prof_marks[k].first);
-            ctx->ms[ctx->prof_marks[k].second] += t;
+            cudaEventElapsedTime(&t, marks[k - 1].first, marks[k].first);
+            ctx->ms[slot] += t;
+            if (slot == 9 || slot == 7 || slot == 8) ctx->ms[2] += t;
         }
-        for (auto &m : ctx->prof_marks) cudaEventDestroy(m.first);
-        ctx->prof_marks.clear();
+        for (auto &m : marks) cudaEventDestroy(m.first);
     }
     return CGRT_OK;
 }
@@ -1830,8 +1793,7 @@ int cgrt_round_update(cgrt_ctx *ctx) {
     // and when an NCCL all-reduce is part of it: measured on 8 GPUs, the collective on the side stream is SLOWER than in stream order
     // (c2: 5.40 vs 4.93 ms per round, c1: 5.72 vs 5.54): NCCL's blocks cannot become resident next to the persistent emission kernel of
     // the next round (4 blocks x 114 registers fill an SM), so the all-reduce starts late on some rank and every rank waits for it
-    static const bool comm_side = getenv("CGRT_COMM_SIDE_STREAM") != nullptr;  // dev: the side-stream variant
-    cudaStream_t U = (ctx->profiling || (ctx->comm && !comm_side)) ? ctx->stream : ctx->ustream;
+    cudaStream_t U = (ctx->profiling || ctx->comm) ? ctx->stream : ctx->ustream;
     if (U != ctx->stream) {
         CK(cudaEventRecord(ctx->ev_tail, ctx->stream));
         CK(cudaStreamWaitEvent(U, ctx->ev_tail, 0));

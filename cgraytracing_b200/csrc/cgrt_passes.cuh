@@ -1435,7 +1435,7 @@ __global__ void __launch_bounds__(64) peer_reduce_update_kernel(unsigned int n, 
         dx = fx; dy = fy; dz = fz; m = fm;
         reinterpret_cast<float4 *>(clear_next)[k] = make_float4(0, 0, 0, 0);
     }
-    if (m > 0) {
+    if (m > 0) {  // round_update_kernel's tail, written out: shared as an inline helper it changes this kernel's register allocation
         int cnt = A.cnt[k];
         double na = cnt * alpha;
         double g = (na + alpha * m) / (na + m);
@@ -1476,6 +1476,18 @@ __global__ void round_update_u1_kernel(unsigned int n, HpArrays A, const double 
 // =================================================================================================================
 __device__ __forceinline__ int gamma_corr(double x) { return int(pow(1 - exp(-x), 1 / 2.2) * 255 + .5); }  // util.h:45-47
 
+// pixel p's linear value, and (rgb8 != nullptr) its tone-mapped bytes; main.cpp:403-411: row i of the PNG is image[height-1-i]
+__device__ __forceinline__ void write_pixel(int width, int height, unsigned int p, d3 acc, double *rgb, uint8_t *rgb8) {
+    rgb[3 * (size_t)p] = acc.x; rgb[3 * (size_t)p + 1] = acc.y; rgb[3 * (size_t)p + 2] = acc.z;
+    if (rgb8) {
+        int h = p / width, w = p % width;
+        size_t q = (size_t)(height - 1 - h) * width + w;
+        rgb8[3 * q] = (uint8_t)(char)gamma_corr(acc.x);
+        rgb8[3 * q + 1] = (uint8_t)(char)gamma_corr(acc.y);
+        rgb8[3 * q + 2] = (uint8_t)(char)gamma_corr(acc.z);
+    }
+}
+
 __global__ void image_gather_kernel(int width, int height, double n_emitted, const uint32_t *__restrict__ pix_start,
                                     const uint32_t *__restrict__ pix_perm, const HpHot *__restrict__ hot, const double *__restrict__ flux,
                                     double *__restrict__ rgb, uint8_t *__restrict__ rgb8) {
@@ -1488,14 +1500,7 @@ __global__ void image_gather_kernel(int width, int height, double n_emitted, con
         d3 fl = mk(flux[4 * (size_t)k], flux[4 * (size_t)k + 1], flux[4 * (size_t)k + 2]);
         acc = acc + fl * (1.0 / (CGRT_PI * r2 * n_emitted));
     }
-    rgb[3 * (size_t)p] = acc.x; rgb[3 * (size_t)p + 1] = acc.y; rgb[3 * (size_t)p + 2] = acc.z;
-    if (rgb8) {  // main.cpp:403-411: row i of the PNG is image[height-1-i]
-        int h = p / width, w = p % width;
-        size_t q = (size_t)(height - 1 - h) * width + w;
-        rgb8[3 * q] = (uint8_t)(char)gamma_corr(acc.x);
-        rgb8[3 * q + 1] = (uint8_t)(char)gamma_corr(acc.y);
-        rgb8[3 * q + 2] = (uint8_t)(char)gamma_corr(acc.z);
-    }
+    write_pixel(width, height, p, acc, rgb, rgb8);
 }
 
 // SPPM image: main.cpp:252-258 with the pixel's statistics in place of its hitpoints' — the expression and the tone map / flip of
@@ -1507,14 +1512,7 @@ __global__ void sppm_image_kernel(int width, int height, double n_emitted, const
     d3 acc = mk(0, 0, 0);
     d3 fl = mk(tau[4 * (size_t)p], tau[4 * (size_t)p + 1], tau[4 * (size_t)p + 2]);
     acc = acc + fl * (1.0 / (CGRT_PI * r2[p] * n_emitted));
-    rgb[3 * (size_t)p] = acc.x; rgb[3 * (size_t)p + 1] = acc.y; rgb[3 * (size_t)p + 2] = acc.z;
-    if (rgb8) {
-        int h = p / width, w = p % width;
-        size_t q = (size_t)(height - 1 - h) * width + w;
-        rgb8[3 * q] = (uint8_t)(char)gamma_corr(acc.x);
-        rgb8[3 * q + 1] = (uint8_t)(char)gamma_corr(acc.y);
-        rgb8[3 * q + 2] = (uint8_t)(char)gamma_corr(acc.z);
-    }
+    write_pixel(width, height, p, acc, rgb, rgb8);
 }
 
 // =================================================================================================================

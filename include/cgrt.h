@@ -149,8 +149,8 @@ int cgrt_comm_destroy(void *comm);
  * under SPPM after cgrt_sppm_eye_pass); every rank then builds the same grid from the union. */
 int cgrt_allgather_hitpoints(cgrt_ctx *ctx, void *nccl_comm, int world);
 /* Attach a communicator: from now on cgrt_round_update all-reduces the accumulators {dflux.xyz, m} over it, in stream order, before
- * applying the update (under SPPM: before the per-pixel fold; attach it before cgrt_set_sppm) (the variant that ran the collective on a side stream underneath the next round's trace launches was measured
- * slower on 8 GPUs: NCCL's blocks do not fit next to the persistent trace kernels). NULL detaches. */
+ * applying the update (under SPPM: before the per-pixel fold; attach it before cgrt_set_sppm). In stream order: on a side stream under
+ * the next round's trace launches it measured slower on 8 GPUs (NCCL's blocks do not fit next to the persistent trace kernels). NULL detaches. */
 int cgrt_set_comm(cgrt_ctx *ctx, void *nccl_comm, int world);
 /* The same exchange without a collective call, over peer memory (GPUs of one box, NVLink / NVSwitch): every rank's accumulators live in a
  * block all ranks have mapped; cgrt_round_update publishes "round deposited" flags and ONE kernel on a side stream reads every rank's

@@ -382,6 +382,20 @@ def test_chunked_and_pipelined_photon_pass(gpu, oracle_lib, overlap, monkeypatch
         assert g.counters()["gpu_launches"] > 3 * 5 * 12
 
 
+def test_profiled_photon_pass_timing_slots(gpu, monkeypatch):
+    """With profiling on, a multi-chunk photon pass over a mesh scene fills every photon-pass slot of timings() (bench.py reports
+    them), and the trace slot covers its emission, traversal and continuation parts."""
+    monkeypatch.setenv("CGRT_PHOTON_CHUNK", "7001")
+    with gpu.Context(0, gpu.preset("c2_bunny_chess"), gpu.RenderConfig(width=128, height=96)) as g:
+        g.set_profiling(True)
+        g.eye_pass(); g.build_grid()
+        g.photon_pass(0, 30000)
+        t = g.timings()
+    for k in ("photon_trace", "deposit_sort", "photon_deposit", "trace_emit", "trace_traverse", "trace_continue"):
+        assert t[k] > 0, (k, t)
+    assert t["photon_trace"] >= t["trace_emit"] + t["trace_traverse"] + t["trace_continue"], t
+
+
 def test_dof_camera_and_samples_bit_exact(gpu, oracle_lib):
     """BASELINE config 4: thin-lens camera (main.cpp:203-207) with num_of_samples > 1 over the displaced floor and the objtype-2 mesh.
     Run twice in one process: the second context re-uses pooled device memory, so anything read before it is written shows up."""

@@ -5,9 +5,3 @@ python -m pytest tests -m gpu -x -q 2>&1 | tail -3
 python __graft_entry__.py smoke 2>&1 | tail -1
 python bench.py > gpurun_out/${TAG}_bench.json 2> gpurun_out/${TAG}_bench.err; tail -2 gpurun_out/${TAG}_bench.err
 python bench.py --impl reference > gpurun_out/${TAG}_bench_reference_arm.json 2> gpurun_out/${TAG}_ref.err; tail -2 gpurun_out/${TAG}_ref.err
-CMD="python bench.py --steps 1 --warmup 1 --cpu-photons 0 --e2e-rounds 0 --f64-too 0"
-$CMD > gpurun_out/ncu_plain.log 2>&1 &&
-ncu --metrics gpu__time_duration.sum,smsp__thread_inst_executed_per_inst_executed.ratio,smsp__inst_executed.sum,sm__warps_active.avg.pct_of_peak_sustained_active,smsp__issue_active.avg.pct_of_peak_sustained_active,dram__bytes_read.sum,dram__bytes_write.sum --clock-control none -c 400 --csv --log-file gpurun_out/${TAG}_launches.csv $CMD > gpurun_out/ncu_launch.log 2>&1
-$CMD > gpurun_out/ncu_plain2.log 2>&1 &&
-ncu --set full --clock-control none --import-source on -k regex:"photon_" -s 24 -c 12 -f -o gpurun_out/${TAG}_prof $CMD > gpurun_out/ncu_full.log 2>&1
-tail -2 gpurun_out/ncu_full.log | cut -c1-200
