@@ -1244,6 +1244,22 @@ int cgrt_import_hitpoints_dev(cgrt_ctx *ctx, const void *records_dev, int64_t co
         FAIL(CGRT_ERR_INVALID, "SPPM is on: import the round's visible points between cgrt_sppm_eye_pass and cgrt_build_grid");
     if (ctx->grid_built) FAIL(CGRT_ERR_INVALID, "grid already built");
     CK(cudaSetDevice(ctx->device));
+    if (count >= (1ll << 32)) FAIL(CGRT_ERR_INVALID, "more hitpoint records than one import holds");
+    if (count) {  // the records come from the caller: checked before they replace anything (see hp_validate_kernel)
+        unsigned int *d_bad, bad = 0;
+        CKS(dalloc(ctx, &d_bad, 1));
+        CK(cudaMemsetAsync(d_bad, 0, sizeof(unsigned int), ctx->stream));
+        hp_validate_kernel<<<nblk((size_t)count, 256), 256, 0, ctx->stream>>>(static_cast<const double *>(records_dev), (unsigned int)count, ctx->P.celllength,
+                                                                           ctx->P.hashsize, ctx->P.width, ctx->P.height, d_bad);
+        ctx->launches++;
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(&bad, d_bad, sizeof bad, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        CKS(dfree(ctx, d_bad));
+        if (bad & 1u) FAIL(CGRT_ERR_INVALID, "import: a record's bucket key is >= hashsize");
+        if (bad & 2u) FAIL(CGRT_ERR_INVALID, "import: a record's bucket key is not the cell key of its position");
+        if (bad & 4u) FAIL(CGRT_ERR_INVALID, "import: a record's pixel lies outside the image");
+    }
     // replaces the current set (the caller passes the all-gathered union, which includes this rank's own records)
     ctx->hp_count = 0;
     CKS(ensure_hp_capacity(ctx, (size_t)count));

@@ -253,6 +253,25 @@ __global__ void hp_extract_keys_kernel(const double *__restrict__ rec, unsigned 
     if (i < n) keys[i] = (uint64_t)__double_as_longlong(rec[(size_t)i * 12 + 9]);
 }
 
+// Imported records are checked before build_grid uses their key and pixel as indices (lower_bound_table_kernel,
+// sppm_visible_radius_kernel): bit 0 = a key >= hashsize, bit 1 = a key that is not the cell key of the position (the hitpoint would sit
+// in a bucket no photon near it gathers), bit 2 = a pixel outside the image.
+__global__ void hp_validate_kernel(const double *__restrict__ rec, unsigned int n, double celllength, uint32_t hashsize, int width, int height,
+                                   unsigned int *__restrict__ bad) {
+    unsigned int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double *r = rec + (size_t)i * 12;
+    const uint32_t key = (uint32_t)((uint64_t)__double_as_longlong(r[9]) >> 32);
+    const uint64_t hw = (uint64_t)__double_as_longlong(r[10]);
+    int ix, iy, iz;
+    cell_coord(mk(r[0], r[1], r[2]), celllength, 1.0 / celllength, ix, iy, iz);
+    unsigned int f = 0;
+    if (key >= hashsize) f |= 1u;
+    else if (key != cell_hash(ix, iy, iz, hashsize)) f |= 2u;
+    if ((uint32_t)(hw >> 32) >= (uint32_t)height || (uint32_t)hw >= (uint32_t)width) f |= 4u;
+    if (f) atomicOr(bad, f);
+}
+
 struct HpArrays {
     float4 *pre;           // fp32 prefilter {x, y, z, (r+E)^2} read per candidate
     float4 *pre_n;         // fp32 accept filter {nx, ny, nz, (r-E)^2}

@@ -119,7 +119,8 @@ int cgrt_count_traversal(cgrt_ctx *ctx, int64_t n, const double *org, const doub
 /* Eye pass (main.cpp:183-219) over image rows [y0,y1) as an iterative wavefront; appends hitpoints. */
 int cgrt_eye_pass(cgrt_ctx *ctx, int y0, int y1);
 /* Tile-sharded eye pass: export this rank's unsorted hitpoint records / import the union (all-gather in between).
- * Records are CGRT_HP_RECORD_DOUBLES doubles each. */
+ * Records are CGRT_HP_RECORD_DOUBLES doubles each. The import refuses the whole set (CGRT_ERR_INVALID, the current set kept) when a
+ * record's bucket key is >= hashsize or is not the cell key of its position, or when its pixel lies outside the image. */
 #define CGRT_HP_RECORD_DOUBLES 12
 int cgrt_export_hitpoints_dev(cgrt_ctx *ctx, void **records_dev, int64_t *count);
 int cgrt_import_hitpoints_dev(cgrt_ctx *ctx, const void *records_dev, int64_t count);
