@@ -3,6 +3,7 @@
 // compacted with warp ballots (one atomic per warp); the hash table of vectors becomes a sorted array + cell-start
 // table; photon deposits are atomics into per-round accumulators.
 #pragma once
+#include "../../include/cgrt.h"
 #include "cgrt_build.cuh"
 
 namespace cgrt {
@@ -81,10 +82,12 @@ struct Counters {
 
 // =================================================================================================================
 // Eye pass, one kernel per depth level. Level 0 generates the camera rays (main.cpp:188-209) in registers.
-// Hitpoint records (12 doubles): pos, normal, f*adj, bits(sortkey), bits(h<<32|w), 0.
+// Hitpoint records (CGRT_HP_RECORD_DOUBLES doubles): pos, normal, f*adj, bits(sortkey), bits(h<<32|w), 0.
 // sortkey = bucket key << 32 | (path*16 + dfs bits): sorting by it gives the reference's bucket order (hash.h:52,
 // main.cpp:252-254) whatever order the wavefront produced the hitpoints in.
 // =================================================================================================================
+enum { HP_POS = 0, HP_NRM = 3, HP_F = 6, HP_KEY = 9, HP_PIX = 10 };  // offsets into a hitpoint record
+static_assert(HP_PIX + 2 == CGRT_HP_RECORD_DOUBLES, "hitpoint record layout");
 #define CGRT_TRACE_BLOCK 128
 #ifndef CGRT_PHOTON_BLOCK
 #define CGRT_PHOTON_BLOCK 128   /* threads per block of photon_trace_kernel */
@@ -198,13 +201,13 @@ __global__ void __launch_bounds__(CGRT_TRACE_BLOCK) eye_bounce_kernel(const __gr
         uint32_t pix = path / (uint32_t)P.samples;
         uint64_t hw = ((uint64_t)(pix / (uint32_t)P.width) << 32) | (uint64_t)(pix % (uint32_t)P.width);
         d3 fa = f * adj;
-        double *r = hp_rec + (size_t)hs * 12;
-        r[0] = X.x; r[1] = X.y; r[2] = X.z;
-        r[3] = n_ff.x; r[4] = n_ff.y; r[5] = n_ff.z;
-        r[6] = fa.x; r[7] = fa.y; r[8] = fa.z;
-        r[9] = __longlong_as_double((long long)sortkey);
-        r[10] = __longlong_as_double((long long)hw);
-        r[11] = 0.0;
+        double *r = hp_rec + (size_t)hs * CGRT_HP_RECORD_DOUBLES;
+        r[HP_POS] = X.x; r[HP_POS + 1] = X.y; r[HP_POS + 2] = X.z;
+        r[HP_NRM] = n_ff.x; r[HP_NRM + 1] = n_ff.y; r[HP_NRM + 2] = n_ff.z;
+        r[HP_F] = fa.x; r[HP_F + 1] = fa.y; r[HP_F + 2] = fa.z;
+        r[HP_KEY] = __longlong_as_double((long long)sortkey);
+        r[HP_PIX] = __longlong_as_double((long long)hw);
+        r[HP_PIX + 1] = 0.0;
     }
 
     // ---- mirror / glass: children (main.cpp:129-157)
@@ -250,7 +253,7 @@ __global__ void __launch_bounds__(CGRT_TRACE_BLOCK) eye_bounce_kernel(const __gr
 // =================================================================================================================
 __global__ void hp_extract_keys_kernel(const double *__restrict__ rec, unsigned int n, uint64_t *__restrict__ keys) {
     unsigned int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) keys[i] = (uint64_t)__double_as_longlong(rec[(size_t)i * 12 + 9]);
+    if (i < n) keys[i] = (uint64_t)__double_as_longlong(rec[(size_t)i * CGRT_HP_RECORD_DOUBLES + HP_KEY]);
 }
 
 // Imported records are checked before build_grid uses their key and pixel as indices (lower_bound_table_kernel,
@@ -260,11 +263,11 @@ __global__ void hp_validate_kernel(const double *__restrict__ rec, unsigned int 
                                    unsigned int *__restrict__ bad) {
     unsigned int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const double *r = rec + (size_t)i * 12;
-    const uint32_t key = (uint32_t)((uint64_t)__double_as_longlong(r[9]) >> 32);
-    const uint64_t hw = (uint64_t)__double_as_longlong(r[10]);
+    const double *r = rec + (size_t)i * CGRT_HP_RECORD_DOUBLES;
+    const uint32_t key = (uint32_t)((uint64_t)__double_as_longlong(r[HP_KEY]) >> 32);
+    const uint64_t hw = (uint64_t)__double_as_longlong(r[HP_PIX]);
     int ix, iy, iz;
-    cell_coord(mk(r[0], r[1], r[2]), celllength, 1.0 / celllength, ix, iy, iz);
+    cell_coord(mk(r[HP_POS], r[HP_POS + 1], r[HP_POS + 2]), celllength, 1.0 / celllength, ix, iy, iz);
     unsigned int f = 0;
     if (key >= hashsize) f |= 1u;
     else if (key != cell_hash(ix, iy, iz, hashsize)) f |= 2u;
@@ -285,23 +288,31 @@ struct HpArrays {
     uint32_t *seq;         // path*16 + dfs bits
 };
 
+// A new radius for hitpoint k (hh = its hot record, position read from it): the exact record and both fp32 filter bounds follow it.
+// Every radius change after hp_gather_sorted_kernel goes through here, so no filter is ever left at an older radius.
+__device__ __forceinline__ void set_radius(const HpArrays &A, unsigned int k, const HpHot &hh, double r2) {
+    A.hot[k].r2 = r2;
+    A.pre[k] = make_prefilter(hh.px, hh.py, hh.pz, r2);
+    A.pre_n[k].w = prefilter_inner(hh.px, hh.py, hh.pz, r2);
+}
+
 __global__ void hp_gather_sorted_kernel(const double *__restrict__ rec, const uint32_t *__restrict__ perm, unsigned int n, double r2_init,
                                         HpArrays A, uint64_t *__restrict__ pixkeys, int width) {
     unsigned int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
-    const double *r = rec + (size_t)perm[k] * 12;
+    const double *r = rec + (size_t)perm[k] * CGRT_HP_RECORD_DOUBLES;
     HpHot h;
-    h.px = r[0]; h.py = r[1]; h.pz = r[2]; h.r2 = r2_init;
-    h.nx = r[3]; h.ny = r[4]; h.nz = r[5]; h.pad = 0.0;
+    h.px = r[HP_POS]; h.py = r[HP_POS + 1]; h.pz = r[HP_POS + 2]; h.r2 = r2_init;
+    h.nx = r[HP_NRM]; h.ny = r[HP_NRM + 1]; h.nz = r[HP_NRM + 2]; h.pad = 0.0;
     A.hot[k] = h;
     A.pre[k] = make_prefilter(h.px, h.py, h.pz, r2_init);
     A.pre_n[k] = make_float4((float)h.nx, (float)h.ny, (float)h.nz, prefilter_inner(h.px, h.py, h.pz, r2_init));
-    A.pre_f[k] = make_float4((float)r[6], (float)r[7], (float)r[8], 0.f);
-    A.f[4 * (size_t)k] = r[6]; A.f[4 * (size_t)k + 1] = r[7]; A.f[4 * (size_t)k + 2] = r[8]; A.f[4 * (size_t)k + 3] = 0.0;
+    A.pre_f[k] = make_float4((float)r[HP_F], (float)r[HP_F + 1], (float)r[HP_F + 2], 0.f);
+    A.f[4 * (size_t)k] = r[HP_F]; A.f[4 * (size_t)k + 1] = r[HP_F + 1]; A.f[4 * (size_t)k + 2] = r[HP_F + 2]; A.f[4 * (size_t)k + 3] = 0.0;
     A.flux[4 * (size_t)k] = 0.0; A.flux[4 * (size_t)k + 1] = 0.0; A.flux[4 * (size_t)k + 2] = 0.0; A.flux[4 * (size_t)k + 3] = 0.0;
     A.cnt[k] = 0;
-    uint64_t sk = (uint64_t)__double_as_longlong(r[9]);
-    uint64_t hw = (uint64_t)__double_as_longlong(r[10]);
+    uint64_t sk = (uint64_t)__double_as_longlong(r[HP_KEY]);
+    uint64_t hw = (uint64_t)__double_as_longlong(r[HP_PIX]);
     A.key[k] = (uint32_t)(sk >> 32);
     A.seq[k] = (uint32_t)sk;
     int hh = (int)(hw >> 32), ww = (int)(uint32_t)hw;
@@ -309,16 +320,13 @@ __global__ void hp_gather_sorted_kernel(const double *__restrict__ rec, const ui
     pixkeys[k] = (uint64_t)hh * (uint64_t)width + (uint64_t)ww;
 }
 
-// SPPM: every visible point of a round takes its pixel's current radius (in place of the r2_init hp_gather_sorted_kernel wrote) and
-// the prefilter records follow it, exactly as round_update_kernel writes them when a radius shrinks.
+// SPPM: every visible point of a round takes its pixel's current radius (in place of the r2_init hp_gather_sorted_kernel wrote).
 __global__ void sppm_visible_radius_kernel(unsigned int n, HpArrays A, const double *__restrict__ pix_r2, int width) {
     unsigned int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
     const double r2 = pix_r2[(size_t)A.hw[2 * (size_t)k] * (size_t)width + (size_t)A.hw[2 * (size_t)k + 1]];
-    HpHot hh = A.hot[k];
-    A.hot[k].r2 = r2;
-    A.pre[k] = make_prefilter(hh.px, hh.py, hh.pz, r2);
-    A.pre_n[k].w = prefilter_inner(hh.px, hh.py, hh.pz, r2);
+    const HpHot hh = A.hot[k];  // a local copy: passing A.hot[k] itself compiles to 24 more instructions
+    set_radius(A, k, hh, r2);
 }
 
 // start[v] = first sorted index whose key is >= v, for v in [0, nvals]; keys ascending.
@@ -773,9 +781,11 @@ __global__ void __launch_bounds__(CGRT_PHOTON_BLOCK, CGRT_TRACE_MINB) photon_tra
 // group instead of once per photon hit): up to 64 candidates at a time are staged in shared memory as 16-byte fp32
 // prefilter records {x, y, z, (r + E)^2} (E bounds the float rounding of both positions: the filter can only pass too
 // much) and every lane tests its own hit against each of them from a shared-memory broadcast, collecting a 64-bit mask.
-// Surviving pairs (~10-15 %) are drained into a per-warp queue and processed 32 at a time by ALL lanes with the
-// reference's exact fp64 test (main.cpp:116) on the 64-byte exact records, then deposited with atomics. Two of the 27 cells hashing to one bucket list it twice, like the reference
-// (SURVEY Q13). ACC: 0 = fp64 atomics {dflux.xyz, m}; 1 = one red.global.add.v4.f32.
+// Surviving pairs (~10-15 %) are decided by decide_pair_f32, or by the reference's exact fp64 test (main.cpp:116) where the float
+// bounds cannot tell, and deposited with atomics. Two of the 27 cells hashing to one bucket list it twice, like the reference (SURVEY Q13).
+//   ACC 0 (fp64 atomics {dflux.xyz, m}) and 2 (per-photon update, deposit_u1): the batch is copied to shared memory (HitShared); the
+//         surviving pairs are drained into a per-warp queue and processed 32 at a time by ALL lanes (deposit_pair).
+//   ACC 1 (one red.global.add.v4.f32 per deposit): every lane walks its own surviving pairs, its hit in registers.
 // ---------------------------------------------------------------------------------------------------------------------
 #define CGRT_DEPOSIT_BLOCK 256
 #ifndef CGRT_DEPOSIT_MINB
@@ -791,44 +801,25 @@ __device__ __forceinline__ double4 ldg4(const double4 *p) {  // 32 bytes of a de
     return make_double4(a.x, a.y, b.x, b.y);
 }
 
-// What a warp keeps in shared memory about the 32 records of its batch (structure of arrays, one row per component).
-// ACC 0 (fp64 accumulators): the exact fp64 record, because every deposit is computed from the fp64 flux.
-// ACC 1 (float accumulators): only the fp32 copy and the slot of the record; the few pairs the fp32 filters cannot decide re-read the
-// record from the deposit table.
-template <int ACC>
-struct HitShared;
-template <>
-struct HitShared<0> {
+// What a warp keeps in shared memory about the 32 records of its batch in the fp64-accumulator modes (ACC 0 and 2; structure of
+// arrays, one row per component): the exact fp64 record, because every deposit is computed from the fp64 flux. The float-accumulator
+// mode keeps each lane's hit in its registers instead.
+struct HitShared {
     double v[9][32];  // pos.xyz, nrm.xyz, flux.xyz
     float f[6][32];   // fp32 pos.xyz, nrm.xyz
 };
-template <>
-struct HitShared<1> {
-    float f[9][32];   // fp32 pos.xyz, nrm.xyz, flux.xyz
-    uint32_t src[32]; // slot of the record in the deposit table
-};
-
-template <>
-struct HitShared<2> : HitShared<0> {};  // per-photon update: fp64 records like ACC 0
 
 struct ExactHit {  // the fp64 photon side of one pair
     d3 X, nrm, flux;
 };
-__device__ __forceinline__ ExactHit exact_hit(const HitShared<0> &H, uint32_t hl, const DepositRec *) {
+__device__ __forceinline__ ExactHit exact_hit(const HitShared &H, uint32_t hl) {
     ExactHit e;
     e.X = mk(H.v[0][hl], H.v[1][hl], H.v[2][hl]); e.nrm = mk(H.v[3][hl], H.v[4][hl], H.v[5][hl]); e.flux = mk(H.v[6][hl], H.v[7][hl], H.v[8][hl]);
     return e;
 }
-__device__ __forceinline__ ExactHit exact_hit(const HitShared<2> &H, uint32_t hl, const DepositRec *r) { return exact_hit(static_cast<const HitShared<0> &>(H), hl, r); }
-__device__ __forceinline__ ExactHit exact_hit(const HitShared<1> &H, uint32_t hl, const DepositRec *__restrict__ rec) {
-    // float-accumulator mode: the table holds compact records (DepositRecC); the flux was rounded to float by the producer
-    const double2 *r = reinterpret_cast<const double2 *>(reinterpret_cast<const DepositRecC *>(rec) + H.src[hl]);
-    const double2 r0 = __ldcs(r), r1 = __ldcs(r + 1), r2 = __ldcs(r + 2), r3 = __ldcs(r + 3);
-    ExactHit e;
-    e.X = mk(r0.x, r0.y, r1.x); e.nrm = mk(r1.y, r2.x, r2.y);
-    const long long f01 = __double_as_longlong(r3.x), f2 = __double_as_longlong(r3.y);
-    e.flux = mk((double)__uint_as_float((uint32_t)f01), (double)__uint_as_float((uint32_t)(f01 >> 32)), (double)__uint_as_float((uint32_t)f2));
-    return e;
+
+__device__ __forceinline__ void red_add_v4(float *ap, float a, float b, float c, float d) {
+    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(ap), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
 template <int ACC>
@@ -837,9 +828,7 @@ __device__ __forceinline__ void deposit_add(void *__restrict__ acc, uint32_t hid
         double *ap = reinterpret_cast<double *>(acc) + 4 * (size_t)hidx;
         atomicAdd(ap, cc.x); atomicAdd(ap + 1, cc.y); atomicAdd(ap + 2, cc.z); atomicAdd(ap + 3, 1.0);
     } else {
-        float *ap = reinterpret_cast<float *>(acc) + 4 * (size_t)hidx;
-        asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(ap), "f"((float)cc.x), "f"((float)cc.y), "f"((float)cc.z), "f"(1.0f)
-                     : "memory");
+        red_add_v4(reinterpret_cast<float *>(acc) + 4 * (size_t)hidx, (float)cc.x, (float)cc.y, (float)cc.z, 1.0f);
     }
 }
 
@@ -900,48 +889,46 @@ __device__ __forceinline__ void deposit_u1(const ExactHit &e, uint32_t hidx, con
     }
 }
 
-// One pair that passed the prefilter. Its outcome is decided in fp32 from shared memory whenever the rounding bounds allow it:
+// The fp32 decision of one pair that passed the prefilter, from the candidate's filter records q = {x, y, z, (r + E)^2} and
+// qn = {nx, ny, nz, (r - E)^2} and the hit's float position h and normal n:
 //   distance   s = |fl(hp) - fl(X)|^2 <= (r - E)^2 proves dot(dd, dd) <= r2 (prefilter_inner); the prefilter already had s <= (r + E)^2
 //   normals    |fl-dot - dot| <= 5 * 2^-24 * sum |hn_i * nrm_i| (two input roundings and the float evaluation); 1e-6 * sum + 1e-9
 //              is the margin used, on either side of CGRT_EPS
-// A pair both filters accept is deposited without touching the hitpoint's exact record (float accumulators: from the fp32 copy of f in
-// shared memory; fp64 accumulators: f from global, flux from the shared fp64 record — the deposited value is the reference's).
-// A pair the normal filter rejects is dropped. Only pairs in the thin shells in between (about 1e-3 of them) take the fp64 path.
-template <int ACC>
-__device__ __forceinline__ void deposit_pair(const HitShared<ACC> &H, uint32_t hl, uint32_t hidx, float4 q, float4 qn, float4 qf,
-                                             const DepositRec *__restrict__ rec, const HpHot *__restrict__ hot, const double *__restrict__ hp_f,
-                                             void *__restrict__ acc, const U1State &U, unsigned int &ndep) {
-    if (ACC == 2) {  // per-photon update: the prefilter (round-start radius) only narrows the candidates down
-        deposit_u1(exact_hit(H, hl, rec), hidx, hot, hp_f, acc, U, ndep);
-        return;
-    }
-    const float ddx = q.x - H.f[0][hl], ddy = q.y - H.f[1][hl], ddz = q.z - H.f[2][hl];
+// A pair the normal filter rejects is dropped; a pair both filters accept is deposited without touching the hitpoint's exact record.
+// Only pairs in the thin shells in between (about 1e-3 of them) take the reference's fp64 test.
+enum { PAIR_REJECT, PAIR_ACCEPT, PAIR_EXACT };
+__device__ __forceinline__ int decide_pair_f32(float4 q, float4 qn, float hx, float hy, float hz, float nx, float ny, float nz) {
+    const float ddx = q.x - hx, ddy = q.y - hy, ddz = q.z - hz;
     const float s = fmaf(ddz, ddz, fmaf(ddy, ddy, ddx * ddx));
-    const float nx = H.f[3][hl], ny = H.f[4][hl], nz = H.f[5][hl];
     const float dn = fmaf(qn.z, nz, fmaf(qn.y, ny, qn.x * nx));
     const float sn = fmaf(fabsf(qn.z), fabsf(nz), fmaf(fabsf(qn.y), fabsf(ny), fabsf(qn.x * nx)));
     const float mg = fmaf(1e-6f, sn, 1e-9f);
     const float eps = (float)CGRT_EPS;
-    if (dn < eps - mg) return;  // the normal test fails whatever the distance
-    if (s <= qn.w && dn > eps + mg) {
-        if (ACC == 0) {
-            const double2 *fp = reinterpret_cast<const double2 *>(hp_f + 4 * (size_t)hidx);
-            double2 f0 = __ldg(fp), f1 = __ldg(fp + 1);
-            const HitShared<0> &H0 = reinterpret_cast<const HitShared<0> &>(H);
-            d3 cc = (mk(f0.x, f0.y, f1.x) * mk(H0.v[6][hl], H0.v[7][hl], H0.v[8][hl])) * (1.0 / CGRT_PI);
-            deposit_add<0>(acc, hidx, cc);
-        } else if (ACC == 1) {
-            const HitShared<1> &H1 = reinterpret_cast<const HitShared<1> &>(H);
-            const float ipi = (float)(1.0 / CGRT_PI);
-            float *ap = reinterpret_cast<float *>(acc) + 4 * (size_t)hidx;
-            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(ap), "f"((qf.x * H1.f[6][hl]) * ipi), "f"((qf.y * H1.f[7][hl]) * ipi),
-                         "f"((qf.z * H1.f[8][hl]) * ipi), "f"(1.0f)
-                         : "memory");
-        }
+    if (dn < eps - mg) return PAIR_REJECT;  // the normal test fails whatever the distance
+    return (s <= qn.w && dn > eps + mg) ? PAIR_ACCEPT : PAIR_EXACT;
+}
+
+// One queued pair of the fp64-accumulator modes, its hit in the warp's shared copy. An accepted pair deposits f from global times the
+// flux of the shared fp64 record: the deposited value is the reference's.
+template <int ACC>
+__device__ __forceinline__ void deposit_pair(const HitShared &H, uint32_t hl, uint32_t hidx, float4 q, float4 qn, const HpHot *__restrict__ hot,
+                                             const double *__restrict__ hp_f, void *__restrict__ acc, const U1State &U, unsigned int &ndep) {
+    static_assert(ACC != 1, "the float-accumulator mode decides its pairs in photon_deposit_kernel's walk");
+    if (ACC == 2) {  // per-photon update: the prefilter (round-start radius) only narrows the candidates down
+        deposit_u1(exact_hit(H, hl), hidx, hot, hp_f, acc, U, ndep);
+        return;
+    }
+    const int d = decide_pair_f32(q, qn, H.f[0][hl], H.f[1][hl], H.f[2][hl], H.f[3][hl], H.f[4][hl], H.f[5][hl]);
+    if (d == PAIR_REJECT) return;
+    if (d == PAIR_ACCEPT) {
+        const double2 *fp = reinterpret_cast<const double2 *>(hp_f + 4 * (size_t)hidx);
+        double2 f0 = __ldg(fp), f1 = __ldg(fp + 1);
+        d3 cc = (mk(f0.x, f0.y, f1.x) * mk(H.v[6][hl], H.v[7][hl], H.v[8][hl])) * (1.0 / CGRT_PI);
+        deposit_add<0>(acc, hidx, cc);
         ndep++;
         return;
     }
-    deposit_exact<ACC == 2 ? 0 : ACC>(exact_hit(H, hl, rec), hidx, hot, hp_f, acc, ndep);
+    deposit_exact<0>(exact_hit(H, hl), hidx, hot, hp_f, acc, ndep);
 }
 
 template <int ACC>
@@ -960,10 +947,10 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
     __shared__ float4 cf_all[ACC == 1 ? NW : 1][64];
     __shared__ uint32_t cidx_all[NW][64];
     __shared__ uint32_t queue_all[NW][64];
-    __shared__ HitShared<ACC> hit_all[NW];
+    __shared__ HitShared hit_all[ACC == 1 ? 1 : NW];
     const int lane = threadIdx.x & 31;
     const int wib = threadIdx.x >> 5;
-    HitShared<ACC> &H = hit_all[wib];
+    HitShared &H = hit_all[ACC == 1 ? 0 : wib];
     float4 *cpre = cpre_all[wib];
     float4 *cnrm = cnrm_all[wib];
     float4 *cf = cf_all[ACC == 1 ? wib : 0];
@@ -980,12 +967,13 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
     bool st_ok = false;
     const size_t n_slots = (size_t)__ldg(n_valid);
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&ctr->gathered_hits, (unsigned long long)n_slots);
-    // one exact step: 32 queued pairs (fewer at the end of a stage), one per lane
-    auto step = [&](int first, int count) {
+    // one exact step of the pair queue (ACC 0, 2): 32 queued pairs (fewer at the end of a stage), one per lane. Generic, so that its body is
+    // only compiled where it is called.
+    auto step = [&](auto first, int count) {
         if (lane < count) {
             const uint32_t e = queue[first + lane];
             const uint32_t hl = e & 31u, b = e >> 8;
-            deposit_pair<ACC>(H, hl, cidx[b], cpre[b], cnrm[b], ACC == 1 ? cf[b] : make_float4(0.f, 0.f, 0.f, 0.f), rec, hot, hp_f, acc, U, ndep);
+            deposit_pair<ACC>(H, hl, cidx[b], cpre[b], cnrm[b], hot, hp_f, acc, U, ndep);
         }
     };
     // spans are handed out from a global cursor (n_valid[1], zeroed by bin_scan_sums_kernel); the next one is requested before the
@@ -1026,10 +1014,9 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
                     ix = (int)(uint32_t)cxy; iy = (int)(uint32_t)(cxy >> 32); iz = (int)(uint32_t)__double_as_longlong(r2.z);
                     H.f[0][lane] = hx; H.f[1][lane] = hy; H.f[2][lane] = hz;
                     H.f[3][lane] = (float)r0.w; H.f[4][lane] = (float)r1.x; H.f[5][lane] = (float)r1.y;
-                    HitShared<0> &H0 = reinterpret_cast<HitShared<0> &>(H);
-                    H0.v[0][lane] = r0.x; H0.v[1][lane] = r0.y; H0.v[2][lane] = r0.z;
-                    H0.v[3][lane] = r0.w; H0.v[4][lane] = r1.x; H0.v[5][lane] = r1.y;
-                    H0.v[6][lane] = r1.z; H0.v[7][lane] = r1.w; H0.v[8][lane] = r2.x;
+                    H.v[0][lane] = r0.x; H.v[1][lane] = r0.y; H.v[2][lane] = r0.z;
+                    H.v[3][lane] = r0.w; H.v[4][lane] = r1.x; H.v[5][lane] = r1.y;
+                    H.v[6][lane] = r1.z; H.v[7][lane] = r1.w; H.v[8][lane] = r2.x;
                 }
             }
             __syncwarp();
@@ -1150,29 +1137,21 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
                         // Float accumulators: every lane walks the candidates that passed its own prefilter, its hit in registers — no pair
                         // queue and no shared-memory copy of the hits. The lanes idle while the busiest one finishes (4.8 pairs per hit
                         // on average, ~10 at most), but the shared-memory traffic of the queue form costs more on the pipe that bounds
-                        // this kernel (c3: 5.55 -> 5.42 ms, c2: 1.55 -> 1.44 ms). A pair is decided exactly like deposit_pair decides it.
+                        // this kernel (c3: 5.55 -> 5.42 ms, c2: 1.55 -> 1.44 ms). An accepted pair deposits from the fp32 copy of f.
                         unsigned int mine = 0;
                         while (m_lo | m_hi) {
                             int b;
                             if (m_lo) { b = __ffs(m_lo) - 1; m_lo &= m_lo - 1; }
                             else { b = 32 + __ffs(m_hi) - 1; m_hi &= m_hi - 1; }
                             mine++;
-                            const float4 q = cpre[b], qn4 = cnrm[b];
-                            const float ddx = q.x - hx, ddy = q.y - hy, ddz = q.z - hz;
-                            const float s2 = fmaf(ddz, ddz, fmaf(ddy, ddy, ddx * ddx));
-                            const float dn = fmaf(qn4.z, hown[2], fmaf(qn4.y, hown[1], qn4.x * hown[0]));
-                            const float sn = fmaf(fabsf(qn4.z), fabsf(hown[2]), fmaf(fabsf(qn4.y), fabsf(hown[1]), fabsf(qn4.x * hown[0])));
-                            const float mg = fmaf(1e-6f, sn, 1e-9f);
-                            const float eps = (float)CGRT_EPS;
-                            if (dn < eps - mg) continue;
+                            const int d = decide_pair_f32(cpre[b], cnrm[b], hx, hy, hz, hown[0], hown[1], hown[2]);
+                            if (d == PAIR_REJECT) continue;
                             const uint32_t hidx = cidx[b];
-                            if (s2 <= qn4.w && dn > eps + mg) {
+                            if (d == PAIR_ACCEPT) {
                                 const float4 qf = cf[b];
                                 const float ipi = (float)(1.0 / CGRT_PI);
-                                float *ap = reinterpret_cast<float *>(acc) + 4 * (size_t)hidx;
-                                asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(ap), "f"((qf.x * hown[3]) * ipi), "f"((qf.y * hown[4]) * ipi),
-                                             "f"((qf.z * hown[5]) * ipi), "f"(1.0f)
-                                             : "memory");
+                                red_add_v4(reinterpret_cast<float *>(acc) + 4 * (size_t)hidx, (qf.x * hown[3]) * ipi, (qf.y * hown[4]) * ipi,
+                                           (qf.z * hown[5]) * ipi, 1.0f);
                                 ndep++;
                             } else {
                                 // the thin shells the float filters cannot decide: the reference's fp64 test on the record itself
@@ -1302,6 +1281,23 @@ __global__ void __launch_bounds__(256) bin_scatter_kernel(const uint32_t *__rest
 // K12: per-round radius / flux update (main.cpp:119-122 batched over a round, SURVEY Q1 "U2"):
 //   g = (n a + a M) / (n a + M);  flux = (flux + dflux) g;  r2 *= g;  n += M.   Clears the accumulators.
 // =================================================================================================================
+__device__ __forceinline__ double u2_gain(int n, double m, double alpha) {
+    double na = n * alpha;
+    return (na + alpha * m) / (na + m);
+}
+// The rule for hitpoint k, which accepted m > 0 photons carrying dflux = (dx, dy, dz) this round.
+__device__ __forceinline__ void round_update_tail(const HpArrays &A, unsigned int k, double alpha, double dx, double dy, double dz, double m) {
+    int cnt = A.cnt[k];
+    double g = u2_gain(cnt, m, alpha);
+    double *fl = A.flux + 4 * (size_t)k;
+    fl[0] = (fl[0] + dx) * g;
+    fl[1] = (fl[1] + dy) * g;
+    fl[2] = (fl[2] + dz) * g;
+    const HpHot hh = A.hot[k];
+    set_radius(A, k, hh, hh.r2 * g);
+    A.cnt[k] = cnt + (int)m;
+}
+
 template <int ACC>
 __global__ void round_update_kernel(unsigned int n, double alpha, HpArrays A, void *__restrict__ acc) {
     unsigned int k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1318,21 +1314,7 @@ __global__ void round_update_kernel(unsigned int n, double alpha, HpArrays A, vo
         dx = a.x; dy = a.y; dz = a.z; m = a.w;
         *ap = make_float4(0, 0, 0, 0);
     }
-    if (m > 0) {
-        int cnt = A.cnt[k];
-        double na = cnt * alpha;
-        double g = (na + alpha * m) / (na + m);
-        double *fl = A.flux + 4 * (size_t)k;
-        fl[0] = (fl[0] + dx) * g;
-        fl[1] = (fl[1] + dy) * g;
-        fl[2] = (fl[2] + dz) * g;
-        HpHot hh = A.hot[k];
-        hh.r2 *= g;
-        A.hot[k].r2 = hh.r2;
-        A.pre[k] = make_prefilter(hh.px, hh.py, hh.pz, hh.r2);
-        A.pre_n[k].w = prefilter_inner(hh.px, hh.py, hh.pz, hh.r2);
-        A.cnt[k] = cnt + (int)m;
-    }
+    if (m > 0) round_update_tail(A, k, alpha, dx, dy, dz, m);
 }
 
 // =================================================================================================================
@@ -1362,8 +1344,7 @@ __global__ void sppm_fold_kernel(unsigned int npix, double alpha, const uint32_t
     }
     if (m > 0) {
         int c = cnt[p];
-        double na = c * alpha;
-        double g = (na + alpha * m) / (na + m);
+        double g = u2_gain(c, m, alpha);
         double *t = tau + 4 * (size_t)p;
         t[0] = (t[0] + dx) * g;
         t[1] = (t[1] + dy) * g;
@@ -1423,7 +1404,9 @@ __global__ void __launch_bounds__(64) peer_reduce_update_kernel(unsigned int n, 
                                                                 void *__restrict__ clear_next) {
     unsigned int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
-    double dx = 0, dy = 0, dz = 0, m = 0;
+    // The declaration order reaches ptxas's register assignment of <0>: this one compiles to the code that was timed (other orders
+    // compile differently, and re-timing this kernel takes two GPUs).
+    double dz = 0, m = 0, dy = 0, dx = 0;
     if (ACC == 0) {
         for (int g0 = 0; g0 < world; g0 += 4) {
             double2 lo[4], hi[4];
@@ -1454,21 +1437,7 @@ __global__ void __launch_bounds__(64) peer_reduce_update_kernel(unsigned int n, 
         dx = fx; dy = fy; dz = fz; m = fm;
         reinterpret_cast<float4 *>(clear_next)[k] = make_float4(0, 0, 0, 0);
     }
-    if (m > 0) {  // round_update_kernel's tail, written out: shared as an inline helper it changes this kernel's register allocation
-        int cnt = A.cnt[k];
-        double na = cnt * alpha;
-        double g = (na + alpha * m) / (na + m);
-        double *fl = A.flux + 4 * (size_t)k;
-        fl[0] = (fl[0] + dx) * g;
-        fl[1] = (fl[1] + dy) * g;
-        fl[2] = (fl[2] + dz) * g;
-        HpHot hh = A.hot[k];
-        hh.r2 *= g;
-        A.hot[k].r2 = hh.r2;
-        A.pre[k] = make_prefilter(hh.px, hh.py, hh.pz, hh.r2);
-        A.pre_n[k].w = prefilter_inner(hh.px, hh.py, hh.pz, hh.r2);
-        A.cnt[k] = cnt + (int)m;
-    }
+    if (m > 0) round_update_tail(A, k, alpha, dx, dy, dz, m);
 }
 
 // Per-photon update mode: the counts are live; a "round update" only folds them into what the next round's filters and the image read:
@@ -1481,12 +1450,8 @@ __global__ void round_update_u1_kernel(unsigned int n, HpArrays A, const double 
     const double r2 = r2tab[cnt < cap ? cnt : cap - 1];
     double *fl = A.flux + 4 * (size_t)k;
     fl[0] = S[4 * (size_t)k] * r2; fl[1] = S[4 * (size_t)k + 1] * r2; fl[2] = S[4 * (size_t)k + 2] * r2;
-    HpHot hh = A.hot[k];
-    if (hh.r2 != r2) {
-        A.hot[k].r2 = r2;
-        A.pre[k] = make_prefilter(hh.px, hh.py, hh.pz, r2);
-        A.pre_n[k].w = prefilter_inner(hh.px, hh.py, hh.pz, r2);
-    }
+    const HpHot hh = A.hot[k];
+    if (hh.r2 != r2) set_radius(A, k, hh, r2);
 }
 
 // =================================================================================================================
