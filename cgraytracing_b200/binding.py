@@ -119,6 +119,7 @@ class Context:
         self.close()
 
     def set_config(self, cfg, accum_mode=None):
+        """accum_mode (default cfg.accum_mode, else 0): 0 fp64, 1 float, 2 fixed point (bit-reproducible; include/cgrt.h)."""
         k = CgrtConfig()
         self.L.cgrt_default_config(C.byref(k))
         for f in ("width", "height", "max_depth", "num_of_samples", "use_dof", "hashsize"):

@@ -245,6 +245,7 @@ struct cgrt_ctx {
     int cull = 1;
     Counters *d_ctr = nullptr;
     TravCounters *d_tc = nullptr;
+    int *d_fxerr = nullptr;  // fixed-point accumulators: FIX_ERR_* bits raised by the deposit and update kernels; stays raised
     uint64_t launches = 0;
     unsigned int deposit_grid = 148 * 8;  // resident deposit blocks: 8 x 256 threads per SM
     int profiling = 0;   // 1: time every photon kernel with events (serialises host and device at the end of each pass)
@@ -596,8 +597,23 @@ int ensure_queue(cgrt_ctx *ctx, int which, size_t cap) {
     ctx->q_cap[which] = cap;
     return 0;
 }
-// float accumulators with the per-round update: the 64-byte record (DepositRecC); everything else keeps the 96-byte fp64 record
-inline bool compact_records(const cgrt_ctx *ctx) { return ctx->cfg.accum_mode == 1 && ctx->cfg.update_mode != 0; }
+// float or fixed-point accumulators with the per-round update: the 64-byte record (DepositRecC) of the float walk; everything else keeps
+// the 96-byte fp64 record
+inline bool compact_records(const cgrt_ctx *ctx) { return ctx->cfg.accum_mode != 0 && ctx->cfg.update_mode != 0; }
+// bytes of one accumulator lane: fp64 (accum_mode 0), float (1), int64 fixed point (2)
+inline size_t acc_elem(const cgrt_ctx *ctx) { return ctx->cfg.accum_mode == 1 ? sizeof(float) : sizeof(double); }
+// The fixed-point mode's error word; the streams that write it must have been synchronised.
+int check_fixed(cgrt_ctx *ctx) {
+    if (ctx->cfg.accum_mode != 2) return 0;
+    int e = 0;
+    CK(cudaMemcpy(&e, ctx->d_fxerr, sizeof e, cudaMemcpyDeviceToHost));
+    if (e & FIX_ERR_VALUE)
+        FAIL(CGRT_ERR_CAPACITY, "fixed-point accumulators: a deposit value f * flux / pi above 2^16 (or not a number); the flux sums are invalid");
+    if (e & FIX_ERR_COUNT)
+        FAIL(CGRT_ERR_CAPACITY, "fixed-point accumulators: more than 2^24 photons accepted by one hitpoint (SPPM: one pixel) in one round; "
+                                "the flux sums are invalid");
+    return 0;
+}
 int ensure_photon_buffers(cgrt_ctx *ctx, size_t photons, size_t slots) {
     const size_t rb = deposit_rec_bytes(compact_records(ctx));
     bool fresh = false;
@@ -749,7 +765,7 @@ void peer_release(cgrt_ctx *ctx) {
 // =================================================================================================================
 extern "C" {
 
-int cgrt_version(void) { return 102; }
+int cgrt_version(void) { return 103; }
 
 void cgrt_default_config(cgrt_config *c) {
     memset(c, 0, sizeof *c);
@@ -809,7 +825,8 @@ int cgrt_create(int device, cgrt_ctx **out) {
         delete ctx;
         return CGRT_ERR_CUDA;
     }
-    if (dalloc(ctx, &ctx->d_hp_count, 1) || dalloc(ctx, &ctx->d_qcount, 16) || dalloc(ctx, &ctx->d_ctr, 1) || dalloc(ctx, &ctx->d_tc, 1)) {
+    if (dalloc(ctx, &ctx->d_hp_count, 1) || dalloc(ctx, &ctx->d_qcount, 16) || dalloc(ctx, &ctx->d_ctr, 1) || dalloc(ctx, &ctx->d_tc, 1) ||
+        dalloc(ctx, &ctx->d_fxerr, 1)) {
         delete ctx;
         return CGRT_ERR_CUDA;
     }
@@ -817,6 +834,7 @@ int cgrt_create(int device, cgrt_ctx **out) {
     cudaMemsetAsync(ctx->d_qcount, 0, 16 * sizeof(unsigned int), ctx->stream);
     cudaMemsetAsync(ctx->d_ctr, 0, sizeof(Counters), ctx->stream);
     cudaMemsetAsync(ctx->d_tc, 0, sizeof(TravCounters), ctx->stream);
+    cudaMemsetAsync(ctx->d_fxerr, 0, sizeof(int), ctx->stream);
     cudaStreamSynchronize(ctx->stream);
     *out = ctx;
     return CGRT_OK;
@@ -870,6 +888,7 @@ int cgrt_set_config(cgrt_ctx *ctx, const cgrt_config *cfg) {
     if (ctx->hp_count) FAIL(CGRT_ERR_INVALID, "config cannot change after the eye pass");
     if (ctx->sppm) FAIL(CGRT_ERR_INVALID, "config cannot change while SPPM is on (the pixel statistics are sized and seeded from it)");
     if (cfg->update_mode != 0 && cfg->update_mode != 1) FAIL(CGRT_ERR_INVALID, "config: update_mode must be 0 (per photon) or 1 (per round)");
+    if (cfg->accum_mode < 0 || cfg->accum_mode > 2) FAIL(CGRT_ERR_INVALID, "config: accum_mode must be 0 (fp64), 1 (float) or 2 (fixed point)");
     if (cfg->update_mode == 0 && ctx->comm) FAIL(CGRT_ERR_INVALID, "config: the per-photon update is not shard-invariant (one GPU only)");
     ctx->cfg = *cfg;
     if (cfg->update_mode == 0) ctx->cfg.accum_mode = 0;  // per-photon update: fp64 sums S = sum c / r2_old in the accumulator buffer
@@ -891,7 +910,7 @@ int cgrt_synchronize(cgrt_ctx *ctx) {
         CK(cudaMemcpy(&perr, ctx->peer.block + peer_err_off(ctx->peer), sizeof perr, cudaMemcpyDeviceToHost));
         if (perr) FAIL(CGRT_ERR_NCCL, "peer exchange: rank " + std::to_string(perr - 1) + " did not publish its round in time");
     }
-    return CGRT_OK;
+    return check_fixed(ctx);
 }
 
 // ---- scene ---------------------------------------------------------------------------------------------------------
@@ -1313,10 +1332,10 @@ static int build_grid_impl(cgrt_ctx *ctx) {
     // The arrays the deposit kernel gathers from — prefilter, exact records, f, accumulators — live in one slab. (Marking the slab
     // persisting in L2 with an access-policy window was measured: the deposit kernel did not move (11.0 ms, it is not bound by L2
     // misses) while the counting sort lost its L2-resident cursors (1.2 -> 4.2 ms), so no window is set.)
-    size_t acc_bytes = (size_t)n * 4 * (ctx->cfg.accum_mode == 0 ? sizeof(double) : sizeof(float));
+    size_t acc_bytes = (size_t)n * 4 * acc_elem(ctx);
     {
         auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-        const size_t acc_cap = m * 4 * (ctx->cfg.accum_mode == 0 ? sizeof(double) : sizeof(float));
+        const size_t acc_cap = m * 4 * acc_elem(ctx);
         size_t o_pre = 0, o_pren = o_pre + up(m * sizeof(float4)), o_pref = o_pren + up(m * sizeof(float4));
         size_t o_hot = o_pref + up(m * sizeof(float4)), o_f = o_hot + up(m * sizeof(HpHot));
         size_t o_acc = o_f + up(m * 4 * sizeof(double)), total = o_acc + up(acc_cap);
@@ -1513,16 +1532,19 @@ static int photon_pass_impl(cgrt_ctx *ctx, uint64_t first, uint64_t count, const
             size_t want = (spans * 32 + CGRT_DEPOSIT_BLOCK - 1) / CGRT_DEPOSIT_BLOCK;
             unsigned int dblocks = (unsigned int)(want < (size_t)ctx->deposit_grid ? want : (size_t)ctx->deposit_grid);
             U1State U1;
-            U1.cnt = ctx->A.cnt; U1.r2tab = ctx->r2tab; U1.cap = ctx->r2cap;
+            U1.cnt = ctx->A.cnt; U1.r2tab = ctx->r2tab; U1.cap = ctx->r2cap; U1.err = ctx->d_fxerr;
             if (ctx->cfg.update_mode == 0)
                 photon_deposit_kernel<2><<<dblocks, CGRT_DEPOSIT_BLOCK, 0, D>>>(P, reinterpret_cast<const DepositRec *>(B.rec), B.perm, B.nvalid, ctx->cell_start, ctx->A.pre, ctx->A.pre_n,
                                                                                 ctx->A.pre_f, ctx->A.hot, ctx->A.f, ctx->acc, ctx->d_ctr, U1);
             else if (ctx->cfg.accum_mode == 0)
                 photon_deposit_kernel<0><<<dblocks, CGRT_DEPOSIT_BLOCK, 0, D>>>(P, reinterpret_cast<const DepositRec *>(B.rec), B.perm, B.nvalid, ctx->cell_start, ctx->A.pre, ctx->A.pre_n,
                                                                                 ctx->A.pre_f, ctx->A.hot, ctx->A.f, ctx->acc, ctx->d_ctr, U1);
-            else
+            else if (ctx->cfg.accum_mode == 1)
                 photon_deposit_kernel<1><<<dblocks, CGRT_DEPOSIT_BLOCK, 0, D>>>(P, reinterpret_cast<const DepositRec *>(B.rec), B.perm, B.nvalid, ctx->cell_start, ctx->A.pre, ctx->A.pre_n,
                                                                                 ctx->A.pre_f, ctx->A.hot, ctx->A.f, ctx->acc, ctx->d_ctr, U1);
+            else
+                photon_deposit_kernel<ACC_FIXED><<<dblocks, CGRT_DEPOSIT_BLOCK, 0, D>>>(P, reinterpret_cast<const DepositRec *>(B.rec), B.perm, B.nvalid, ctx->cell_start,
+                                                                                        ctx->A.pre, ctx->A.pre_n, ctx->A.pre_f, ctx->A.hot, ctx->A.f, ctx->acc, ctx->d_ctr, U1);
             ctx->launches++;
         } else {
             stamp(6);
@@ -1602,7 +1624,8 @@ static int allreduce_on(cgrt_ctx *ctx, void *comm, cudaStream_t st) {
     NcclApi &N = nccl_api();
     if (!N.ok) FAIL(CGRT_ERR_NCCL, "NCCL is not available: " + N.why);
     if (ctx->nhp == 0) return CGRT_OK;
-    int r = N.AllReduce(ctx->acc, ctx->acc, (size_t)ctx->nhp * 4, ctx->cfg.accum_mode == 0 ? NCCL_FLOAT64 : NCCL_FLOAT32, NCCL_SUM, comm, st);
+    const int type = ctx->cfg.accum_mode == 0 ? NCCL_FLOAT64 : ctx->cfg.accum_mode == 1 ? NCCL_FLOAT32 : NCCL_INT64;
+    int r = N.AllReduce(ctx->acc, ctx->acc, (size_t)ctx->nhp * 4, type, NCCL_SUM, comm, st);
     if (r != 0) return nccl_fail(ctx, r, "ncclAllReduce");
     ctx->launches++;
     return CGRT_OK;
@@ -1630,7 +1653,7 @@ int cgrt_peer_export(cgrt_ctx *ctx, void *handle128) {
     CKS(join_update(ctx));
     CK(cudaStreamSynchronize(ctx->stream));
     cgrt_ctx::Peer &P = ctx->peer;
-    const size_t elem = ctx->cfg.accum_mode == 0 ? sizeof(double) : sizeof(float);
+    const size_t elem = acc_elem(ctx);
     P.acc_bytes = (((size_t)ctx->nhp * 4 * elem) + 255) & ~(size_t)255;
     if (P.acc_bytes == 0) P.acc_bytes = 256;
     P.bytes = 2 * P.acc_bytes + 2 * CGRT_MAX_PEERS * sizeof(int) + 256;
@@ -1797,8 +1820,11 @@ int cgrt_round_update(cgrt_ctx *ctx) {
         if (n > 0) {
             if (ctx->cfg.accum_mode == 0)
                 sppm_fold_kernel<0><<<nblk(npix, 256), 256, 0, ctx->stream>>>(npix, ctx->P.alpha, ctx->pix_start, ctx->pix_perm, ctx->acc, ctx->pix_tau, ctx->pix_r2, ctx->pix_cnt);
-            else
+            else if (ctx->cfg.accum_mode == 1)
                 sppm_fold_kernel<1><<<nblk(npix, 256), 256, 0, ctx->stream>>>(npix, ctx->P.alpha, ctx->pix_start, ctx->pix_perm, ctx->acc, ctx->pix_tau, ctx->pix_r2, ctx->pix_cnt);
+            else
+                sppm_fold_fixed_kernel<<<nblk(npix, 256), 256, 0, ctx->stream>>>(npix, ctx->P.alpha, ctx->pix_start, ctx->pix_perm, reinterpret_cast<long long *>(ctx->acc),
+                                                                                 ctx->pix_tau, ctx->pix_r2, ctx->pix_cnt, ctx->d_fxerr);
             ctx->launches++;
             CK(cudaGetLastError());
         }
@@ -1833,7 +1859,9 @@ int cgrt_round_update(cgrt_ctx *ctx) {
         void *clear_next = P.block + (size_t)(P.parity ^ 1) * P.acc_bytes;
         if (n > 0) {
             if (ctx->cfg.accum_mode == 0) peer_reduce_update_kernel<0><<<nblk(n, 64), 64, 0, V>>>(n, ctx->P.alpha, ctx->A, accs, P.world, clear_next);
-            else peer_reduce_update_kernel<1><<<nblk(n, 64), 64, 0, V>>>(n, ctx->P.alpha, ctx->A, accs, P.world, clear_next);
+            else if (ctx->cfg.accum_mode == 1) peer_reduce_update_kernel<1><<<nblk(n, 64), 64, 0, V>>>(n, ctx->P.alpha, ctx->A, accs, P.world, clear_next);
+            else peer_reduce_update_fixed_kernel<<<nblk(n, 64), 64, 0, V>>>(n, ctx->P.alpha, ctx->A, accs, P.world, reinterpret_cast<long long *>(clear_next),
+                                                                            ctx->d_fxerr);
         }
         ctx->launches += 3;
         CK(cudaGetLastError());
@@ -1860,7 +1888,8 @@ int cgrt_round_update(cgrt_ctx *ctx) {
         }
     } else if (n > 0) {
         if (ctx->cfg.accum_mode == 0) round_update_kernel<0><<<nblk(n, 256), 256, 0, U>>>(n, ctx->P.alpha, ctx->A, ctx->acc);
-        else round_update_kernel<1><<<nblk(n, 256), 256, 0, U>>>(n, ctx->P.alpha, ctx->A, ctx->acc);
+        else if (ctx->cfg.accum_mode == 1) round_update_kernel<1><<<nblk(n, 256), 256, 0, U>>>(n, ctx->P.alpha, ctx->A, ctx->acc);
+        else round_update_fixed_kernel<<<nblk(n, 256), 256, 0, U>>>(n, ctx->P.alpha, ctx->A, reinterpret_cast<long long *>(ctx->acc), ctx->d_fxerr);
         ctx->launches++;
         CK(cudaGetLastError());
     }
@@ -1895,7 +1924,7 @@ int cgrt_gather_image(cgrt_ctx *ctx, double n_emitted, double *rgb, uint8_t *rgb
     CKS(download_free(ctx, rgb, d_rgb, npix * 3));
     if (rgb8) CKS(download_free(ctx, rgb8, d_rgb8, npix * 3));
     timer.stop();
-    return CGRT_OK;
+    return check_fixed(ctx);
 }
 
 // ---- stochastic progressive photon mapping --------------------------------------------------------------------------
@@ -1963,7 +1992,7 @@ int cgrt_sppm_download_pixels(cgrt_ctx *ctx, double *tau, double *r2, int32_t *n
     }
     if (r2) CK(cudaMemcpy(r2, ctx->pix_r2, npix * sizeof(double), cudaMemcpyDeviceToHost));
     if (n) CK(cudaMemcpy(n, ctx->pix_cnt, npix * sizeof(int), cudaMemcpyDeviceToHost));
-    return CGRT_OK;
+    return check_fixed(ctx);
 }
 
 // ---- multi-run averaging (average.cpp) ------------------------------------------------------------------------------
@@ -2041,7 +2070,7 @@ int cgrt_download_hitpoints(cgrt_ctx *ctx, double *pos, double *normal, double *
     if (hw) CK(cudaMemcpy(hw, ctx->A.hw, m * 2 * sizeof(int), cudaMemcpyDeviceToHost));
     if (key) CK(cudaMemcpy(key, ctx->A.key, m * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     if (seq) CK(cudaMemcpy(seq, ctx->A.seq, m * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-    return CGRT_OK;
+    return check_fixed(ctx);
 }
 
 int cgrt_download_accum(cgrt_ctx *ctx, double *dflux, double *mcount) {
@@ -2058,15 +2087,23 @@ int cgrt_download_accum(cgrt_ctx *ctx, double *dflux, double *mcount) {
             if (dflux) { dflux[3 * i] = a[4 * i]; dflux[3 * i + 1] = a[4 * i + 1]; dflux[3 * i + 2] = a[4 * i + 2]; }
             if (mcount) mcount[i] = a[4 * i + 3];
         }
-    } else {
+    } else if (ctx->cfg.accum_mode == 1) {
         std::vector<float> a(m * 4);
         CK(cudaMemcpy(a.data(), ctx->acc, m * 4 * sizeof(float), cudaMemcpyDeviceToHost));
         for (size_t i = 0; i < m; i++) {
             if (dflux) { dflux[3 * i] = a[4 * i]; dflux[3 * i + 1] = a[4 * i + 1]; dflux[3 * i + 2] = a[4 * i + 2]; }
             if (mcount) mcount[i] = a[4 * i + 3];
         }
+    } else {  // fixed point: sum q * 2^-22 and M, as the round update reads them
+        std::vector<long long> a(m * 4);
+        CK(cudaMemcpy(a.data(), ctx->acc, m * 4 * sizeof(long long), cudaMemcpyDeviceToHost));
+        for (size_t i = 0; i < m; i++) {
+            if (dflux)
+                for (int c = 0; c < 3; c++) dflux[3 * i + c] = (double)a[4 * i + c] * CGRT_FIX_INV_SCALE;
+            if (mcount) mcount[i] = (double)a[4 * i + 3];
+        }
     }
-    return CGRT_OK;
+    return check_fixed(ctx);
 }
 
 int cgrt_download_grid(cgrt_ctx *ctx, uint32_t *cell_start) {

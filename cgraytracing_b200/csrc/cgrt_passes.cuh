@@ -786,6 +786,7 @@ __global__ void __launch_bounds__(CGRT_PHOTON_BLOCK, CGRT_TRACE_MINB) photon_tra
 //   ACC 0 (fp64 atomics {dflux.xyz, m}) and 2 (per-photon update, deposit_u1): the batch is copied to shared memory (HitShared); the
 //         surviving pairs are drained into a per-warp queue and processed 32 at a time by ALL lanes (deposit_pair).
 //   ACC 1 (one red.global.add.v4.f32 per deposit): every lane walks its own surviving pairs, its hit in registers.
+//   ACC_FIXED (accum_mode 2): the walk of ACC 1 with the fixed-point deposit (deposit_fixed) of every accepted pair.
 // ---------------------------------------------------------------------------------------------------------------------
 #define CGRT_DEPOSIT_BLOCK 256
 #ifndef CGRT_DEPOSIT_MINB
@@ -862,6 +863,7 @@ struct U1State {
     int *cnt;              // accepted photons per hitpoint (HpArrays::cnt, live)
     const double *r2tab;   // r2 after n accepted photons, n < cap
     int cap;
+    int *err;              // fixed-point mode (ACC_FIXED): the context's error word (see deposit_fixed); unused by the other modes
 };
 __device__ __forceinline__ void deposit_u1(const ExactHit &e, uint32_t hidx, const HpHot *__restrict__ hot, const double *__restrict__ hp_f,
                                            void *__restrict__ acc, const U1State &U, unsigned int &ndep) {
@@ -908,6 +910,59 @@ __device__ __forceinline__ int decide_pair_f32(float4 q, float4 qn, float hx, fl
     return (s <= qn.w && dn > eps + mg) ? PAIR_ACCEPT : PAIR_EXACT;
 }
 
+// The deposit of an accepted pair in the float walk (accum_mode 1 and 2), per channel: the hitpoint's fp32 f (pre_f) times the photon's
+// fp32 flux (the compact record), times fp32 1/pi; round to nearest, never contracted (-fmad=false). The fixed-point mode deposits this
+// value for every accepted pair, the thin-shell pairs of the fp64 test included, so that it is a pure function of the pair.
+__device__ __forceinline__ float deposit_value_f32(float f, float flux) { return (f * flux) * (float)(1.0 / CGRT_PI); }
+
+// Fixed-point accumulators (accum_mode 2, template id ACC_FIXED): per hitpoint {sum q_x, sum q_y, sum q_z, M} as four int64, where
+// q = round-half-even(cf * 2^22) of the value cf above. Integer sums do not depend on the order of the adds, so the round's sums — and
+// with them flux, radii, counts and the image — are the same bits whatever the warp order, launch split, rank count or reduction.
+// Resolution 2^-22: every cf >= 2 is held exactly, a smaller one to within 2^-23. Range: cf <= 2^16 and M <= 2^24 keep every sum
+// <= 2^62; a deposit or a count outside it raises the context's error word (never a silent wrap), which the next synchronising call
+// reports. 2^24 is also where the float mode's count lane stops being exact. oracle_fixed/fixed_capi.cpp restates this definition.
+#define ACC_FIXED 3
+#define CGRT_FIX_SCALE 4194304.0f         /* 2^22 */
+#define CGRT_FIX_INV_SCALE (1.0 / 4194304.0)
+#define CGRT_FIX_MAX_VALUE 65536.0f       /* 2^16 */
+#define CGRT_FIX_MAX_COUNT 16777216ll     /* 2^24 */
+enum { FIX_ERR_VALUE = 1, FIX_ERR_COUNT = 2 };
+
+__device__ __forceinline__ long long fixed_q(float cf) { return __float2ll_rn(cf * CGRT_FIX_SCALE); }
+// The reds are inline PTX, not atomicAdd / atomicOr: for the builtins the compiler adds its warp-aggregation code around every atomic,
+// which took the walk of photon_deposit_kernel<ACC_FIXED> past its 64 registers (148 B of spill stores); with plain reds it has none.
+__device__ __forceinline__ void red_add_s64(long long *ap, long long v) {
+    asm volatile("red.global.add.u64 [%0], %1;" ::"l"(ap), "l"(v) : "memory");
+}
+// One accepted pair into hitpoint accumulator ap: three integer reds and the count (PTX has no vector integer red for sm_100a).
+__device__ __forceinline__ void deposit_fixed(long long *ap, float cx, float cy, float cz, int *err) {
+    if (!(cx <= CGRT_FIX_MAX_VALUE) || !(cy <= CGRT_FIX_MAX_VALUE) || !(cz <= CGRT_FIX_MAX_VALUE)) {  // also catches NaN
+        asm volatile("red.global.or.b32 [%0], %1;" ::"l"(err), "r"((int)FIX_ERR_VALUE) : "memory");
+        return;
+    }
+    red_add_s64(ap, fixed_q(cx));
+    red_add_s64(ap + 1, fixed_q(cy));
+    red_add_s64(ap + 2, fixed_q(cz));
+    red_add_s64(ap + 3, 1ll);
+}
+// The round's fixed-point sums {sq, M} of one hitpoint or pixel as the U2 rule's dflux and M; raises the error word when M > 2^24.
+__device__ __forceinline__ void fixed_to_update(long long sx, long long sy, long long sz, long long mc, int *err, double &dx, double &dy, double &dz,
+                                                double &m) {
+    if (mc > CGRT_FIX_MAX_COUNT) atomicOr(err, FIX_ERR_COUNT);
+    dx = (double)sx * CGRT_FIX_INV_SCALE; dy = (double)sy * CGRT_FIX_INV_SCALE; dz = (double)sz * CGRT_FIX_INV_SCALE;
+    m = (double)mc;
+}
+// The reference's fp64 test of one pair (main.cpp:116), from the hitpoint's exact record. It restates the test inside deposit_exact, which
+// keeps its own copy so that the kernels of accum_mode 0 and 1 compile to the code that was timed: the two must stay in step.
+__device__ __forceinline__ bool accept_exact(const ExactHit &e, uint32_t hidx, const HpHot *__restrict__ hot) {
+    const double2 *hp = reinterpret_cast<const double2 *>(hot + hidx);
+    double2 a0 = __ldg(hp), a1 = __ldg(hp + 1), b0 = __ldg(hp + 2), b1 = __ldg(hp + 3);
+    d3 hpos = mk(a0.x, a0.y, a1.x);
+    d3 hn = mk(b0.x, b0.y, b1.x);
+    d3 dd = hpos - e.X;
+    return (dot(hn, e.nrm) > CGRT_EPS) && (dot(dd, dd) <= a1.y);
+}
+
 // One queued pair of the fp64-accumulator modes, its hit in the warp's shared copy. An accepted pair deposits f from global times the
 // flux of the shared fp64 record: the deposited value is the reference's.
 template <int ACC>
@@ -942,18 +997,19 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
     // per warp: 64 staged candidates (fp32 filter records + hitpoint index) and the queue of (record, candidate) pairs that passed
     // the prefilter
     constexpr int NW = CGRT_DEPOSIT_BLOCK / 32;
+    constexpr bool WALK = ACC == 1 || ACC == ACC_FIXED;  // the float walk: compact records, every lane walks its own pairs
     __shared__ float4 cpre_all[NW][64];
     __shared__ float4 cnrm_all[NW][64];
-    __shared__ float4 cf_all[ACC == 1 ? NW : 1][64];
+    __shared__ float4 cf_all[WALK ? NW : 1][64];
     __shared__ uint32_t cidx_all[NW][64];
     __shared__ uint32_t queue_all[NW][64];
-    __shared__ HitShared hit_all[ACC == 1 ? 1 : NW];
+    __shared__ HitShared hit_all[WALK ? 1 : NW];
     const int lane = threadIdx.x & 31;
     const int wib = threadIdx.x >> 5;
-    HitShared &H = hit_all[ACC == 1 ? 0 : wib];
+    HitShared &H = hit_all[WALK ? 0 : wib];
     float4 *cpre = cpre_all[wib];
     float4 *cnrm = cnrm_all[wib];
-    float4 *cf = cf_all[ACC == 1 ? wib : 0];
+    float4 *cf = cf_all[WALK ? wib : 0];
     uint32_t *cidx = cidx_all[wib];
     uint32_t *queue = queue_all[wib];
     const unsigned int lt = (1u << lane) - 1u;
@@ -995,7 +1051,7 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
             uint32_t src_own = 0;
             if (valid) {
                 const uint32_t src = __ldcs(perm + j);
-                if (ACC == 1) {
+                if (WALK) {
                     // compact record: position and normal fp64, flux as three floats; the cell is recomputed from the position (hash.h:38-42).
                     // The float copy of the hit stays in this lane's registers: in this mode every lane walks its own surviving pairs.
                     const double2 *r = reinterpret_cast<const double2 *>(reinterpret_cast<const DepositRecC *>(rec) + src);
@@ -1088,7 +1144,7 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
                                 keep = fmaf(ez, ez, fmaf(ey, ey, ex * ex)) <= q.w;
                                 if (keep) {  // the other two filter records only for candidates that survive the cull (c5: deposit 89 -> 84 ms)
                                     q_n = __ldg(pre_n + hidx);
-                                    if (ACC == 1) q_f = __ldg(pre_f + hidx);
+                                    if (WALK) q_f = __ldg(pre_f + hidx);
                                 }
                             }
                             const unsigned int km = __ballot_sync(0xffffffffu, keep);
@@ -1096,7 +1152,7 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
                                 const int at = nc + __popc(km & lt);
                                 cpre[at] = q;
                                 cnrm[at] = q_n;
-                                if (ACC == 1) cf[at] = q_f;
+                                if (WALK) cf[at] = q_f;
                                 cidx[at] = hidx;
                             }
                             nc += __popc(km);
@@ -1133,7 +1189,7 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
                         }
                     }
                     if (!((grp >> lane) & 1u)) { m_lo = 0; m_hi = 0; }
-                    if constexpr (ACC == 1) {
+                    if constexpr (WALK) {
                         // Float accumulators: every lane walks the candidates that passed its own prefilter, its hit in registers — no pair
                         // queue and no shared-memory copy of the hits. The lanes idle while the busiest one finishes (4.8 pairs per hit
                         // on average, ~10 at most), but the shared-memory traffic of the queue form costs more on the pipe that bounds
@@ -1147,11 +1203,22 @@ __global__ void __launch_bounds__(CGRT_DEPOSIT_BLOCK, CGRT_DEPOSIT_MINB) photon_
                             const int d = decide_pair_f32(cpre[b], cnrm[b], hx, hy, hz, hown[0], hown[1], hown[2]);
                             if (d == PAIR_REJECT) continue;
                             const uint32_t hidx = cidx[b];
-                            if (d == PAIR_ACCEPT) {
+                            if constexpr (ACC == ACC_FIXED) {
+                                if (d == PAIR_EXACT) {  // the thin shells: the reference's fp64 test decides, the deposit is the same value
+                                    const double2 *r = reinterpret_cast<const double2 *>(reinterpret_cast<const DepositRecC *>(rec) + src_own);
+                                    const double2 r0 = __ldcs(r), r1 = __ldcs(r + 1), r2 = __ldcs(r + 2);
+                                    ExactHit e;
+                                    e.X = mk(r0.x, r0.y, r1.x); e.nrm = mk(r1.y, r2.x, r2.y);
+                                    if (!accept_exact(e, hidx, hot)) continue;
+                                }
                                 const float4 qf = cf[b];
-                                const float ipi = (float)(1.0 / CGRT_PI);
-                                red_add_v4(reinterpret_cast<float *>(acc) + 4 * (size_t)hidx, (qf.x * hown[3]) * ipi, (qf.y * hown[4]) * ipi,
-                                           (qf.z * hown[5]) * ipi, 1.0f);
+                                deposit_fixed(reinterpret_cast<long long *>(acc) + 4 * (size_t)hidx, deposit_value_f32(qf.x, hown[3]),
+                                              deposit_value_f32(qf.y, hown[4]), deposit_value_f32(qf.z, hown[5]), U.err);
+                                ndep++;
+                            } else if (d == PAIR_ACCEPT) {
+                                const float4 qf = cf[b];
+                                red_add_v4(reinterpret_cast<float *>(acc) + 4 * (size_t)hidx, deposit_value_f32(qf.x, hown[3]), deposit_value_f32(qf.y, hown[4]),
+                                           deposit_value_f32(qf.z, hown[5]), 1.0f);
                                 ndep++;
                             } else {
                                 // the thin shells the float filters cannot decide: the reference's fp64 test on the record itself
@@ -1316,6 +1383,17 @@ __global__ void round_update_kernel(unsigned int n, double alpha, HpArrays A, vo
     }
     if (m > 0) round_update_tail(A, k, alpha, dx, dy, dz, m);
 }
+// The same for the fixed-point accumulators (accum_mode 2).
+__global__ void round_update_fixed_kernel(unsigned int n, double alpha, HpArrays A, long long *__restrict__ acc, int *err) {
+    unsigned int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    longlong2 *ap = reinterpret_cast<longlong2 *>(acc + 4 * (size_t)k);
+    const longlong2 a = ap[0], b = ap[1];
+    ap[0] = make_longlong2(0, 0); ap[1] = make_longlong2(0, 0);
+    double dx, dy, dz, m;
+    fixed_to_update(a.x, a.y, b.x, b.y, err, dx, dy, dz, m);
+    if (m > 0) round_update_tail(A, k, alpha, dx, dy, dz, m);
+}
 
 // =================================================================================================================
 // SPPM fold: the U2 rule above per PIXEL. One thread per pixel walks the round's visible points of that pixel in canonical order
@@ -1342,6 +1420,31 @@ __global__ void sppm_fold_kernel(unsigned int npix, double alpha, const uint32_t
             *ap = make_float4(0, 0, 0, 0);
         }
     }
+    if (m > 0) {
+        int c = cnt[p];
+        double g = u2_gain(c, m, alpha);
+        double *t = tau + 4 * (size_t)p;
+        t[0] = (t[0] + dx) * g;
+        t[1] = (t[1] + dy) * g;
+        t[2] = (t[2] + dz) * g;
+        r2[p] *= g;
+        cnt[p] = c + (int)m;
+    }
+}
+// The same for the fixed-point accumulators (accum_mode 2): the pixel's integer sums, converted once. M is checked per pixel.
+__global__ void sppm_fold_fixed_kernel(unsigned int npix, double alpha, const uint32_t *__restrict__ pix_start, const uint32_t *__restrict__ pix_perm,
+                                       long long *__restrict__ acc, double *__restrict__ tau, double *__restrict__ r2, int *__restrict__ cnt, int *err) {
+    unsigned int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= npix) return;
+    long long sx = 0, sy = 0, sz = 0, sm = 0;
+    for (uint32_t j = pix_start[p]; j < pix_start[p + 1]; j++) {
+        longlong2 *ap = reinterpret_cast<longlong2 *>(acc + 4 * (size_t)pix_perm[j]);
+        const longlong2 a = ap[0], b = ap[1];
+        sx += a.x; sy += a.y; sz += b.x; sm += b.y;
+        ap[0] = make_longlong2(0, 0); ap[1] = make_longlong2(0, 0);
+    }
+    double dx, dy, dz, m;
+    fixed_to_update(sx, sy, sz, sm, err, dx, dy, dz, m);
     if (m > 0) {
         int c = cnt[p];
         double g = u2_gain(c, m, alpha);
@@ -1437,6 +1540,32 @@ __global__ void __launch_bounds__(64) peer_reduce_update_kernel(unsigned int n, 
         dx = fx; dy = fy; dz = fz; m = fm;
         reinterpret_cast<float4 *>(clear_next)[k] = make_float4(0, 0, 0, 0);
     }
+    if (m > 0) round_update_tail(A, k, alpha, dx, dy, dz, m);
+}
+// The same for the fixed-point accumulators (accum_mode 2): integer sums give the same bits in any rank order; M is checked after the
+// exchange.
+__global__ void __launch_bounds__(64) peer_reduce_update_fixed_kernel(unsigned int n, double alpha, HpArrays A, const __grid_constant__ PeerPtrs acc,
+                                                                      int world, long long *__restrict__ clear_next, int *err) {
+    unsigned int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    long long sx = 0, sy = 0, sz = 0, sm = 0;
+    for (int g0 = 0; g0 < world; g0 += 4) {
+        longlong2 lo[4], hi[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            lo[j] = make_longlong2(0, 0); hi[j] = make_longlong2(0, 0);
+            if (g0 + j < world) {
+                const longlong2 *ap = reinterpret_cast<const longlong2 *>(reinterpret_cast<const long long *>(acc.p[g0 + j]) + 4 * (size_t)k);
+                lo[j] = __ldcg(ap); hi[j] = __ldcg(ap + 1);
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < 4; j++) { sx += lo[j].x; sy += lo[j].y; sz += hi[j].x; sm += hi[j].y; }
+    }
+    longlong2 *cn = reinterpret_cast<longlong2 *>(clear_next + 4 * (size_t)k);
+    cn[0] = make_longlong2(0, 0); cn[1] = make_longlong2(0, 0);
+    double dx, dy, dz, m;
+    fixed_to_update(sx, sy, sz, sm, err, dx, dy, dz, m);
     if (m > 0) round_update_tail(A, k, alpha, dx, dy, dz, m);
 }
 

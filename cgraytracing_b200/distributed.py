@@ -131,7 +131,7 @@ class GpuEngine:
             dist.all_gather_object(blobs, mine, group=self.group)
             self.ctx.peer_attach(self.rank, self.world, blobs)
         ptr, n = self.ctx.accum_dev()
-        ts = "<f8" if self.ctx.accum_mode == 0 else "<f4"
+        ts = {0: "<f8", 1: "<f4", 2: "<i8"}[self.ctx.accum_mode]  # fp64, float, or int64 fixed point (summed exactly by any all-reduce)
         self._acc = self.torch.as_tensor(_DevArray(ptr, n, ts), device=f"cuda:{self.device}") if n else None
 
     def photon_pass(self, first, count):

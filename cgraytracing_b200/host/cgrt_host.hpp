@@ -306,7 +306,7 @@ struct RenderOptions {
     int num_threads = 8;                 // :224 — the reference traces num_photon * num_threads photons in total (:222,256)
     int rounds = 1;                      // per-round radius/flux updates the total is split into (reference: per photon, SURVEY Q1)
     int hashsize = 1000001;              // :184
-    int accum_mode = 0;                  // 0: fp64 atomics, 1: float32 x4 accumulators
+    int accum_mode = 0;                  // 0: fp64 atomics, 1: float32 x4 accumulators, 2: int64 fixed point (the same bits on any GPU count)
     bool per_photon_update = false;      // true: the reference's own rule, main.cpp:119-122 — every accepted photon shrinks the radius at once
                                          // (one GPU; `rounds` then only says how often filter radii are refreshed). false: one update per round
     uint64_t seed = 20261018ull;

@@ -17,7 +17,7 @@ using namespace cgrt_host;
 
 int main(int argc, char **argv) {
     if (argc < 7) {
-        std::fprintf(stderr, "usage: %s <bunny|dragon|spheres> <width> <height> <photons> <rounds> <out.ppm> [assets-dir] [gpus] [peer|nccl] [off|jitter|corner]\n",
+        std::fprintf(stderr, "usage: %s <bunny|dragon|spheres> <width> <height> <photons> <rounds> <out.ppm> [assets-dir] [gpus] [peer|nccl] [off|jitter|corner] [accum_mode]\n",
                      argv[0]);
         return 2;
     }
@@ -33,6 +33,7 @@ int main(int argc, char **argv) {
         else if (mode == "corner") opt.sppm = CGRT_SPPM_CORNER;
         else if (mode != "off") { std::fprintf(stderr, "unknown mode %s (off|jitter|corner)\n", mode.c_str()); return 2; }
     }
+    if (argc > 11) opt.accum_mode = std::atoi(argv[11]);  // 2: fixed-point accumulators (the same image on any GPU count)
     try {
         // floor texture: Texture(tdata, Vec3(0,1,0), Vec3(-21,0,0), 42, 40, false) — main.cpp:320 with ChessBoard.png
         int tw = 0, th = 0;

@@ -27,7 +27,7 @@ typedef enum cgrt_status {
     CGRT_ERR_INVALID = -1,   /* bad argument / call order */
     CGRT_ERR_CUDA = -2,      /* a CUDA call failed; see cgrt_last_error */
     CGRT_ERR_NO_DEVICE = -3, /* no usable GPU: there is NO CPU fallback */
-    CGRT_ERR_CAPACITY = -4,  /* a fixed-size table (objects, textures, BVHs, queue) is full */
+    CGRT_ERR_CAPACITY = -4,  /* a fixed-size table (objects, textures, BVHs, queue) is full, or a fixed-point sum left its range (accum_mode 2) */
     CGRT_ERR_NCCL = -5
 } cgrt_status;
 
@@ -38,7 +38,11 @@ typedef struct cgrt_config {
     int32_t num_of_samples;     /* main.cpp:177 */
     int32_t use_dof;            /* 1: trace the thin-lens ray of main.cpp:203-207 instead of the pinhole ray of :209 */
     int32_t hashsize;           /* Hashtable(hashsize, r), main.cpp:184 */
-    int32_t accum_mode;         /* 0: fp64 atomics (parity), 1: one red.global.add.v4.f32 per deposit (fast) */
+    int32_t accum_mode;         /* 0: fp64 atomics (parity), 1: one red.global.add.v4.f32 per deposit (fast), 2: fixed point — every accepted
+                                 * pair adds round-half-even(cf * 2^22) to int64 sums, cf = ((float)f * (float)flux) * (float)(1/pi), so flux,
+                                 * radii, counts and image are the same bits on every run and any GPU count. A value cf > 2^16 or a round's
+                                 * M > 2^24 (per hitpoint; SPPM: per pixel) makes the next synchronising call return CGRT_ERR_CAPACITY.
+                                 * Any other value is CGRT_ERR_INVALID. update_mode 0 always uses 0. */
     int32_t update_mode;        /* 1 (default): one radius/flux update per round against the round-start radius (SURVEY Q1 "U2", the rule that
                                  * shards over GPUs); 0: the reference's own rule, main.cpp:119-122 — every accepted photon shrinks the radius at
                                  * once and later photons are tested against the shrunk radius ("U1"; one GPU, fp64 accumulators) */
@@ -136,7 +140,8 @@ int cgrt_photon_pass(cgrt_ctx *ctx, uint64_t first, uint64_t count);
  *   after cgrt_build_grid; x, y unused). Ray k draws the random numbers of photon index first_index + k (bounce = depth onwards). */
 int cgrt_trace(cgrt_ctx *ctx, int64_t n, const double *org, const double *dir, const double *weight, int flag, int depth,
                const int32_t *x, const int32_t *y, uint64_t first_index);
-/* Device view of the per-round accumulators {dflux[3], m} (4 x fp64 per hitpoint, canonical order) for the all-reduce. */
+/* Device view of the per-round accumulators {dflux[3], m} (4 lanes per hitpoint, canonical order) for the all-reduce: fp64 (accum_mode
+ * 0), float (1) or int64 fixed point {sum q[3], M} (2). */
 int cgrt_accum_dev(cgrt_ctx *ctx, void **ptr_dev, int64_t *n_doubles);
 /* ---- multi-GPU (SURVEY section 8e): NCCL is bound at run time (the copy already loaded in the process, else libnccl.so.2); none of
  * these is needed on one GPU. A communicator is an ncclComm_t passed as void*. ------------------------------------------------ */
@@ -220,6 +225,7 @@ int cgrt_average_f64(cgrt_ctx *ctx, int n, const double *const *imgs, int64_t nv
 int cgrt_num_hitpoints(cgrt_ctx *ctx, int64_t *n);
 int cgrt_download_hitpoints(cgrt_ctx *ctx, double *pos, double *normal, double *f, double *flux, double *r2, int32_t *n,
                             int32_t *hw, uint32_t *key, uint32_t *seq);
+/* The round's accumulators as the update reads them; accum_mode 2: sum q * 2^-22 and M. */
 int cgrt_download_accum(cgrt_ctx *ctx, double *dflux, double *m);
 int cgrt_download_grid(cgrt_ctx *ctx, uint32_t *cell_start /* hashsize+1 */);
 int cgrt_get_counters(cgrt_ctx *ctx, cgrt_counters *out);
@@ -251,7 +257,7 @@ int cgrt_check_guards(cgrt_ctx *ctx, uint64_t *damaged);
 /* Photons one trace launch of cgrt_photon_pass takes (sized from free device memory at the first pass; 0 before it). */
 int cgrt_photon_chunk(cgrt_ctx *ctx, uint64_t *photons_per_launch);
 /* Bytes of one slot of the deposit table (record written per recorded photon hit, read once by the gather) under the context's
- * configuration — 64 with float accumulators, 96 with fp64 ones (NULL: 96): the unit of the measurement's compulsory-traffic accounting. */
+ * configuration — 64 with float or fixed-point accumulators, 96 with fp64 ones (NULL: 96): the unit of the measurement's compulsory-traffic accounting. */
 int cgrt_deposit_record_bytes(const cgrt_ctx *ctx);
 /* The library keeps the large device buffers of destroyed contexts (deposit tables, photon queues, ray queues) parked per device and
  * hands them to the next context: a render() creates and destroys one. Parked blocks are released automatically when an allocation
